@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- depth frames/sec of the hGRU-pose forward (8 timesteps, 15x15 horizontal kernels).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one forward pass of the whole hot path (stem -> 8-step hGRU -> readout) over one batch
@@ -46,7 +46,32 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-stages", action="store_true", help="skip the crop / post-processing stage timings")
     ap.add_argument("--no-extra", action="store_true", help="skip the short runs of the other BASELINE configs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the predictions of the last timed step to DIR/out_put.npy (float32), so that two "
+                         "builds can be compared output for output on the same seeded inputs")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_output(directory, name, x):
+    """Writes x as DIR/<name>.npy in float32.  An output larger than DUMP_LIMIT_BYTES (many ranks' gathered
+    predictions) is cut to a fixed, seeded sample of its rows, whose sorted indices go to DIR/<name>_rows.npy."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    x = np.ascontiguousarray(x, dtype=np.float32)
+    if x.nbytes > DUMP_LIMIT_BYTES:
+        n_rows = DUMP_LIMIT_BYTES // (x[:1].nbytes + 8)          # + 8 bytes per row for its float64 index
+        rows = np.sort(np.random.default_rng(0).choice(len(x), n_rows, replace=False))
+        x = x[rows]
+        np.save(os.path.join(directory, name + "_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(directory, name + ".npy"), x)
 
 
 def config_label(batch, channels, timesteps):
@@ -249,9 +274,11 @@ def run_ours(a):
         # sharded: every step's predictions are all-gathered, asynchronously into one of two buffers, so a step does
         # not wait for the collective (and through it for the slowest rank) before the next forward starts
         gatherer = PredictionGatherer(B, 69, device="cuda") if (gather and world > 1) else None
+        last = [None]
 
         def step_dev():
             out = m.build(depth_dev, 69)
+            last[0] = out
             if gatherer is not None:
                 gatherer.submit(out)
                 if os.environ.get("BENCH_SYNC_GATHER") == "1":      # A/B switch: wait for every step's collective
@@ -274,6 +301,8 @@ def run_ours(a):
         g_mean, g_min = ctypes.c_float(0), ctypes.c_float(0)
         lib.pose_plan_sm_clock_ghz(m._plan, ctypes.byref(g_mean), ctypes.byref(g_min))
         lib.hgru_enable_kernel_timing(0)
+        # what the last timed step handed its caller: this rank's predictions, or every rank's once gathered
+        last_out = gatherer.result().clone() if gatherer is not None else last[0]
         clk = clocks.stop(t0, t1) if clocks else None
         if clk is not None:
             # nvidia-smi keeps reporting the nominal clock; this is what the conv kernel's own clock64 / %globaltimer saw
@@ -304,7 +333,7 @@ def run_ours(a):
         flops_per_launch = 2.0 * B * 64 * 64 * 15 * 15 * channels * channels     # SURVEY 8(d): 2*H*W*S^2*k^2 per frame
         res = {"ms_dev": ms_dev, "ms_host": ms_host, "ms_stream": ms_stream if depth_pin is not None else None,
                "launches_per_step": launches, "clk": clk,
-               "flops_per_launch": flops_per_launch, "roof": None, "out": out_check,
+               "flops_per_launch": flops_per_launch, "roof": None, "out": out_check, "last_out": last_out,
                "sm_clock_in_kernel_ghz": round(float(g_mean.value), 4) if g_mean.value else None}
         if k_n.value > 0 and mode in ("bf16", "bf16x3"):
             avg_ms = k_ms.value / k_n.value
@@ -344,6 +373,8 @@ def run_ours(a):
             dist.destroy_process_group()
         return
 
+    if a.dump_outputs:
+        dump_output(a.dump_outputs, "out_put", r["last_out"].cpu().numpy())
     frames = B * world * a.steps
     value = frames / (ms_dev * 1e-3)
     e2e = frames / (ms_host * 1e-3)

@@ -163,7 +163,8 @@ def test_circuit_step_methods_mirror_the_reference_signatures():
     names and order; they need CUDA tensors (no CPU fallback)."""
     import inspect
     import re
-    src = open("/root/reference/hgru_module.py").read() if os.path.exists("/root/reference/hgru_module.py") else None
+    ref_path = os.path.join(os.environ.get("MONKEY_POSE_REFERENCE", ""), "hgru_module.py")
+    src = open(ref_path).read() if os.path.isfile(ref_path) else None
     want = {
         "conv_2d_op": ["self", "data", "weight_key", "out_key", "weights", "symmetric_weights", "rectify"],
         "p_convolution": ["self", "data", "key", "rectification"],
@@ -178,7 +179,7 @@ def test_circuit_step_methods_mirror_the_reference_signatures():
     for name, args in want.items():
         got = [a for a in inspect.signature(getattr(mp.ContextualCircuit, name)).parameters if not a.startswith("_")]
         assert got == args, (name, got)
-        if src is not None:                      # this container only: the table above IS the reference's
+        if src is not None:                      # with the reference's source: the table above IS the reference's
             m = re.search(r"def %s\(([^)]*)\)" % name, src)
             ref = [a.split("=")[0].strip() for a in m.group(1).replace("\n", " ").split(",") if a.strip()]
             assert ref == args, (name, ref)

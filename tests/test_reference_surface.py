@@ -1,9 +1,12 @@
-"""CPU, this container only (needs /root/reference): every function and method the reference defines in the files of
-the hot path and its neighbouring stages has a same-named counterpart in the mirror package -- as a kernel-backed
-method, or (for what SURVEY.md section 8 row a19 lists as declared but not on the configured path) as a method that
-raises the reference's own NotImplementedError.  The few names left out are listed here with the reason."""
+"""CPU: every function and method the reference defines in the files of the hot path and its neighbouring stages has a
+same-named counterpart in the mirror package -- as a kernel-backed method, or (for what SURVEY.md section 8 row a19
+lists as declared but not on the configured path) as a method that raises the reference's own NotImplementedError.  The
+few names left out are listed here with the reason.  The reference's names are stored in golden/reference_surface.json;
+with MONKEY_POSE_REFERENCE naming a checkout of the reference (krg-nandu/monkey-pose) they are also read from its source,
+the stored ones must be among them, and the tests use the names read."""
+import json
 import os
-import re
+import sys
 
 import pytest
 import torch
@@ -11,21 +14,22 @@ import torch
 import monkey_pose_b200 as mp
 from monkey_pose_b200 import pose_evaluation, tf_monkeydetector
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="the reference tree is only present in the build container")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+sys.path.insert(0, GOLDEN)
+import make_golden_reference_surface as surface  # noqa: E402
 
-DEF = re.compile(r"^([ \t]*)def\s+(\w+)\s*\(", re.M)
+STORED = json.load(open(os.path.join(GOLDEN, "reference_surface.json")))
+REF = os.environ.get("MONKEY_POSE_REFERENCE", "")
 
 
 def _defs(path, cls=None):
-    """Names defined at module level (cls None) or inside class `cls` of a (Python-2) source file."""
-    src = open(os.path.join(REF, path)).read()
-    if cls is None:
-        return [m.group(2) for m in DEF.finditer(src) if m.group(1) == ""]
-    start = re.search(r"^class\s+%s\b.*$" % cls, src, re.M).end()
-    nxt = re.search(r"^(class|def)\s+\w+", src[start:], re.M)
-    body = src[start:start + nxt.start()] if nxt else src[start:]
-    return [m.group(2) for m in DEF.finditer(body) if m.group(1) != ""]
+    """Names the reference defines at module level (cls None) or inside class `cls` of `path`."""
+    names = list(STORED[path][cls or ""])
+    if os.path.isdir(REF):
+        read = list(surface.defs(open(os.path.join(REF, path)).read(), cls or ""))
+        assert set(names) <= set(read), (path, cls, sorted(set(names) - set(read)))
+        names = read
+    return names
 
 
 def test_contextual_circuit_surface():
