@@ -40,6 +40,10 @@ extern "C" {
 #define HGRU_MODE_FP32 0 /* fp32 SIMT FFMA: the <= 1e-4 parity path                                */
 #define HGRU_MODE_BF16 1 /* tcgen05 tensor cores, bf16 operands, fp32 accumulate + fp32 state      */
 #define HGRU_MODE_BF16X3 2 /* tcgen05, bf16 hi/lo operand splits (3 products): fp32-class accuracy, S = 15    */
+/* tcgen05, fp16 operands (11 significand bits, bf16: 8) at the bf16 mode's speed; otherwise the bf16 mode.  S = 15,
+ * k <= 64.  Conversions saturate at +-65504 (never inf / NaN): an initial state beyond that is clamped in the first
+ * timestep's gated operand. */
+#define HGRU_MODE_FP16 3
 
 typedef struct hgru_plan_s* hgru_plan_t;
 typedef struct pose_plan_s* pose_plan_t;

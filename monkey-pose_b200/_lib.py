@@ -12,7 +12,8 @@ LIB_PATH = os.path.join(_HERE, "libhgru_b200.so")
 MODE_FP32 = 0
 MODE_BF16 = 1
 MODE_BF16X3 = 2
-MODES = {"fp32": MODE_FP32, "bf16": MODE_BF16, "bf16x3": MODE_BF16X3}
+MODE_FP16 = 3
+MODES = {"fp32": MODE_FP32, "bf16": MODE_BF16, "bf16x3": MODE_BF16X3, "fp16": MODE_FP16}
 
 HGRU_PARAM_ORDER = ("p_r", "i_r", "i_b", "o_r", "o_b", "beta", "nu", "gamma", "kappa", "omega",
                     "rho", "lateral_bias")

@@ -112,8 +112,9 @@ gate_tc_kernel(const __nv_bfloat16* __restrict__ act /*[N][CG][HW][8]*/, const T
 
 // Initial state of the tensor-core path in one pass (hgru_module.py:884-887, 696-711): O_0 (NHWC fp32, k channels, or
 // null = zeros) -> H2 (quad-chunked fp32, zero padded) + the first timestep's gated operand
-// A = bf16(sigmoid(O_0 *1x1 i_r + i_b) . O_0).  Same shape as gate_tc_kernel: CTA = 128 pixels of one frame, the
-// 1x1 conv is one UMMA tile; the bf16 K-major operand tile is written to shared memory by the threads that
+// A = F(sigmoid(O_0 *1x1 i_r + i_b) . O_0) (F: the 16-bit operand format, op_format.cuh; the packed i_r is in F too).
+// Same shape as gate_tc_kernel: CTA = 128 pixels of one frame, the
+// 1x1 conv is one UMMA tile; the 16-bit K-major operand tile is written to shared memory by the threads that
 // convert the state, so the state is read from HBM exactly once.  (The SIMT version of this pass was bound by its
 // shared-memory weight reads: 148 us per 256 frames at k = 25.)
 // a.wpk = packed i_r, a.bias = i_b, a.H2 = H2 out, a.out_bf16 = operand out, a.act_pad as for the stacked conv.
@@ -127,7 +128,7 @@ struct InitCfg {
   static constexpr uint32_t TMEM_COLS = KP < 32 ? 32 : KP;
 };
 
-template <int KP>
+template <int KP, class F = OpBf16>
 __global__ void __launch_bounds__(128)
 init_state_tc_kernel(const float* __restrict__ h0 /*[N][HW][k] or nullptr*/, const TcConvArgs a) {
   using namespace sm100;
@@ -180,9 +181,9 @@ init_state_tc_kernel(const float* __restrict__ h0 /*[N][HW][k] or nullptr*/, con
       st_stream(a.H2 + quad_off(a, n, 2 * cg + 1, pin),
                 make_float4(hv[8 * cg + 4], hv[8 * cg + 5], hv[8 * cg + 6], hv[8 * cg + 7]));
     }
-    __nv_bfloat162 h[4];
+    typename F::T2 h[4];
 #pragma unroll
-    for (int q = 0; q < 4; ++q) h[q] = __floats2bfloat162_rn(hv[8 * cg + 2 * q], hv[8 * cg + 2 * q + 1]);
+    for (int q = 0; q < 4; ++q) h[q] = F::cvt2(hv[8 * cg + 2 * q], hv[8 * cg + 2 * q + 1]);
     *reinterpret_cast<uint4*>(gen + cg * 2048 + m * 16) = *reinterpret_cast<const uint4*>(h);   // K-major operand tile
   }
   fence_proxy_async();          // operand tile -> visible to the tensor core
@@ -195,7 +196,7 @@ init_state_tc_kernel(const float* __restrict__ h0 /*[N][HW][k] or nullptr*/, con
     const bool leader = elect_one();
     mbar_wait(bar_ld, 0);
     tc_fence_after();
-    constexpr uint32_t idesc = make_idesc(1, 128, KP);
+    constexpr uint32_t idesc = make_idesc(F::kIdescFmt, 128, KP);
     const uint64_t adesc = make_smem_desc(a_buf, 2048, 128);        // LBO: chunk plane, SBO: 8 pixels
     const uint64_t bdesc = make_smem_desc(w_buf, KP * 16, 128);
 #pragma unroll
@@ -214,7 +215,7 @@ init_state_tc_kernel(const float* __restrict__ h0 /*[N][HW][k] or nullptr*/, con
 #pragma unroll
     for (int j = 0; j < 8; ++j)      // pad channels: hv = 0
       r[j] = (c0 + j < k) ? fast_sigmoid(acc[j] + __ldg(a.bias + c0 + j)) * hv[c0 + j] : 0.f;
-    if (live) store_act_chunk(a, a.out_bf16, n, c0 >> 3, pin, r);
+    if (live) store_act_chunk<F>(a, a.out_bf16, n, c0 >> 3, pin, r);
   }
   (void)lane;
   tc_fence_before();

@@ -47,10 +47,12 @@ namespace hgru {
 
 // GX3: the epilogue-issued 1x1 gate conv runs on bf16 hi/lo splits too (bf16x3 mode): staging tiles for both halves
 // of the new state, gate weights as [w_hi | w_lo] stacked along N plus w_hi (the SPLIT3 packing of hconv_tc.cuh).
-template <int KP_, int T_, int KC_, int CS_, bool GX3_ = false>
+// F_: format of the 16-bit operands, window, weights and gate staging tile (op_format.cuh).
+template <int KP_, int T_, int KC_, int CS_, bool GX3_ = false, class F_ = OpBf16>
 struct StackCfg {
   static constexpr int KP = KP_, T = T_, KC = KC_, CS = CS_;
   static constexpr bool GX3 = GX3_;
+  using Fmt = F_;
   static constexpr int S = 15, PAD = 7;
   static constexpr int KSTEPS = KP / 16;
   static constexpr int CG = KP / 8;
@@ -123,13 +125,15 @@ struct StackCfg {
   static_assert(CS == 1 || CS == 2, "single CTA or CTA pair");
   static_assert(STAGE_BYTES % 256 == 0, "stage must be whole 256-byte rows");
   static_assert(2 * COLS <= 256, "TMA box limit");
+  static_assert(!GX3 || Fmt::kIdescFmt == OpBf16::kIdescFmt, "hi/lo gate splits are bf16");
 };
 
-// Stacked weight packing: HWIO fp32 [15][15][k][k] -> bf16 [dy][q][rank][g][2 chunks][128/CS n'][8 ci],
+// Stacked weight packing: HWIO fp32 [15][15][k][k] -> F [dy][q][rank][g][2 chunks][128/CS n'][8 ci],
 // n = rank*(128/CS) + n' = s*KC + c  <->  tap dx = T*g + T-1-s, output channel c
 // (zero where dx >= 15 or c, ci >= k).  `rank` = which CTA of a pair holds that half of B.
-// `lo_part` = 1 packs the bf16 remainder  bf16(w - bf16(w))  instead (second weight set of the bf16x3 mode).
-__global__ void pack_weights_stack_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ wpk,
+// `lo_part` = 1 packs the remainder  F(w - F(w))  instead (second weight set of the bf16x3 mode).
+template <class F = OpBf16>
+__global__ void pack_weights_stack_kernel(const float* __restrict__ w, typename F::T* __restrict__ wpk,
                                           int k, int ksteps, int T, int KC, int NG, int CS, int lo_part = 0) {
   const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
   const size_t total = static_cast<size_t>(15) * ksteps * NG * 2 * 128 * 8;
@@ -149,8 +153,8 @@ __global__ void pack_weights_stack_kernel(const float* __restrict__ w, __nv_bflo
   const int ci = q * 16 + ch * 8 + j;
   float v = 0.f;
   if (s < T && dx >= 0 && dx < 15 && c < k && ci < k) v = w[((static_cast<size_t>(dy) * 15 + dx) * k + ci) * k + c];
-  const __nv_bfloat16 hi = __float2bfloat16(v);
-  wpk[i] = lo_part ? __float2bfloat16(v - __bfloat162float(hi)) : hi;
+  const typename F::T hi = F::cvt(v);
+  wpk[i] = lo_part ? F::cvt(v - F::to_float(hi)) : hi;
 }
 
 // Same for the remainder-packed schedule (StackCfg::REM, KC = 25): [stage 24][g][2 chunks][128 n'][8 j] with the
@@ -159,7 +163,8 @@ __global__ void pack_weights_stack_kernel(const float* __restrict__ w, __nv_bflo
 //   stage 15 + i    (0..6) : chunks = channels 16..23 of filter rows 2i and 2i + 1
 //   stage 22               : chunk 0 = channels 16..23 of row 14, chunk 1 = channel 24 of rows 0..7
 //   stage 23               : chunk 0 = channel 24 of rows 8..14 (+ one zero), chunk 1 = zero
-__global__ void pack_weights_stack_rem_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ wpk, int k,
+template <class F = OpBf16>
+__global__ void pack_weights_stack_rem_kernel(const float* __restrict__ w, typename F::T* __restrict__ wpk, int k,
                                               int T, int KC, int NG, int lo_part = 0) {
   const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
   const size_t total = static_cast<size_t>(24) * NG * 2 * 128 * 8;
@@ -180,8 +185,8 @@ __global__ void pack_weights_stack_rem_kernel(const float* __restrict__ w, __nv_
   float v = 0.f;
   if (dy >= 0 && s < T && dx >= 0 && dx < 15 && c < k && ci < k)
     v = w[((static_cast<size_t>(dy) * 15 + dx) * k + ci) * k + c];
-  const __nv_bfloat16 hi = __float2bfloat16(v);
-  wpk[i] = lo_part ? __float2bfloat16(v - __bfloat162float(hi)) : hi;
+  const typename F::T hi = F::cvt(v);
+  wpk[i] = lo_part ? F::cvt(v - F::to_float(hi)) : hi;
 }
 
 namespace detail {
@@ -290,7 +295,7 @@ __device__ __forceinline__ void stack_mma_issuer(const TcConvArgs& a, uint32_t t
   (void)kMask;
   const bool leader = elect_one();
   tmem_base = __shfl_sync(0xffffffffu, tmem_base, 0);      // read from shared memory: mark it warp-uniform
-  constexpr uint32_t idesc = make_idesc(1 /*bf16*/, 128 * CS, Cfg::NPAD);
+  constexpr uint32_t idesc = make_idesc(Cfg::Fmt::kIdescFmt, 128 * CS, Cfg::NPAD);
   const uint64_t adesc0 = make_smem_desc(win, Cfg::CHUNK_PITCH, Cfg::ROW_PITCH);
   const uint64_t bdesc0 = make_smem_desc(w_buf, Cfg::NLOC * 16, 128);
   uint32_t st = 0, ph = 0;
@@ -562,14 +567,14 @@ __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0
       if (store) Epi::template finish<NCH, CN>(a, n, pin, C0, out, pre, hv);
       if constexpr (PROF) { const long long t = clock64(); e_fin += t - e0; e0 = t; }
       if (gate_follows) {
-        // ---- fused gate: new state -> bf16 staging tile -> 1x1 conv on the tensor core -> sigmoid ----
+        // ---- fused gate: new state -> 16-bit (Cfg::Fmt) staging tile -> 1x1 conv on the tensor core -> sigmoid ----
         {
           uint8_t* stg = smem_raw + (gate_a - smem_u32(smem_raw));
 #pragma unroll
           for (int i = 0; i < NCH / 8; ++i) {
-            __nv_bfloat162 h[4];
+            typename Cfg::Fmt::T2 h[4];
 #pragma unroll
-            for (int q = 0; q < 4; ++q) h[q] = __floats2bfloat162_rn(hv[8 * i + 2 * q], hv[8 * i + 2 * q + 1]);
+            for (int q = 0; q < 4; ++q) h[q] = Cfg::Fmt::cvt2(hv[8 * i + 2 * q], hv[8 * i + 2 * q + 1]);
             *reinterpret_cast<uint4*>(stg + ((C0 >> 3) + i) * 2048 + m * 16) = *reinterpret_cast<const uint4*>(h);
             if constexpr (Cfg::GX3) {      // the bf16 remainders, as a second tile
               __nv_bfloat162 l[4];
@@ -591,11 +596,11 @@ __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0
           const bool leader = elect_one();
           tc_fence_after();
           if (leader) {
-            constexpr uint32_t gdesc = make_idesc(1, 128, KP);
+            constexpr uint32_t gdesc = make_idesc(Cfg::Fmt::kIdescFmt, 128, KP);
             const uint64_t ad = make_smem_desc(gate_a, 2048, 128);
             if constexpr (Cfg::GX3) {
               // hi * [w_hi | w_lo] -> columns [0, 2 KP), then lo * w_hi added into columns [0, KP)
-              constexpr uint32_t gdesc_w = make_idesc(1, 128, 2 * KP);
+              constexpr uint32_t gdesc_w = make_idesc(Cfg::Fmt::kIdescFmt, 128, 2 * KP);
               const uint64_t ad_lo = make_smem_desc(gate_a + Cfg::GATE_A_HALF, 2048, 128);
               const uint64_t bd_w = make_smem_desc(gate_w, 2 * KP * 16, 128);
               const uint64_t bd_n = make_smem_desc(gate_w + 4 * KP * 16, KP * 16, 128);
@@ -661,13 +666,14 @@ __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0
   }
 }
 
+// F: 16-bit operand format (op_format.cuh); Epi writes the next launch's operands in the same format.
 template <int KP, int T, int KC, int CS, class Epi, bool PROF = false, int WSETS = 1, bool PART = false,
-          bool GX3 = false>
-__global__ void __launch_bounds__((StackCfg<KP, T, KC, CS, GX3>::NTHREADS), 1)
+          bool GX3 = false, class F = OpBf16>
+__global__ void __launch_bounds__((StackCfg<KP, T, KC, CS, GX3, F>::NTHREADS), 1)
 hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ CUtensorMap w_map,
                    const TcConvArgs a) {
   using namespace sm100;
-  using Cfg = StackCfg<KP, T, KC, CS, GX3>;
+  using Cfg = StackCfg<KP, T, KC, CS, GX3, F>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t win = base;

@@ -28,6 +28,7 @@
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
+#include "op_format.cuh"
 #include "sm100_ptx.cuh"
 
 namespace hgru {
@@ -96,6 +97,8 @@ struct TcConvArgs {
   int kreal;                // real channel count (pad channels are written as zero)
   int units_x, units_y;     // units per frame
   int num_units;
+  // (16-bit tensors are typed bf16 here; in the fp16 mode the hGRU conv operands and weights hold fp16,
+  //  see op_format.cuh -- the kernels only move their bytes or write them through the launch's format)
   const __nv_bfloat16* wpk; // packed weights [KSTEPS][taps][2][CO_PAD][8]
   const float* bias;        // [KP] lateral bias / conv bias (zero padded)
   const float* scale;       // [KP] (EpiBiasReluAffine) batch-norm scale, zero padded
@@ -247,52 +250,58 @@ __device__ __forceinline__ float fast_tanh(float x) {
 }
 // per-channel parameter quad; generic load: the stacked kernel stages these vectors in shared memory
 __device__ __forceinline__ float4 ld_par4(const float* p) { return *reinterpret_cast<const float4*>(p); }
-__device__ __forceinline__ void store_chunk_bf16(__nv_bfloat16* base, int KP, int HWp, int n, int cg,
-                                                 size_t pin, const float* r) {
-  __nv_bfloat162 h[4];
+// 8 channels of one pixel -> a chunked 16-bit operand tensor in format F (see op_format.cuh)
+template <class F = OpBf16>
+__device__ __forceinline__ void store_chunk16(__nv_bfloat16* base, int KP, int HWp, int n, int cg, size_t pin,
+                                              const float* r) {
+  typename F::T2 h[4];
 #pragma unroll
-  for (int j = 0; j < 4; ++j) h[j] = __floats2bfloat162_rn(r[2 * j], r[2 * j + 1]);
+  for (int j = 0; j < 4; ++j) h[j] = F::cvt2(r[2 * j], r[2 * j + 1]);
   __nv_bfloat16* o = base + ((static_cast<size_t>(n) * (KP >> 3) + cg) * HWp + pin) * 8;
   st_stream(o, *reinterpret_cast<const uint4*>(h));
 }
 // Operand store that honours TcConvArgs::act_pad (remainder-packed layout, see StackCfg::REM): chunk planes
 // have act_pad zero rows on top; the last chunk is the row-packed plane P[y][x][j] = v(y + j, x) of channel
 // KP - 8, so this pixel's value goes to the 8 planes rows y - j (j = 0..7), element j.
+// (F: the operand format, op_format.cuh; the hi / lo splits of split_out are made in it too)
+template <class F = OpBf16>
 __device__ __forceinline__ void store_act_chunk1(const TcConvArgs& a, __nv_bfloat16* base, int n, int cg,
                                                  size_t pin, const float* r);
+template <class F = OpBf16>
 __device__ __forceinline__ void store_act_chunk(const TcConvArgs& a, __nv_bfloat16* base, int n, int cg,
                                                 size_t pin, const float* r) {
   if (a.split_out) {
     float hi[8], lo[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
-      hi[j] = __bfloat162float(__float2bfloat16(r[j]));
+      hi[j] = F::to_float(F::cvt(r[j]));
       lo[j] = r[j] - hi[j];
     }
     if (a.split_out == 2) {      // two tensors in the stacked kernel's own layout
-      store_act_chunk1(a, base, n, cg, pin, hi);
-      store_act_chunk1(a, base + a.lo_off, n, cg, pin, lo);
+      store_act_chunk1<F>(a, base, n, cg, pin, hi);
+      store_act_chunk1<F>(a, base + a.lo_off, n, cg, pin, lo);
       return;
     }
-    store_chunk_bf16(base, 2 * a.KP, a.H * a.W, n, cg, pin, hi);
-    store_chunk_bf16(base, 2 * a.KP, a.H * a.W, n, (a.KP >> 3) + cg, pin, lo);
+    store_chunk16<F>(base, 2 * a.KP, a.H * a.W, n, cg, pin, hi);
+    store_chunk16<F>(base, 2 * a.KP, a.H * a.W, n, (a.KP >> 3) + cg, pin, lo);
     return;
   }
-  store_act_chunk1(a, base, n, cg, pin, r);
+  store_act_chunk1<F>(a, base, n, cg, pin, r);
 }
+template <class F>
 __device__ __forceinline__ void store_act_chunk1(const TcConvArgs& a, __nv_bfloat16* base, int n, int cg,
                                                  size_t pin, const float* r) {
   if (a.act_pad == 0) {
-    store_chunk_bf16(base, a.KP, a.H * a.W, n, cg, pin, r);
+    store_chunk16<F>(base, a.KP, a.H * a.W, n, cg, pin, r);
     return;
   }
   const size_t plane = static_cast<size_t>(a.H + a.act_pad) * a.W;
   const size_t pp = pin + static_cast<size_t>(a.act_pad) * a.W;
   if (cg != (a.KP >> 3) - 1) {
-    store_chunk_bf16(base, a.KP, static_cast<int>(plane), n, cg, pp, r);
+    store_chunk16<F>(base, a.KP, static_cast<int>(plane), n, cg, pp, r);
   } else {
-    __nv_bfloat16* o = base + ((static_cast<size_t>(n) * (a.KP >> 3) + cg) * plane + pp) * 8;
-    const __nv_bfloat16 v = __float2bfloat16(r[0]);
+    typename F::T* o = reinterpret_cast<typename F::T*>(base) + ((static_cast<size_t>(n) * (a.KP >> 3) + cg) * plane + pp) * 8;
+    const typename F::T v = F::cvt(r[0]);
 #ifdef HGRU_DBG_REM_ONE_STORE
     o[0] = v;      // development: upper bound of what a cheaper remainder-plane write could give (wrong results)
 #else
@@ -370,8 +379,8 @@ struct EpiBiasReluAffine {
           hi[j] = __bfloat162float(__float2bfloat16(r[j]));
           lo[j] = r[j] - hi[j];
         }
-        store_chunk_bf16(a.out_bf16, 2 * a.KP, a.H * a.W, n, c >> 3, pin, hi);
-        store_chunk_bf16(a.out_bf16, 2 * a.KP, a.H * a.W, n, (a.KP >> 3) + (c >> 3), pin, lo);
+        store_chunk16(a.out_bf16, 2 * a.KP, a.H * a.W, n, c >> 3, pin, hi);
+        store_chunk16(a.out_bf16, 2 * a.KP, a.H * a.W, n, (a.KP >> 3) + (c >> 3), pin, lo);
       }
     }
   }
@@ -385,8 +394,8 @@ struct EpiBiasReluAffine {
 //
 // input_integration fused into the C1 conv (hgru_module.py:657, 795-804):
 //   C1 = acc + lateral_bias;  H1 = tanh(X - (beta*H2 + nu) * C1)
-// writes H1 fp32 and its bf16 chunked operand copy.  bias = lateral_bias, v0 = beta, v1 = nu.
-template <bool HALF>
+// writes H1 fp32 and its chunked operand copy (format F, op_format.cuh).  bias = lateral_bias, v0 = beta, v1 = nu.
+template <bool HALF, class F = OpBf16>
 struct EpiH1T {
   static constexpr bool kGate = true;
   template <int NCH>
@@ -479,7 +488,7 @@ struct EpiH1T {
         st_stream(a.out + quad_off(a, n, (c0 + c) >> 2, pin), make_float4(r[0], r[1], r[2], r[3]));
         st_stream(a.out + quad_off(a, n, ((c0 + c) >> 2) + 1, pin), make_float4(r[4], r[5], r[6], r[7]));
       }
-      store_act_chunk(a, a.out_bf16, n, (c0 + c) >> 3, pin, r);
+      store_act_chunk<F>(a, a.out_bf16, n, (c0 + c) >> 3, pin, r);
       if (hout) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) hout[c + j] = r[j];
@@ -501,11 +510,12 @@ struct EpiH1T {
 };
 using EpiH1 = EpiH1T<false>;
 using EpiH1h = EpiH1T<true>;      // fused bf16 pipeline: H1 and G2 leave as fp16
+using EpiH1hF16 = EpiH1T<true, OpFp16>;      // ... with fp16 conv operands (the fp16 mode)
 // output_integration + adaptation fused into the C2 conv (hgru_module.py:657, 806-823, 847-849):
 //   C2 = acc + lateral_bias; e = gamma*C2; Ht = tanh(kappa*(H1+e) + omega*(H1*e));
-//   H2 = (G2*H2 + (1-G2)*Ht) * rho_t      (in place) + bf16 chunked copy of the new H2.
+//   H2 = (G2*H2 + (1-G2)*Ht) * rho_t      (in place) + chunked operand copy of the new H2 (format F).
 // bias = lateral_bias, v0 = gamma, v1 = kappa, v2 = omega.
-template <bool HALF>
+template <bool HALF, class F = OpBf16>
 struct EpiH2T {
   static constexpr bool kGate = true;
   // HALF: h1 / g hold the raw 16-byte fp16 chunks (8 channels each) until `finish` unpacks them
@@ -542,7 +552,7 @@ struct EpiH2T {
     }
   }
   // input gate of the NEXT timestep on the tensor-core result of H2 *1x1 i_r (hgru_module.py:696-711):
-  // G1 = sigmoid(. + i_b); gated operand = bf16(G1 . H2) for the next C1 conv.
+  // G1 = sigmoid(. + i_b); gated operand = F(G1 . H2) for the next C1 conv.
   template <int NCH, int NREAL = NCH>
   __device__ static __forceinline__ void gate(const TcConvArgs& a, int n, size_t pin, int c0, const float* gacc,
                                               const float* hv) {
@@ -560,7 +570,7 @@ struct EpiH2T {
         for (int j = 0; j < 4; ++j)   // pad channels: hv = 0
           r[4 * h + j] = (c + 4 * h + j < NREAL) ? fast_sigmoid(gacc[c + 4 * h + j] + bv[j]) * hv[c + 4 * h + j] : 0.f;
       }
-      store_act_chunk(a, a.gate_act_out, n, (c0 + c) >> 3, pin, r);
+      store_act_chunk<F>(a, a.gate_act_out, n, (c0 + c) >> 3, pin, r);
     }
   }
   template <int NCH, int NREAL = NCH>
@@ -619,7 +629,7 @@ struct EpiH2T {
       st_stream(a.H2 + quad_off(a, n, (c0 + c) >> 2, pin), make_float4(r[0], r[1], r[2], r[3]));
       if (c + 4 < NREAL)      // (a quad of pure layout padding is never read back: it stays at its initial zeros)
         st_stream(a.H2 + quad_off(a, n, ((c0 + c) >> 2) + 1, pin), make_float4(r[4], r[5], r[6], r[7]));
-      if (a.out_bf16) store_chunk_bf16(a.out_bf16, a.KP, a.H * a.W, n, (c0 + c) >> 3, pin, r);
+      if (a.out_bf16) store_chunk16<F>(a.out_bf16, a.KP, a.H * a.W, n, (c0 + c) >> 3, pin, r);
       if (a.fc_a) {
         // last timestep: emit the fc_1 operand (channel-major K order c*HW + pin, bf16 hi/lo split)
         const size_t HWp = static_cast<size_t>(a.H) * a.W;
@@ -656,6 +666,7 @@ struct EpiH2T {
 };
 using EpiH2 = EpiH2T<false>;
 using EpiH2h = EpiH2T<true>;
+using EpiH2hF16 = EpiH2T<true, OpFp16>;
 // mix gate as a 1x1 tensor-core conv (hgru_module.py:729-740): G2 = sigmoid(acc + o_b) -> fp32.
 struct EpiGateOut {
   template <int CO_PAD>
@@ -697,19 +708,21 @@ struct EpiGateIn {
         r[4 * h + 2] = fast_sigmoid(acc[c + 4 * h + 2] + b.z) * v.z;
         r[4 * h + 3] = fast_sigmoid(acc[c + 4 * h + 3] + b.w) * v.w;
       }
-      store_chunk_bf16(a.out_bf16, a.KP, a.H * a.W, n, c >> 3, pin, r);   // pad channels: H2 pad is 0
+      store_chunk16(a.out_bf16, a.KP, a.H * a.W, n, c >> 3, pin, r);   // pad channels: H2 pad is 0
     }
   }
 };
 
+// F: format of the 16-bit operands (op_format.cuh); fp16 exists for the FUSE path (its Epi writes the same format).
 template <int S, int KSTEPS, int CO_PAD, int TILES_X, int G, int WSTAGES, class Epi, bool SPLIT3 = false,
-          bool FUSE = false>
+          bool FUSE = false, class F = OpBf16>
 __global__ void __launch_bounds__(256, 1)
 hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) {
   using namespace sm100;
   using Cfg = TcConvCfg<S, KSTEPS, CO_PAD, TILES_X, G, WSTAGES, SPLIT3, FUSE>;
   constexpr int NP = Cfg::kParts, NW = Cfg::kWSteps;
   static_assert(!FUSE || !SPLIT3, "the fused-gate epilogue serves the plain bf16 path");
+  static_assert(FUSE || F::kIdescFmt == OpBf16::kIdescFmt, "16-bit operand formats other than bf16: FUSE path only");
   extern __shared__ uint8_t smem_raw[];
   // aligned carve-up
   const uint32_t base = (smem_u32(smem_raw) + static_cast<uint32_t>(Cfg::kAlign - 1)) & ~static_cast<uint32_t>(Cfg::kAlign - 1);
@@ -829,8 +842,8 @@ hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) 
     const bool leader = elect_one();
     const long long clk0 = a.clk_out ? clock64() : 0;
     const unsigned long long ns0 = a.clk_out ? global_timer_ns() : 0ull;
-    constexpr uint32_t idesc_n = make_idesc(1 /*bf16*/, 128, CO_PAD);
-    constexpr uint32_t idesc_w = make_idesc(1 /*bf16*/, 128, Cfg::kAccN);      // SPLIT3: the wide a_hi pass
+    constexpr uint32_t idesc_n = make_idesc(F::kIdescFmt, 128, CO_PAD);
+    constexpr uint32_t idesc_w = make_idesc(F::kIdescFmt, 128, Cfg::kAccN);      // SPLIT3: the wide a_hi pass
     // descriptor templates: only the 14-bit start-address field changes per instruction
     const uint64_t adesc0 = make_smem_desc(in_buf, Cfg::kChunkPitch, Cfg::kRowPitch);
     const uint64_t bdesc0_n = make_smem_desc(w_buf, CO_PAD * 16, 128);
@@ -855,7 +868,7 @@ hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) 
         uint32_t dx = 0;
         if constexpr (Cfg::kPairTap) {
           // ---- paired-tap schedule (see TcConvCfg::kPairTap): stage = blocks (2 sg', 2 sg' + 1) of filter row dy ----
-          constexpr uint32_t idesc_p = make_idesc(1, 128, 128);
+          constexpr uint32_t idesc_p = make_idesc(F::kIdescFmt, 128, 128);
           const uint64_t bdesc0_p = make_smem_desc(w_buf, 2048, 128);      // block: chunk pitch 2 KB, 128 rows
           for (int sg = 0; sg < Cfg::kStagesPerKstep; ++sg) {
             const int dy = sg >> 2, sb = sg & 3;
@@ -967,13 +980,13 @@ hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) 
             if (ok) Epi::template finish<16>(a, n, pin, c0, acc, pre, hv + c0);
           }
           if (a.do_gate) {
-            // ---- fused gate: new state -> bf16 staging tile -> 1x1 conv on the tensor core -> sigmoid ----
+            // ---- fused gate: new state -> 16-bit (F) staging tile -> 1x1 conv on the tensor core -> sigmoid ----
             uint8_t* stg = smem_raw + (gate_a - smem_u32(smem_raw));
 #pragma unroll
             for (int i = 0; i < CO_PAD / 8; ++i) {
-              __nv_bfloat162 h[4];
+              typename F::T2 h[4];
 #pragma unroll
-              for (int q = 0; q < 4; ++q) h[q] = __floats2bfloat162_rn(hv[8 * i + 2 * q], hv[8 * i + 2 * q + 1]);
+              for (int q = 0; q < 4; ++q) h[q] = F::cvt2(hv[8 * i + 2 * q], hv[8 * i + 2 * q + 1]);
               *reinterpret_cast<uint4*>(stg + i * 2048 + m * 16) = *reinterpret_cast<const uint4*>(h);
             }
             fence_proxy_async();          // staging writes -> visible to the async (tensor core) proxy
@@ -984,7 +997,7 @@ hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) 
               const bool leader = elect_one();
               tc_fence_after();
               if (leader) {
-                constexpr uint32_t gdesc = make_idesc(1, 128, CO_PAD);
+                constexpr uint32_t gdesc = make_idesc(F::kIdescFmt, 128, CO_PAD);
                 const uint64_t ad = make_smem_desc(gate_a, 2048, 128);
                 const uint64_t bd = make_smem_desc(gate_w, CO_PAD * 16, 128);
 #pragma unroll

@@ -194,6 +194,9 @@ struct hgru_plan_s {
   int act_pad = 0;                  // pad rows of the bf16 operand planes (remainder-packed layout)
   bool state_ready = false;         // the caller already ran hgru_init_state_bf16 for the coming forward
   KernelTimer timer;
+  // bf16 and fp16 modes: one pipeline (16-bit operands, no hi/lo splits), parameterised by the operand format
+  bool op16() const { return mode == HGRU_MODE_BF16 || mode == HGRU_MODE_FP16; }
+  OpFormat fmt() const { return mode == HGRU_MODE_FP16 ? FMT_FP16 : FMT_BF16; }
   float* vec(int i) const { return vecs.as<float>() + static_cast<size_t>(i) * KP; }
   size_t workspace() const {
     return p_r.bytes + i_r.bytes + o_r.bytes + vecs.bytes + rho.bytes + wpk.bytes + wpk_i.bytes +
@@ -204,11 +207,27 @@ struct hgru_plan_s {
 
 enum { V_IB = 0, V_OB, V_BETA, V_NU, V_GAMMA, V_KAPPA, V_OMEGA, V_LBIAS };
 
+// development switch (environment variable set to 1)
+static bool dev_switch(const char* name) {
+  const char* e = getenv(name);
+  return e && e[0] == '1';
+}
+
 static int hgru_plan_init(hgru_plan_s* p, int N, int H, int W, int k, int S, int T, int mode) {
   if (N < 1 || H < 1 || W < 1 || k < 1 || T < 1) return fail(HGRU_E_INVALID, "hgru_plan_create: non-positive shape");
   if (S < 1 || (S % 2) == 0 || S > 15) return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: S must be odd and <= 15");
-  if (mode != HGRU_MODE_FP32 && mode != HGRU_MODE_BF16 && mode != HGRU_MODE_BF16X3)
+  if (mode != HGRU_MODE_FP32 && mode != HGRU_MODE_BF16 && mode != HGRU_MODE_BF16X3 && mode != HGRU_MODE_FP16)
     return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: unknown mode");
+  if (mode == HGRU_MODE_FP16) {
+    // fp16 operands exist for the 15x15 kernels only: tap-stacked (k <= 32) and fused paired-tap (k <= 64)
+    if (S != 15 || k > 64) return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: fp16 mode supports S = 15 and k <= 64");
+    // development switches that select a kernel without an fp16 variant
+    const bool wide = k > 32;
+    const char* sw = dev_switch("HGRU_SIMT_INIT") ? "HGRU_SIMT_INIT"
+                     : (wide && dev_switch("HGRU_NO_FUSE64")) ? "HGRU_NO_FUSE64"
+                     : (!wide && dev_switch("HGRU_FP32_HG")) ? "HGRU_FP32_HG" : nullptr;
+    if (sw) return fail(HGRU_E_UNSUPPORTED, std::string("hgru_plan_create: fp16 mode has no kernel for ") + sw + "=1");
+  }
   p->N = N; p->H = H; p->W = W; p->k = k; p->S = S; p->T = T; p->mode = mode;
   p->KP = round_up(k, 16);
   if (mode != HGRU_MODE_FP32 && p->KP == 48) p->KP = 64;      // tensor-core kernels exist for 16 / 32 / 64 padded channels
@@ -282,6 +301,7 @@ static int hgru_plan_init(hgru_plan_s* p, int N, int H, int W, int k, int S, int
     TcGeom g;
     if (!tc_geometry(S, p->KP, &g))
       return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: bf16 mode supports S in {1,3,5,7,15} and k <= 64");
+    // (bf16 and fp16 modes; the fp16 mode's shapes were checked above)
     const int ksteps = p->KP / 16;
     const size_t tapb = sizeof(__nv_bfloat16) * ksteps * 2 * p->KP * 8;
     StackGeom sg;
@@ -339,6 +359,24 @@ static void hgru_plan_free(hgru_plan_s* p) {
   for (auto b : all) b->release();
 }
 
+// weights of the bf16 / fp16 modes in their operand format F: p_r for the plan's 15x15 kernel, i_r and o_r for the
+// 1x1 gates
+template <class F>
+static void pack_op16_weights(hgru_plan_s* p, const float* p_r, const float* i_r, const float* o_r, cudaStream_t st) {
+  const int k = p->k, KP = p->KP, taps = p->S * p->S, ksteps = KP / 16;
+  auto out = [](DevBuf& b) { return b.as<typename F::T>(); };
+  if (p->fused_tc) {
+    const size_t tp = static_cast<size_t>(ksteps) * 15 * 8 * 2 * 128 * 8;
+    hgru::pack_weights_pairtap_kernel<F><<<nblk(tp), 256, 0, st>>>(p_r, out(p->wpk), k, ksteps);
+  } else if (!p->stacked) {
+    const size_t total = static_cast<size_t>(ksteps) * taps * 2 * KP * 8;
+    hgru::pack_weights_kernel<F><<<nblk(total), 256, 0, st>>>(p_r, out(p->wpk), taps, k, ksteps, KP);
+  }
+  const size_t t1 = static_cast<size_t>(ksteps) * 2 * KP * 8;
+  hgru::pack_weights_kernel<F><<<nblk(t1), 256, 0, st>>>(i_r, out(p->wpk_i), 1, k, ksteps, KP);
+  hgru::pack_weights_kernel<F><<<nblk(t1), 256, 0, st>>>(o_r, out(p->wpk_o), 1, k, ksteps, KP);
+}
+
 static int hgru_set_params_impl(hgru_plan_s* p, const float* p_r, const float* i_r, const float* i_b,
                                 const float* o_r, const float* o_b, const float* beta, const float* nu,
                                 const float* gamma, const float* kappa, const float* omega,
@@ -360,7 +398,7 @@ static int hgru_set_params_impl(hgru_plan_s* p, const float* p_r, const float* i
     stack_geometry(p->S, KP, k, &sg);
     const size_t ts = static_cast<size_t>(sg.stages) * sg.NG * 2 * 128 * 8;      // elements of one weight set
     for (int part = 0; part < 2; ++part) {      // set 0 = bf16(w), set 1 = bf16(w - bf16(w))
-      int rc = stack_pack_weights(p_r, p->wpk.as<__nv_bfloat16>() + part * ts, k, sg, part, st);
+      int rc = stack_pack_weights(p_r, p->wpk.as<__nv_bfloat16>() + part * ts, k, sg, part, FMT_BF16, st);
       if (rc) return rc;
     }
     const size_t tg = static_cast<size_t>(3 * (KP / 16)) * 2 * KP * 8;
@@ -370,22 +408,14 @@ static int hgru_set_params_impl(hgru_plan_s* p, const float* p_r, const float* i
     const int ksteps = KP / 16;
     const size_t total = static_cast<size_t>(3 * ksteps) * taps * 2 * KP * 8;
     hgru::pack_weights_split3_kernel<<<nblk(total), 256, 0, st>>>(p_r, p->wpk.as<__nv_bfloat16>(), taps, k, ksteps, KP);
-  } else {
-    const int ksteps = KP / 16;
-    const size_t total = static_cast<size_t>(ksteps) * taps * 2 * KP * 8;
+  } else {      // bf16 / fp16
     StackGeom sg;
     if (p->stacked && stack_geometry(p->S, KP, k, &sg)) {
-      int rc = stack_pack_weights(p_r, p->wpk.as<__nv_bfloat16>(), k, sg, 0, st);
+      int rc = stack_pack_weights(p_r, p->wpk.as<__nv_bfloat16>(), k, sg, 0, p->fmt(), st);
       if (rc) return rc;
-    } else if (p->fused_tc) {
-      const size_t tp = static_cast<size_t>(ksteps) * 15 * 8 * 2 * 128 * 8;
-      hgru::pack_weights_pairtap_kernel<<<nblk(tp), 256, 0, st>>>(p_r, p->wpk.as<__nv_bfloat16>(), k, ksteps);
-    } else {
-      hgru::pack_weights_kernel<<<nblk(total), 256, 0, st>>>(p_r, p->wpk.as<__nv_bfloat16>(), taps, k, ksteps, KP);
     }
-    const size_t t1 = static_cast<size_t>(ksteps) * 2 * KP * 8;
-    hgru::pack_weights_kernel<<<nblk(t1), 256, 0, st>>>(i_r, p->wpk_i.as<__nv_bfloat16>(), 1, k, ksteps, KP);
-    hgru::pack_weights_kernel<<<nblk(t1), 256, 0, st>>>(o_r, p->wpk_o.as<__nv_bfloat16>(), 1, k, ksteps, KP);
+    if (p->fmt() == FMT_FP16) pack_op16_weights<hgru::OpFp16>(p, p_r, i_r, o_r, st);
+    else pack_op16_weights<hgru::OpBf16>(p, p_r, i_r, o_r, st);
   }
   CUDA_TRY(cudaGetLastError());
   p->params_set = true;
@@ -446,13 +476,20 @@ static int hgru_run_fp32(hgru_plan_s* p, const float* Xp, float* H1_trace, float
 // C2+H2).  All integration math happens on TMEM accumulators.
 // Initial state of the bf16 path: O_0 (NHWC, or zeros) -> H2 (quad-chunked fp32) + the first gated operand.
 // Touches only H2 / actA, so it can run before (and concurrently with the input copy of) the stem.
-template <int KP>
+template <int KP, class F>
 static int launch_init_tc(const float* h0, const hgru::TcConvArgs& a, cudaStream_t st) {
   using Cfg = hgru::InitCfg<KP>;
+  if (KP == 64) SMEM_ATTR_ONCE((hgru::init_state_tc_kernel<KP, F>), Cfg::SMEM_BYTES);
   const int tiles_per_frame = (a.H * a.W + 127) / 128;
-  hgru::init_state_tc_kernel<KP><<<a.N * tiles_per_frame, 128, Cfg::SMEM_BYTES, st>>>(h0, a);
+  hgru::init_state_tc_kernel<KP, F><<<a.N * tiles_per_frame, 128, Cfg::SMEM_BYTES, st>>>(h0, a);
   CUDA_TRY(cudaGetLastError());
   return 0;
+}
+template <class F>
+static int launch_init_tc(int KP, const float* h0, const hgru::TcConvArgs& a, cudaStream_t st) {
+  if (KP == 64) return launch_init_tc<64, F>(h0, a, st);
+  if (KP == 32) return launch_init_tc<32, F>(h0, a, st);
+  return launch_init_tc<16, F>(h0, a, st);
 }
 
 static int hgru_init_state_bf16(hgru_plan_s* p, const float* H2_init_nhwc, cudaStream_t st) {
@@ -463,10 +500,8 @@ static int hgru_init_state_bf16(hgru_plan_s* p, const float* H2_init_nhwc, cudaS
     a.N = p->N; a.H = p->H; a.W = p->W; a.KP = p->KP; a.kreal = p->k; a.act_pad = p->act_pad;
     a.wpk = p->wpk_i.as<__nv_bfloat16>(); a.bias = p->vec(V_IB); a.H2 = p->H2.as<float>();
     a.out_bf16 = p->actA.as<__nv_bfloat16>();
-    if (p->KP == 64) SMEM_ATTR_ONCE(hgru::init_state_tc_kernel<64>, hgru::InitCfg<64>::SMEM_BYTES);
-    if (p->KP == 64) return launch_init_tc<64>(H2_init_nhwc, a, st);
-    if (p->KP == 32) return launch_init_tc<32>(H2_init_nhwc, a, st);
-    if (p->KP == 16) return launch_init_tc<16>(H2_init_nhwc, a, st);
+    return p->fmt() == FMT_FP16 ? launch_init_tc<hgru::OpFp16>(p->KP, H2_init_nhwc, a, st)
+                                : launch_init_tc<hgru::OpBf16>(p->KP, H2_init_nhwc, a, st);
   }
   SMEM_ATTR_ONCE(hgru::init_state_gate_kernel, 100 * 1024);
   const int KP = p->KP;
@@ -533,8 +568,8 @@ static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_n
     if (!chain) p->timer.begin(st);
     // (fused pipeline: H1 and G2 travel to the H2 launch as fp16, EpiH1h / EpiH2h; development switch
     // HGRU_FP32_HG=1: as fp32 on the stacked kernel, for A/B runs)
-    if ((rc = p->stacked    ? stack_launch(fp32_hg ? EPI_H1 : EPI_H1_HALF, 1, false, KP, p->stack_T, p->mapA, a, st)
-              : p->fused_tc ? tc_fused64_launch(EPI_H1_HALF, p->mapA, a, st)
+    if ((rc = p->stacked    ? stack_launch(fp32_hg ? EPI_H1 : EPI_H1_HALF, 1, false, KP, p->stack_T, p->fmt(), p->mapA, a, st)
+              : p->fused_tc ? tc_fused64_launch(EPI_H1_HALF, p->fmt(), p->mapA, a, st)
                             : tc_hconv_launch(EPI_H1, p->S, KP, p->mapA, a, st)))
       return rc;
     if (!chain) p->timer.end(st);
@@ -563,8 +598,8 @@ static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_n
     }
     set_flags(a, 2 * t + 1);
     if (!chain) p->timer.begin(st);
-    if ((rc = p->stacked    ? stack_launch(fp32_hg ? EPI_H2 : EPI_H2_HALF, 1, false, KP, p->stack_T, p->mapH1, a, st)
-              : p->fused_tc ? tc_fused64_launch(EPI_H2_HALF, p->mapH1, a, st)
+    if ((rc = p->stacked    ? stack_launch(fp32_hg ? EPI_H2 : EPI_H2_HALF, 1, false, KP, p->stack_T, p->fmt(), p->mapH1, a, st)
+              : p->fused_tc ? tc_fused64_launch(EPI_H2_HALF, p->fmt(), p->mapH1, a, st)
                             : tc_hconv_launch(EPI_H2, p->S, KP, p->mapH1, a, st)))
       return rc;
     if (!chain) p->timer.end(st);
@@ -638,7 +673,7 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
       hgru::TcConvArgs a = base;
       a.wpk = p->wpk.as<__nv_bfloat16>(); a.out = p->C.as<float>();
       set_flags(a, 4 * t);
-      if ((rc = stack_launch(EPI_PARTIAL, 1, false, KP, p->stack_T, p->mapA_lo, a, st))) return rc;
+      if ((rc = stack_launch(EPI_PARTIAL, 1, false, KP, p->stack_T, FMT_BF16, p->mapA_lo, a, st))) return rc;
       a = base;
       a.wpk = p->wpk.as<__nv_bfloat16>(); a.partial = p->C.as<float>();
       a.bias = p->vec(V_LBIAS); a.X = Xp; a.H2 = p->H2.as<float>(); a.v0 = p->vec(V_BETA); a.v1 = p->vec(V_NU);
@@ -646,7 +681,7 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
       a.gate_wpk = p->wpk_o.as<__nv_bfloat16>(); a.gate_bias = p->vec(V_OB); a.gate_out = p->G.as<float>();
       a.do_gate = fused_gate ? 1 : 0;
       set_flags(a, 4 * t + 1);
-      if ((rc = stack_launch(EPI_H1, 2, true, KP, p->stack_T, p->mapA, a, st))) return rc;
+      if ((rc = stack_launch(EPI_H1, 2, true, KP, p->stack_T, FMT_BF16, p->mapA, a, st))) return rc;
       if (!chain) p->timer.end(st);
       if (!fused_gate) {
         // circuit_output gate (:729-740): G2 = sigmoid(H1 *1x1 o_r + o_b), exact fp32
@@ -660,7 +695,7 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
       a = base;
       a.wpk = p->wpk.as<__nv_bfloat16>(); a.out = p->C.as<float>();
       set_flags(a, 4 * t + 2);
-      if ((rc = stack_launch(EPI_PARTIAL, 1, false, KP, p->stack_T, p->mapH1_lo, a, st))) return rc;
+      if ((rc = stack_launch(EPI_PARTIAL, 1, false, KP, p->stack_T, FMT_BF16, p->mapH1_lo, a, st))) return rc;
       a = base;
       a.wpk = p->wpk.as<__nv_bfloat16>(); a.partial = p->C.as<float>();
       a.bias = p->vec(V_LBIAS); a.H1 = p->H1.as<float>(); a.G = p->G.as<float>(); a.H2 = p->H2.as<float>();
@@ -673,7 +708,7 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
         a.fc_a = p->fc_a; a.fc_scale = p->fc_scale; a.fc_shift = p->fc_shift; a.fc_kpad = p->fc_kpad;
       }
       set_flags(a, 4 * t + 3);
-      if ((rc = stack_launch(EPI_H2, 2, true, KP, p->stack_T, p->mapH1, a, st))) return rc;
+      if ((rc = stack_launch(EPI_H2, 2, true, KP, p->stack_T, FMT_BF16, p->mapH1, a, st))) return rc;
       if (!chain) p->timer.end(st);
       else if (t + 1 == p->T) p->timer.end(st, 2 * p->T);      // chained: one interval, counted as 2T convs
       p->launches += 4;
@@ -754,7 +789,7 @@ static int hgru_run_padded(hgru_plan_s* p, const float* Xp, const float* H2_init
   p->launches = 0;
   p->timer.reset();
   int rc;
-  if (p->mode == HGRU_MODE_BF16) {
+  if (p->op16()) {
     rc = hgru_run_bf16(p, Xp, H2_init_nhwc, H1_trace, H2_trace, st);
   } else if (p->mode == HGRU_MODE_BF16X3) {
     rc = hgru_run_bf16x3(p, Xp, H2_init_nhwc, H1_trace, H2_trace, st);
@@ -830,7 +865,7 @@ static int pose_forward_impl(pose_plan_s* p, const float* depth, const float* H2
   if (p->h0_identity && !p->h0_tmp.p) {
     if (int r = p->h0_tmp.alloc(static_cast<size_t>(N) * HW * HW * C * sizeof(float))) return r;
   }
-  if (p->mode == HGRU_MODE_BF16 && !p->h0_identity) {
+  if (h->op16() && !p->h0_identity) {
     // the hGRU's initial-state pass does not depend on the crops: run it first (under their upload, when the
     // caller copies them on another stream)
     // ... and beside the stem: both are latency-bound passes of ~0.1 ms that leave most of the chip idle
@@ -899,7 +934,7 @@ static int pose_forward_impl(pose_plan_s* p, const float* depth, const float* H2
     state_to_nhwc(h, h->Xp.as<float>(), p->h0_tmp.as<float>(), st);
     H2_init = p->h0_tmp.as<float>();
     ++p->launches;
-  } else if (p->mode == HGRU_MODE_BF16) {
+  } else if (h->op16()) {
     CUDA_TRY(cudaStreamWaitEvent(st, p->ev_init, 0));      // join the initial-state pass
   }
   if ((rc = hgru_run_padded(h, h->Xp.as<float>(), H2_init, nullptr, nullptr, st))) return rc;

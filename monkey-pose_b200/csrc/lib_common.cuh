@@ -69,15 +69,18 @@ struct StackGeom { int T, KC, NG, ksteps, box_cols, box_rows, stages, act_pad; }
 bool stack_geometry(int S, int KP, int k, StackGeom* g);
 
 // ---- launchers (one translation unit per kernel family) ----
+// format of the hGRU convs' 16-bit operands and weights (hgru::OpBf16 / hgru::OpFp16): bf16 mode / fp16 mode
+enum OpFormat { FMT_BF16 = 0, FMT_FP16 = 1 };
 enum EpiKind { EPI_H1 = 0, EPI_H2 = 1, EPI_H1_HALF = 2, EPI_H2_HALF = 3, EPI_PARTIAL = 4 };
-// hconv_stack_kernel<..., Epi, WSETS, PART>: tap-stacked 15x15 conv (k <= 32)
-int stack_launch(EpiKind epi, int wsets, bool part, int KP, int T, const CUtensorMap& map, const hgru::TcConvArgs& a,
-                 cudaStream_t st);
-// its weight packing: HWIO fp32 -> the stacked (or remainder-packed) bf16 stage layout; lo_part = the bf16 remainder
-int stack_pack_weights(const float* p_r, __nv_bfloat16* dst, int k, const StackGeom& sg, int lo_part, cudaStream_t st);
+// hconv_stack_kernel<..., Epi, WSETS, PART>: tap-stacked 15x15 conv (k <= 32); FMT_FP16 exists for EPI_H*_HALF
+int stack_launch(EpiKind epi, int wsets, bool part, int KP, int T, OpFormat fmt, const CUtensorMap& map,
+                 const hgru::TcConvArgs& a, cudaStream_t st);
+// its weight packing: HWIO fp32 -> the stacked (or remainder-packed) 16-bit stage layout; lo_part = the remainder
+int stack_pack_weights(const float* p_r, __nv_bfloat16* dst, int k, const StackGeom& sg, int lo_part, OpFormat fmt,
+                       cudaStream_t st);
 // hconv_tc_kernel: plain (EPI_H1 / EPI_H2), FUSE at 64 channels (EPI_H1_HALF / EPI_H2_HALF), SPLIT3 stem, SPLIT3 x3
 int tc_hconv_launch(EpiKind epi, int S, int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
-int tc_fused64_launch(EpiKind epi, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
+int tc_fused64_launch(EpiKind epi, OpFormat fmt, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
 int tc_stem_launch(int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
 int tc_x3_launch(EpiKind epi, int S, int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
 

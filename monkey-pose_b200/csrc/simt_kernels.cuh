@@ -8,6 +8,8 @@
 
 #include <cstdint>
 
+#include "op_format.cuh"
+
 namespace hgru {
 
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.f / (1.f + __expf(-x)); }
@@ -816,10 +818,12 @@ __global__ void bn_fold_kernel(const float* gamma, const float* beta, const floa
   shift[i] = beta[i] - mean[i] * s;
 }
 
-// Weight packing for the tcgen05 conv: HWIO fp32 [S][S][k][k] -> bf16 [KSTEPS][taps][2][CO_PAD][8 ci]
+// Weight packing for the tcgen05 conv: HWIO fp32 [S][S][k][k] -> F [KSTEPS][taps][2][CO_PAD][8 ci]
+// (F: the 16-bit operand format, op_format.cuh).
 // `ci_wrap` > 0: input channel index wraps at ci_wrap (the operand carries hi and lo bf16 halves of the
 // same channels in consecutive chunk planes, both multiplied by the same weights).
-__global__ void pack_weights_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ wpk,
+template <class F = OpBf16>
+__global__ void pack_weights_kernel(const float* __restrict__ w, typename F::T* __restrict__ wpk,
                                     int taps, int k, int ksteps, int co_pad, int ci_wrap = 0) {
   const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
   const size_t total = static_cast<size_t>(ksteps) * taps * 2 * co_pad * 8;
@@ -834,14 +838,15 @@ __global__ void pack_weights_kernel(const float* __restrict__ w, __nv_bfloat16* 
   if (ci_wrap > 0 && ci >= ci_wrap) ci -= ci_wrap;
   float v = 0.f;
   if (ci < k && co < k) v = w[(static_cast<size_t>(tap) * k + ci) * k + co];
-  wpk[i] = __float2bfloat16(v);
+  wpk[i] = F::cvt(v);
 }
 
 // Weight packing for the paired-tap schedule of the fused 64-channel 15x15 kernel (TcConvCfg::kPairTap):
-// HWIO fp32 [15][15][k][k] -> bf16 [kstep q][dy][block b = 0..7][2 chunks][128 rows][8 ci]
+// HWIO fp32 [15][15][k][k] -> F [kstep q][dy][block b = 0..7][2 chunks][128 rows][8 ci]
 //   block 0: rows 0-63 = tap dx = 7 (output channels), rows 64-127 = zero
 //   block 1 + p (p = 0..6): rows 0-63 = tap dx = p + 8, rows 64-127 = tap dx = p
-__global__ void pack_weights_pairtap_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ wpk, int k,
+template <class F = OpBf16>
+__global__ void pack_weights_pairtap_kernel(const float* __restrict__ w, typename F::T* __restrict__ wpk, int k,
                                             int ksteps) {
   const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
   const size_t total = static_cast<size_t>(ksteps) * 15 * 8 * 2 * 128 * 8;
@@ -860,7 +865,7 @@ __global__ void pack_weights_pairtap_kernel(const float* __restrict__ w, __nv_bf
   const int ci = q * 16 + ch * 8 + j;
   float v = 0.f;
   if (dx >= 0 && ci < k && co < k) v = w[((static_cast<size_t>(dy) * 15 + dx) * k + ci) * k + co];
-  wpk[i] = __float2bfloat16(v);
+  wpk[i] = F::cvt(v);
 }
 
 // Weight packing for the SPLIT3 tensor-core conv (hi = bf16(w), lo = bf16(w - hi)): per 16-channel group q

@@ -23,26 +23,26 @@ bool stack_geometry(int S, int KP, int k, StackGeom* g) {
   return true;
 }
 
-int stack_pack_weights(const float* p_r, __nv_bfloat16* dst, int k, const StackGeom& sg, int lo_part, cudaStream_t st) {
-  const size_t ts = static_cast<size_t>(sg.stages) * sg.NG * 2 * 128 * 8;
-  if (sg.act_pad)
-    hgru::pack_weights_stack_rem_kernel<<<nblk(ts), 256, 0, st>>>(p_r, dst, k, sg.T, sg.KC, sg.NG, lo_part);
-  else
-    hgru::pack_weights_stack_kernel<<<nblk(ts), 256, 0, st>>>(p_r, dst, k, sg.ksteps, sg.T, sg.KC, sg.NG, 1, lo_part);
-  CUDA_TRY(cudaGetLastError());
-  return 0;
-}
-
 namespace {
 
-template <int KP, int T, int KC, class Epi, int WSETS = 1, bool PART = false>
+template <class F>
+void pack_stack(const float* p_r, __nv_bfloat16* dst, int k, const StackGeom& sg, int lo_part, cudaStream_t st) {
+  const size_t ts = static_cast<size_t>(sg.stages) * sg.NG * 2 * 128 * 8;
+  auto* o = reinterpret_cast<typename F::T*>(dst);
+  if (sg.act_pad)
+    hgru::pack_weights_stack_rem_kernel<F><<<nblk(ts), 256, 0, st>>>(p_r, o, k, sg.T, sg.KC, sg.NG, lo_part);
+  else
+    hgru::pack_weights_stack_kernel<F><<<nblk(ts), 256, 0, st>>>(p_r, o, k, sg.ksteps, sg.T, sg.KC, sg.NG, 1, lo_part);
+}
+
+template <int KP, int T, int KC, class Epi, int WSETS = 1, bool PART = false, class F = hgru::OpBf16>
 int launch_stack(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t st) {
   // The second launch of a bf16x3 conv (PART) is also the one whose epilogue issues the gate, on hi/lo splits (GX3)
   // -- except at 32 channels, where the two staging tiles do not fit next to a 3-stage weight ring: that
   // configuration keeps its gates in the exact SIMT kernel.
   constexpr bool GX3 = PART && !(KP == 32 && T == 4);
-  using Cfg = hgru::StackCfg<KP, T, KC, 1, GX3>;
-  auto kern = hgru::hconv_stack_kernel<KP, T, KC, 1, Epi, false, WSETS, PART, GX3>;
+  using Cfg = hgru::StackCfg<KP, T, KC, 1, GX3, F>;
+  auto kern = hgru::hconv_stack_kernel<KP, T, KC, 1, Epi, false, WSETS, PART, GX3, F>;
   SMEM_ATTR_ONCE(kern, Cfg::SMEM_BYTES);
   a.units_x = (a.W + 63) / 64;
   a.units_y = (a.H + hgru::kTileRows - 1) / hgru::kTileRows;
@@ -63,18 +63,33 @@ int launch_stack(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t st) {
   return 0;
 }
 
-template <class Epi, int WSETS = 1, bool PART = false>
+template <class Epi, int WSETS = 1, bool PART = false, class F = hgru::OpBf16>
 int dispatch_stack(int KP, int T, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st) {
-  if (KP == 32 && T == 5) return launch_stack<32, 5, 25, Epi, WSETS, PART>(map, a, st);
-  if (KP == 32 && T == 4) return launch_stack<32, 4, 32, Epi, WSETS, PART>(map, a, st);
-  if (KP == 16 && T == 8) return launch_stack<16, 8, 16, Epi, WSETS, PART>(map, a, st);
+  if (KP == 32 && T == 5) return launch_stack<32, 5, 25, Epi, WSETS, PART, F>(map, a, st);
+  if (KP == 32 && T == 4) return launch_stack<32, 4, 32, Epi, WSETS, PART, F>(map, a, st);
+  if (KP == 16 && T == 8) return launch_stack<16, 8, 16, Epi, WSETS, PART, F>(map, a, st);
   return fail(HGRU_E_UNSUPPORTED, "stacked conv: unsupported configuration");
 }
 
 }  // namespace
 
-int stack_launch(EpiKind epi, int wsets, bool part, int KP, int T, const CUtensorMap& map, const hgru::TcConvArgs& a,
-                 cudaStream_t st) {
+int stack_pack_weights(const float* p_r, __nv_bfloat16* dst, int k, const StackGeom& sg, int lo_part, OpFormat fmt,
+                       cudaStream_t st) {
+  if (fmt == FMT_FP16) pack_stack<hgru::OpFp16>(p_r, dst, k, sg, lo_part, st);
+  else pack_stack<hgru::OpBf16>(p_r, dst, k, sg, lo_part, st);
+  CUDA_TRY(cudaGetLastError());
+  return 0;
+}
+
+int stack_launch(EpiKind epi, int wsets, bool part, int KP, int T, OpFormat fmt, const CUtensorMap& map,
+                 const hgru::TcConvArgs& a, cudaStream_t st) {
+  if (fmt == FMT_FP16) {      // fp16 mode: the fused pipeline's two launches per timestep
+    if (!part && wsets == 1 && epi == EPI_H1_HALF)
+      return dispatch_stack<hgru::EpiH1hF16, 1, false, hgru::OpFp16>(KP, T, map, a, st);
+    if (!part && wsets == 1 && epi == EPI_H2_HALF)
+      return dispatch_stack<hgru::EpiH2hF16, 1, false, hgru::OpFp16>(KP, T, map, a, st);
+    return fail(HGRU_E_UNSUPPORTED, "stacked conv: no fp16 variant of this kernel");
+  }
   if (!part && wsets == 1) {
     switch (epi) {
       case EPI_H1_HALF: return dispatch_stack<hgru::EpiH1h>(KP, T, map, a, st);      // fused bf16 pipeline

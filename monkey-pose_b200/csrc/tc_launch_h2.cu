@@ -45,10 +45,10 @@ int dispatch_tc_hconv(int S, int KP, const CUtensorMap& map, const hgru::TcConvA
 // 64 channels, 15x15 (the reference's own width): the same kernel with the 1x1 gate convs issued from its epilogue
 // and the launches of a forward chained per frame (TcConvCfg FUSE) -- two launches per timestep.  Three weight
 // stages instead of four make room for the gate's staging tile and weights.
-template <class Epi, int G = 5, int WS = 3>
+template <class Epi, class F = hgru::OpBf16, int G = 5, int WS = 3>
 int launch_tc_fused64(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t st) {
   using Cfg = hgru::TcConvCfg<15, 4, 64, 4, G, WS, false, true>;
-  auto kern = hgru::hconv_tc_kernel<15, 4, 64, 4, G, WS, Epi, false, true>;
+  auto kern = hgru::hconv_tc_kernel<15, 4, 64, 4, G, WS, Epi, false, true, F>;
   SMEM_ATTR_ONCE(kern, Cfg::kSmemBytes);
   a.units_x = (a.W + 31) / 32;
   a.units_y = (a.H + hgru::kTileRows - 1) / hgru::kTileRows;
@@ -81,6 +81,7 @@ int dispatch_tc_hconv_x3(int S, int KP, const CUtensorMap& map, const hgru::TcCo
 int tc_launch_h2(int family, int S, int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st) {
   if (family == 0) return dispatch_tc_hconv<hgru::EpiH2>(S, KP, map, a, st);
   if (family == 1) return launch_tc_fused64<hgru::EpiH2h>(map, a, st);
+  if (family == 3) return launch_tc_fused64<hgru::EpiH2hF16, hgru::OpFp16>(map, a, st);      // fp16 mode
   return dispatch_tc_hconv_x3<hgru::EpiH2>(S, KP, map, a, st);
 }
 

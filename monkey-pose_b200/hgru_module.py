@@ -129,7 +129,14 @@ class ContextualCircuit(object):
 
         X: torch CUDA tensor [n,h,w,k] float32 (static batch, hgru_module.py:74).
         Non-reference keywords: `params` (dict of the `contextual_circuit/*` variables, by their
-        reference names), `hidden_state` (O_0, [n,h,w,k]), `compute_mode` ('fp32' | 'bf16' | 'bf16x3'), `seed`.
+        reference names), `hidden_state` (O_0, [n,h,w,k]), `compute_mode`, `seed`.
+        compute_mode (arithmetic of the 15x15 and 1x1 convolutions; state and integration math are fp32 in all):
+          'fp32'   SIMT, exact fp32;
+          'bf16'   tcgen05 tensor cores, bf16 operands (8 significand bits), fp32 accumulation;
+          'fp16'   the 'bf16' mode with fp16 operands (11 significand bits) at the same speed; S = 15, k <= 64 (else
+                   NotImplementedError); operands saturate at +-65504, so an initial state beyond that is clamped in
+                   the first timestep's gated operand;
+          'bf16x3' tcgen05 on bf16 hi/lo splits (three products), fp32-class accuracy; S = 15.
         """
         if not (torch.is_tensor(X) and X.dim() == 4):
             raise ValueError("X must be a 4-D torch tensor [n,h,w,k] (CUDA for build())")

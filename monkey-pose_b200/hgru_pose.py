@@ -87,8 +87,9 @@ class model(LayerOps):
         # ---- non-reference knobs (defaults reproduce the reference's shapes) ----
         self.channels = 64            # stem width = hGRU hidden channels k (hgru_pose.py:50,61,71)
         self.fc_hidden = 1024         # hgru_pose.py:91
-        self.compute_mode = 'bf16'    # 'fp32' (SIMT, <=1e-4) | 'bf16' (tcgen05, <=1e-2) | 'bf16x3' (tcgen05 hi/lo
-        #                               splits, <=1e-4, 15x15 kernels)
+        self.compute_mode = 'bf16'    # 'fp32' (SIMT, <=1e-4) | 'bf16' (tcgen05, <=1e-2) | 'fp16' (tcgen05 fp16
+        #                               operands, bf16 speed, <=2.5e-3, 15x15 kernels) | 'bf16x3' (tcgen05 hi/lo
+        #                               splits, <=1e-4, 15x15 kernels); see ContextualCircuit
         self.hidden_state = None      # O_0 [N,64,64,k]; None -> seeded xavier-uniform draw
         self.seed = 42
         self.dropout_seed = 1234      # train_mode=True: seed of the counter-based dropout mask
