@@ -35,11 +35,11 @@ __global__ void fill_bf16(__nv_bfloat16* p, size_t n, float lo, float hi, unsign
 static int g_random_data = 0, g_check_layout = 0, g_audit_fail = 0;
 static float bf16r(float v) { return __bfloat162float(__float2bfloat16(v)); }
 
-template <int KP, int T, int KC, int CS>
+template <int KP, int T, int KC>
 int run_case(int N, int H, int W, int k, int grid_override, int iters) {
-  using Cfg = hgru::StackCfg<KP, T, KC, CS>;
+  using Cfg = hgru::StackCfg<KP, T, KC>;
   const int S = 15, CG = KP / 8;
-  printf("stack case KP=%d T=%d KC=%d CS=%d k=%d N=%d H=%d W=%d smem=%d cols=%d\n", KP, T, KC, CS, k, N, H, W, Cfg::SMEM_BYTES, Cfg::COLS);
+  printf("stack case KP=%d T=%d KC=%d k=%d N=%d H=%d W=%d smem=%d cols=%d\n", KP, T, KC, k, N, H, W, Cfg::SMEM_BYTES, Cfg::COLS);
   size_t npix = (size_t)N * H * W;
   std::vector<float> in(npix * k), w((size_t)S * S * k * k), bias(KP, 0.f);
   srand(123);
@@ -67,25 +67,20 @@ int run_case(int N, int H, int W, int k, int grid_override, int iters) {
   CK(cudaMemcpy(d_act, act.data(), act.size() * 2, cudaMemcpyHostToDevice));
   CK(cudaMemset(d_out, 0xFF, npix * KP * 4));
   if (Cfg::REM) hgru::pack_weights_stack_rem_kernel<<<(unsigned)((wpk_elems + 255) / 256), 256>>>(d_w, d_wpk, k, T, KC, Cfg::NG);
-  else hgru::pack_weights_stack_kernel<<<(unsigned)((wpk_elems + 255) / 256), 256>>>(d_w, d_wpk, k, Cfg::KSTEPS, T, KC, Cfg::NG, CS);
+  else hgru::pack_weights_stack_kernel<<<(unsigned)((wpk_elems + 255) / 256), 256>>>(d_w, d_wpk, k, Cfg::KSTEPS, T, KC, Cfg::NG);
   CK(cudaDeviceSynchronize());
   CUtensorMap map;
   if (hgru::make_act_tensor_map(&map, d_act, N, CG, HA, W, Cfg::COLS, Cfg::ROWS, Cfg::PART_CHUNKS)) { printf("map fail\n"); return 1; }
-  CUtensorMap wmap;
-  if (hgru::make_rows256_map(&wmap, d_wpk, wpk_elems * 2, Cfg::STAGE_ROWS)) { printf("wmap fail\n"); return 1; }
   hgru::TcConvArgs a{};
   a.N = N; a.H = H; a.W = W; a.KP = KP; a.kreal = k; a.act_pad = PADR;
   a.units_x = (W + 63) / 64; a.units_y = (H + 15) / 16; a.num_units = N * a.units_x * a.units_y;
   a.wpk = d_wpk; a.bias = d_bias; a.out = d_out;
-  auto kern = hgru::hconv_stack_kernel<KP, T, KC, CS, hgru::EpiBias>;
+  auto kern = hgru::hconv_stack_kernel<KP, T, KC, hgru::EpiBias>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   int sms = 0; CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, 0));
-  int grid = grid_override > 0 ? grid_override : (a.num_units < sms ? a.num_units : sms);
-  grid = (grid + CS - 1) / CS * CS;
+  const int grid = grid_override > 0 ? grid_override : (a.num_units < sms ? a.num_units : sms);
   cudaLaunchConfig_t cfg{}; cfg.gridDim = dim3(grid); cfg.blockDim = dim3(Cfg::NTHREADS); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
-  cudaLaunchAttribute at[1]; at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = CS; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  cfg.attrs = at; cfg.numAttrs = 1;
-  CK(cudaLaunchKernelEx(&cfg, kern, map, wmap, a));
+  CK(cudaLaunchKernelEx(&cfg, kern, map, a));
   CK(cudaDeviceSynchronize());
   size_t total = npix * k;
   naive_conv<<<(unsigned)((total + 255) / 256), 256>>>(d_in, d_w, d_bias, d_ref, N, H, W, k, S);
@@ -109,15 +104,15 @@ int run_case(int N, int H, int W, int k, int grid_override, int iters) {
   if (iters > 0 && !bad && !nan) {
     long long* d_prof; CK(cudaMalloc(&d_prof, grid * 40 * sizeof(long long))); CK(cudaMemset(d_prof, 0, grid * 40 * sizeof(long long)));
     hgru::TcConvArgs ap = a; ap.prof = d_prof;
-    CK(cudaLaunchKernelEx(&cfg, kern, map, wmap, ap)); CK(cudaDeviceSynchronize());
+    CK(cudaLaunchKernelEx(&cfg, kern, map, ap)); CK(cudaDeviceSynchronize());
     std::vector<long long> pr(grid * 8); CK(cudaMemcpy(pr.data(), d_prof, grid * 8 * sizeof(long long), cudaMemcpyDeviceToHost));
     double av[6] = {0, 0, 0, 0, 0, 0}; for (int b = 0; b < grid; ++b) for (int i = 0; i < 6; ++i) av[i] += pr[b * 8 + i] / (double)grid;
     printf("  prof (avg cycles/CTA): mma_total=%.0f wait_win=%.0f wait_acc_empty=%.0f wait_w_full=%.0f | epi_total=%.0f epi_wait_acc_full=%.0f\n", av[0], av[1], av[2], av[3], av[4], av[5]);
     cudaFree(d_prof);
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
-    for (int i = 0; i < 2; ++i) cudaLaunchKernelEx(&cfg, kern, map, wmap, a);
+    for (int i = 0; i < 2; ++i) cudaLaunchKernelEx(&cfg, kern, map, a);
     cudaEventRecord(e0);
-    for (int i = 0; i < iters; ++i) cudaLaunchKernelEx(&cfg, kern, map, wmap, a);
+    for (int i = 0; i < iters; ++i) cudaLaunchKernelEx(&cfg, kern, map, a);
     cudaEventRecord(e1); CK(cudaDeviceSynchronize());
     float ms; cudaEventElapsedTime(&ms, e0, e1); ms /= iters;
     printf("  time %.3f ms -> %.1f TFLOP/s algorithmic\n", ms, 2.0 * npix * 225.0 * k * k / ms * 1e-9);
@@ -125,9 +120,9 @@ int run_case(int N, int H, int W, int k, int grid_override, int iters) {
   cudaFree(d_in); cudaFree(d_w); cudaFree(d_bias); cudaFree(d_ref); cudaFree(d_out); cudaFree(d_act); cudaFree(d_wpk);
   return (bad || nan) ? 1 : 0;
 }
-template <int KP, int T, int KC, int CS, class Epi>
+template <int KP, int T, int KC, class Epi>
 void time_real_epilogue(const char* name, int N, int H, int W, int k, int gate = 1, int dbg = 0) {
-  using Cfg = hgru::StackCfg<KP, T, KC, CS>;
+  using Cfg = hgru::StackCfg<KP, T, KC>;
   const int CG = KP / 8;
   size_t npix = (size_t)N * H * W;
   float *X, *H1, *G, *H2, *vec; __nv_bfloat16 *act, *actout, *wpk;
@@ -148,9 +143,8 @@ void time_real_epilogue(const char* name, int N, int H, int W, int k, int gate =
     fill_bf16<<<(unsigned)((wpk_elems + 255) / 256), 256>>>(wpk, wpk_elems, -0.05f, 0.05f, 7u);
     CK(cudaDeviceSynchronize());
   }
-  CUtensorMap map, wmap;
+  CUtensorMap map;
   hgru::make_act_tensor_map(&map, act, N, CG, HA, W, Cfg::COLS, Cfg::ROWS, Cfg::PART_CHUNKS);
-  hgru::make_rows256_map(&wmap, wpk, wpk_elems * 2, Cfg::STAGE_ROWS);
   hgru::TcConvArgs a{};
   a.N = N; a.H = H; a.W = W; a.KP = KP; a.kreal = k; a.act_pad = Cfg::ACT_PAD;
   a.units_x = (W + 63) / 64; a.units_y = (H + 15) / 16; a.num_units = N * a.units_x * a.units_y;
@@ -158,17 +152,15 @@ void time_real_epilogue(const char* name, int N, int H, int W, int k, int gate =
   a.X = X; a.H1 = H1; a.G = G; a.H2 = H2; a.out = H1; a.out_bf16 = actout;
   a.gate_wpk = wpk; a.gate_bias = vec; a.gate_out = G; a.gate_act_out = actout; a.do_gate = gate; a.dbg_flags = dbg;
   if (std::is_same<Epi, hgru::EpiH2>::value) a.out_bf16 = nullptr;   // fused pipeline: H2's operand copy comes from the gate
-  auto kern = hgru::hconv_stack_kernel<KP, T, KC, CS, Epi, false>;
-  auto kern_prof = hgru::hconv_stack_kernel<KP, T, KC, CS, Epi, true>;
+  auto kern = hgru::hconv_stack_kernel<KP, T, KC, Epi, false>;
+  auto kern_prof = hgru::hconv_stack_kernel<KP, T, KC, Epi, true>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   CK(cudaFuncSetAttribute(kern_prof, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   int grid = 148;
   cudaLaunchConfig_t cfg{}; cfg.gridDim = dim3(grid); cfg.blockDim = dim3(Cfg::NTHREADS); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
-  cudaLaunchAttribute at[1]; at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = CS; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  cfg.attrs = at; cfg.numAttrs = 1;
   long long* d_prof; CK(cudaMalloc(&d_prof, grid * 40 * sizeof(long long))); CK(cudaMemset(d_prof, 0, grid * 40 * sizeof(long long)));
   hgru::TcConvArgs ap = a; ap.prof = d_prof;
-  CK(cudaLaunchKernelEx(&cfg, kern_prof, map, wmap, ap)); CK(cudaDeviceSynchronize());
+  CK(cudaLaunchKernelEx(&cfg, kern_prof, map, ap)); CK(cudaDeviceSynchronize());
   std::vector<long long> pr(grid * 40); CK(cudaMemcpy(pr.data(), d_prof, grid * 40 * sizeof(long long), cudaMemcpyDeviceToHost));
   double av[6] = {0, 0, 0, 0, 0, 0}; int nl = 0;
   for (int b = 0; b < grid; ++b) { if (pr[b * 8]) ++nl; for (int i = 0; i < 6; ++i) av[i] += pr[b * 8 + i]; }
@@ -176,17 +168,17 @@ void time_real_epilogue(const char* name, int N, int H, int W, int k, int gate =
     printf("    max over CTAs: mma_total=%lld epi_total=%lld | mean CTA wall %.1f us -> SM clock %.3f GHz\n", mx, mxe, ns / nl * 1e-3, av[0] / ns); }
   cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
   cudaEventRecord(e0);
-  for (int i = 0; i < 20; ++i) cudaLaunchKernelEx(&cfg, kern, map, wmap, a);
+  for (int i = 0; i < 20; ++i) cudaLaunchKernelEx(&cfg, kern, map, a);
   cudaEventRecord(e1); CK(cudaDeviceSynchronize());
   float ms; cudaEventElapsedTime(&ms, e0, e1); ms /= 20;
   { // the same PROF launch again, right behind 40 more back-to-back launches: clock under sustained load
-    for (int i = 0; i < 40; ++i) cudaLaunchKernelEx(&cfg, kern, map, wmap, a);
+    for (int i = 0; i < 40; ++i) cudaLaunchKernelEx(&cfg, kern, map, a);
     CK(cudaMemset(d_prof, 0, grid * 40 * sizeof(long long)));
-    CK(cudaLaunchKernelEx(&cfg, kern_prof, map, wmap, ap)); CK(cudaDeviceSynchronize());
+    CK(cudaLaunchKernelEx(&cfg, kern_prof, map, ap)); CK(cudaDeviceSynchronize());
     std::vector<long long> p2(grid * 8); CK(cudaMemcpy(p2.data(), d_prof, grid * 8 * sizeof(long long), cudaMemcpyDeviceToHost));
     double cyc = 0, ns = 0; long long mx = 0; for (int b = 0; b < grid; ++b) { cyc += p2[b * 8]; ns += p2[b * 8 + 6]; if (p2[b * 8] > mx) mx = p2[b * 8]; }
     printf("    sustained: mma_total avg %.0f max %lld cycles, mean CTA wall %.1f us -> SM clock %.3f GHz\n", cyc / grid, mx, ns / grid * 1e-3, cyc / ns); }
-  printf("%s gate=%d CS=%d: %.3f ms | leader avg cycles: mma_total=%.0f wait_win=%.0f wait_acc_empty=%.0f wait_w=%.0f | epi_total=%.0f epi_wait=%.0f\n", name, gate, CS, ms,
+  printf("%s gate=%d: %.3f ms | avg cycles: mma_total=%.0f wait_win=%.0f wait_acc_empty=%.0f wait_w=%.0f | epi_total=%.0f epi_wait=%.0f\n", name, gate, ms,
          av[0] / nl, av[1] / nl, av[2] / nl, av[3] / nl, av[4] / grid, av[5] / grid);
   if (g_check_layout) {
     // Bounds / layout audit of the operand tensor the epilogue wrote (stands in for a memory checker):
@@ -225,49 +217,43 @@ void time_real_epilogue(const char* name, int N, int H, int W, int k, int gate =
 
 int main(int argc, char** argv) {
   int which = argc > 1 ? atoi(argv[1]) : 0, f = 0;
-  if (which == 0 || which == 1) f += run_case<32, 5, 25, 1>(2, 64, 64, 25, 0, 0);
-  if (which == 0 || which == 2) f += run_case<32, 5, 25, 1>(3, 64, 64, 25, 5, 0);      // several units per CTA, idle tail
-  if (which == 0 || which == 3) f += run_case<32, 5, 25, 1>(2, 40, 24, 20, 0, 0);      // ragged, k < KC
-  if (which == 0 || which == 4) f += run_case<32, 4, 32, 1>(2, 64, 64, 32, 0, 0);
-  if (which == 0 || which == 5) f += run_case<16, 8, 16, 1>(2, 32, 48, 16, 0, 0);
-  if (which == 0 || which == 6) f += run_case<32, 5, 25, 2>(3, 64, 64, 25, 6, 0);      // cluster of 2, multicast
-  if (which == 0 || which == 7) f += run_case<32, 5, 25, 1>(256, 64, 64, 25, 0, 5);
-  if (which == 0 || which == 8) f += run_case<32, 5, 25, 2>(256, 64, 64, 25, 0, 5);
-  if (which == 0 || which == 9) f += run_case<32, 4, 32, 2>(256, 64, 64, 32, 0, 5);
+  if (which == 0 || which == 1) f += run_case<32, 5, 25>(2, 64, 64, 25, 0, 0);
+  if (which == 0 || which == 2) f += run_case<32, 5, 25>(3, 64, 64, 25, 5, 0);      // several units per CTA, idle tail
+  if (which == 0 || which == 3) f += run_case<32, 5, 25>(2, 40, 24, 20, 0, 0);      // ragged, k < KC
+  if (which == 0 || which == 4) f += run_case<32, 4, 32>(2, 64, 64, 32, 0, 0);
+  if (which == 0 || which == 5) f += run_case<16, 8, 16>(2, 32, 48, 16, 0, 0);
+  if (which == 0 || which == 7) f += run_case<32, 5, 25>(256, 64, 64, 25, 0, 5);
   if (which == 21) {   // weight ring refills on / off (dbg bit 0), random operand data: what the L2 -> SM weight stream costs
     g_random_data = 1;
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiBias>("EpiBias", 256, 64, 64, 25, 0, 0);
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiBias>("EpiBias noWstream", 256, 64, 64, 25, 0, 1);
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 1, 0);
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiH2>("EpiH2 noWstream", 256, 64, 64, 25, 1, 1);
+    time_real_epilogue<32, 5, 25, hgru::EpiBias>("EpiBias", 256, 64, 64, 25, 0, 0);
+    time_real_epilogue<32, 5, 25, hgru::EpiBias>("EpiBias noWstream", 256, 64, 64, 25, 0, 1);
+    time_real_epilogue<32, 5, 25, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 1, 0);
+    time_real_epilogue<32, 5, 25, hgru::EpiH2>("EpiH2 noWstream", 256, 64, 64, 25, 1, 1);
     g_random_data = 0;
   }
   if (which == 23) {   // epilogue-written operand tensors: guard bands, zero padding, remainder-plane consistency
     g_random_data = 1; g_check_layout = 1;
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiH1>("EpiH1", 256, 64, 64, 25, 1);
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 1);
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiH2>("EpiH2 ragged", 37, 40, 24, 25, 1);
-    time_real_epilogue<32, 4, 32, 1, hgru::EpiH2>("EpiH2 k32", 64, 64, 64, 32, 1);
+    time_real_epilogue<32, 5, 25, hgru::EpiH1>("EpiH1", 256, 64, 64, 25, 1);
+    time_real_epilogue<32, 5, 25, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 1);
+    time_real_epilogue<32, 5, 25, hgru::EpiH2>("EpiH2 ragged", 37, 40, 24, 25, 1);
+    time_real_epilogue<32, 4, 32, hgru::EpiH2>("EpiH2 k32", 64, 64, 64, 32, 1);
     g_random_data = 0; g_check_layout = 0; f += g_audit_fail;
   }
   if (which == 22) {
     for (g_random_data = 0; g_random_data < 2; ++g_random_data) {
       printf("---- %s data\n", g_random_data ? "random" : "zero");
-      time_real_epilogue<32, 5, 25, 1, hgru::EpiBias>("EpiBias", 256, 64, 64, 25, 0);
-      time_real_epilogue<32, 5, 25, 1, hgru::EpiH1>("EpiH1", 256, 64, 64, 25, 1);
-      time_real_epilogue<32, 5, 25, 1, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 1);
+      time_real_epilogue<32, 5, 25, hgru::EpiBias>("EpiBias", 256, 64, 64, 25, 0);
+      time_real_epilogue<32, 5, 25, hgru::EpiH1>("EpiH1", 256, 64, 64, 25, 1);
+      time_real_epilogue<32, 5, 25, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 1);
     }
   }
-  if (which == 20) {   // single CTA (remainder-packed, 24 stages) vs cta_group::2 pair mode (plain schedule, 30 stages), random data
+  if (which == 20) {   // each epilogue with and without its fused gate, random data
     g_random_data = 1;
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiBias>("EpiBias", 256, 64, 64, 25, 0);
-    time_real_epilogue<32, 5, 25, 2, hgru::EpiBias>("EpiBias", 256, 64, 64, 25, 0);
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiH1>("EpiH1", 256, 64, 64, 25, 0);
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiH1>("EpiH1", 256, 64, 64, 25, 1);
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 0);
-    time_real_epilogue<32, 5, 25, 1, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 1);
-    time_real_epilogue<32, 5, 25, 2, hgru::EpiH1>("EpiH1", 256, 64, 64, 25, 1);
-    time_real_epilogue<32, 5, 25, 2, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 1);
+    time_real_epilogue<32, 5, 25, hgru::EpiBias>("EpiBias", 256, 64, 64, 25, 0);
+    time_real_epilogue<32, 5, 25, hgru::EpiH1>("EpiH1", 256, 64, 64, 25, 0);
+    time_real_epilogue<32, 5, 25, hgru::EpiH1>("EpiH1", 256, 64, 64, 25, 1);
+    time_real_epilogue<32, 5, 25, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 0);
+    time_real_epilogue<32, 5, 25, hgru::EpiH2>("EpiH2", 256, 64, 64, 25, 1);
   }
   printf(f ? "FAILED %d\n" : "ALL OK\n", f);
   return f;

@@ -26,15 +26,6 @@
 // programmatic dependent launch, its CTAs taking SMs as this launch's CTAs exit -- waits per frame
 // (wait_flags) in its window producer and epilogue warps.
 //
-// CS = 2 ("pair mode", cta_group::2): two CTAs on one TPC run in lockstep on two units; the leader
-// issues M = 256 MMAs whose A rows come half from each CTA's own window and whose B rows come half
-// from each CTA's weight ring, so every CTA stores, streams and reads only half of the weights.
-// (Measured: worth 0-3 % on equal schedules and not combined with the remainder-packed schedule, so CS = 1 is
-// what runs; DESIGN.md section 4, item 12.)  All pair synchronisation
-// converges on the leader's barriers: both CTAs' TMA loads complete their bytes there
-// (cp.async.bulk.tensor ... cta_group::2), the peer's epilogue threads arrive there remotely, and
-// the leader's commits are multicast back to both CTAs.
-//
 // Warps: w0 weight producer, w1 MMA issuer, w2 TMEM alloc, w3 window producer, w4.. epilogue warpgroups.
 #pragma once
 #include <cuda_bf16.h>
@@ -48,9 +39,9 @@ namespace hgru {
 // GX3: the epilogue-issued 1x1 gate conv runs on bf16 hi/lo splits too (bf16x3 mode): staging tiles for both halves
 // of the new state, gate weights as [w_hi | w_lo] stacked along N plus w_hi (the SPLIT3 packing of hconv_tc.cuh).
 // F_: format of the 16-bit operands, window, weights and gate staging tile (op_format.cuh).
-template <int KP_, int T_, int KC_, int CS_, bool GX3_ = false, class F_ = OpBf16>
+template <int KP_, int T_, int KC_, bool GX3_ = false, class F_ = OpBf16>
 struct StackCfg {
-  static constexpr int KP = KP_, T = T_, KC = KC_, CS = CS_;
+  static constexpr int KP = KP_, T = T_, KC = KC_;
   static constexpr bool GX3 = GX3_;
   using Fmt = F_;
   static constexpr int S = 15, PAD = 7;
@@ -79,9 +70,8 @@ struct StackCfg {
 #endif
   static constexpr int NEPI = 128 * NGRP;                 // epilogue threads
   static constexpr int NTHREADS = 128 + NEPI;             // 4 service warps + NGRP x 4 epilogue warps
-  static constexpr int NLOC = NPAD / CS;                  // B rows held by one CTA
-  static constexpr int BLK_BYTES = 2 * NLOC * 16;         // one CTA's part of a (dy, q, g) weight block
-  static constexpr int STAGE_BYTES = NG * BLK_BYTES;      // all tap groups of one (dy, q), per CTA
+  static constexpr int BLK_BYTES = 2 * NPAD * 16;         // one (dy, q, g) weight block
+  static constexpr int STAGE_BYTES = NG * BLK_BYTES;      // all tap groups of one (dy, q)
   // Remainder packing (k = 25 = 3 full 8-channel chunks + ONE channel): instead of padding K to 32 for every
   // filter row, the last channel is stored as a plane whose 8 "channels" are that channel at 8 consecutive
   // rows, P[y][x][j] = in[y + j][x][c = 24] (written that way by the producing epilogues, 7 pad rows on top).
@@ -90,7 +80,7 @@ struct StackCfg {
 #ifdef HGRU_STACK_NO_REM
   static constexpr bool REM = false;      // development switch: A/B against the plain K schedule
 #else
-  static constexpr bool REM = (CS == 1) && (KC == 25) && (KP == 32);
+  static constexpr bool REM = (KC == 25) && (KP == 32);
 #endif
   static constexpr int ACT_PAD = REM ? 7 : 0;             // zero rows on top of every operand chunk plane
   static constexpr int PASS_STAGES = REM ? (S + S / 2 + 2) : S * KSTEPS;   // weight stages per tile pair
@@ -98,7 +88,7 @@ struct StackCfg {
   static constexpr int GATE_A_BYTES = GATE_A_HALF * (GX3 ? 2 : 1);      // (GX3: hi tile, lo tile)
   static constexpr int GATE_W_BYTES = KSTEPS * 2 * KP * 16 * (GX3 ? 3 : 1);
   static constexpr int GATE_BYTES = GATE_A_BYTES + GATE_W_BYTES;
-  // ring depth: as deep as the 227 KB allow (pair mode: half-size stages)
+  // ring depth: as deep as the 227 KB allow
 #ifdef HGRU_STACK_WSTAGES
   static constexpr int WSTAGES = HGRU_STACK_WSTAGES;      // development switch
 #else
@@ -106,7 +96,7 @@ struct StackCfg {
   // MMA completion -> commit -> producer -> bulk copy, not bandwidth: it is the same with the refills disabled,
   // and a fifth stage at k = 25 cut it from 50K to 37K cycles per launch (profiles/r01_stack_kernel_v19_*.log).
   static constexpr int WFIT = (232448 - WIN_BYTES - GATE_BYTES - 2048) / STAGE_BYTES;
-  static constexpr int WSTAGES = (CS == 2) ? 8 : (WFIT > 6 ? 6 : (WFIT < 3 ? 3 : WFIT));
+  static constexpr int WSTAGES = WFIT > 6 ? 6 : (WFIT < 3 ? 3 : WFIT);
 #endif
   // The window is loaded in WPARTS parts with their own barriers.  With the remainder-packed schedule the first
   // 15 stages of a pass read chunk planes 0-1 only and the last 9 read planes 2-3 only, so the next unit's first
@@ -116,38 +106,31 @@ struct StackCfg {
   static constexpr int PART_BYTES = WIN_BYTES / WPARTS;
   static constexpr int NUM_BARS = 4 + 2 * WSTAGES + 8 + 1;
   static constexpr int PAR_FLOATS = 5 * KP + 4;           // bias, v0, v1, v2, gate_bias (KP each) + rho_t
-  static constexpr int STAGE_ROWS = STAGE_BYTES / 256;    // rows of the 256-byte weight view per stage
   static constexpr int SMEM_BYTES =
       WIN_BYTES + WSTAGES * STAGE_BYTES + GATE_BYTES + NUM_BARS * 8 + 32 + PAR_FLOATS * 4 + 1024;
   static_assert(T * KC <= NPAD, "stacked taps must fit N = 128");
   static_assert(KC <= KP && KP % 16 == 0, "channel padding");
   static_assert((CHUNK_PITCH >> 4) < 16384, "LBO range");
-  static_assert(CS == 1 || CS == 2, "single CTA or CTA pair");
-  static_assert(STAGE_BYTES % 256 == 0, "stage must be whole 256-byte rows");
   static_assert(2 * COLS <= 256, "TMA box limit");
   static_assert(!GX3 || Fmt::kIdescFmt == OpBf16::kIdescFmt, "hi/lo gate splits are bf16");
 };
 
-// Stacked weight packing: HWIO fp32 [15][15][k][k] -> F [dy][q][rank][g][2 chunks][128/CS n'][8 ci],
-// n = rank*(128/CS) + n' = s*KC + c  <->  tap dx = T*g + T-1-s, output channel c
-// (zero where dx >= 15 or c, ci >= k).  `rank` = which CTA of a pair holds that half of B.
+// Stacked weight packing: HWIO fp32 [15][15][k][k] -> F [dy][q][g][2 chunks][128 n][8 ci],
+// n = s*KC + c  <->  tap dx = T*g + T-1-s, output channel c (zero where dx >= 15 or c, ci >= k).
 // `lo_part` = 1 packs the remainder  F(w - F(w))  instead (second weight set of the bf16x3 mode).
 template <class F = OpBf16>
 __global__ void pack_weights_stack_kernel(const float* __restrict__ w, typename F::T* __restrict__ wpk,
-                                          int k, int ksteps, int T, int KC, int NG, int CS, int lo_part = 0) {
+                                          int k, int ksteps, int T, int KC, int NG, int lo_part = 0) {
   const size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x;
   const size_t total = static_cast<size_t>(15) * ksteps * NG * 2 * 128 * 8;
   if (i >= total) return;
-  const int nloc = 128 / CS;
   const int j = i & 7;
   size_t r = i >> 3;
-  const int np = r % nloc; r /= nloc;
+  const int n = r % 128; r /= 128;
   const int ch = r & 1; r >>= 1;
   const int g = r % NG; r /= NG;
-  const int rank = r % CS; r /= CS;
   const int q = r % ksteps;
   const int dy = r / ksteps;
-  const int n = rank * nloc + np;
   const int s = n / KC, c = n - s * KC;
   const int dx = T * g + T - 1 - s;
   const int ci = q * 16 + ch * 8 + j;
@@ -290,14 +273,12 @@ __device__ __forceinline__ void stack_mma_issuer(const TcConvArgs& a, uint32_t t
                                                  uint32_t bar_w_full, uint32_t bar_w_empty, uint32_t bar_acc_full,
                                                  uint32_t bar_acc_empty, int iters, int NT, int npairs) {
   using namespace sm100;
-  constexpr int CS = Cfg::CS, T = Cfg::T;
-  constexpr uint16_t kMask = static_cast<uint16_t>((1u << CS) - 1u);
-  (void)kMask;
+  constexpr int T = Cfg::T;
   const bool leader = elect_one();
   tmem_base = __shfl_sync(0xffffffffu, tmem_base, 0);      // read from shared memory: mark it warp-uniform
-  constexpr uint32_t idesc = make_idesc(Cfg::Fmt::kIdescFmt, 128 * CS, Cfg::NPAD);
+  constexpr uint32_t idesc = make_idesc(Cfg::Fmt::kIdescFmt, 128, Cfg::NPAD);
   const uint64_t adesc0 = make_smem_desc(win, Cfg::CHUNK_PITCH, Cfg::ROW_PITCH);
-  const uint64_t bdesc0 = make_smem_desc(w_buf, Cfg::NLOC * 16, 128);
+  const uint64_t bdesc0 = make_smem_desc(w_buf, Cfg::NPAD * 16, 128);
   uint32_t st = 0, ph = 0;
   bool w_ready = false;       // the current weight stage was already seen complete by the previous stage's probe
   uint32_t tc = 0;            // running tile counter: TMEM slot = tc & 3, use count = tc >> 2
@@ -310,13 +291,12 @@ __device__ __forceinline__ void stack_mma_issuer(const TcConvArgs& a, uint32_t t
   }
   for (int it = 0; it < iters; ++it) {
     const int u = it * static_cast<int>(gridDim.x) + static_cast<int>(blockIdx.x);
-    const bool valid = u < a.num_units;
-    if (CS == 1 && !valid) break;      // idle tail (a CTA pair keeps going: its members share the weight stream)
+    if (u >= a.num_units) break;      // idle tail
     // Left-most unit of an image row: tap group 0 of the carry tile reads window columns 0..7 = image columns
     // T-16 .. T-9 < 0, all zero-filled by TMA, so those MMAs add nothing and are not issued.
     const bool carry_zero = (u % a.units_x) == 0;
     if constexpr (PROF) t0 = clock64();
-    if (valid) mbar_wait_warp(bar_win_full, vit & 1);
+    mbar_wait_warp(bar_win_full, vit & 1);
     if constexpr (PROF) t_win += clock64() - t0;
     tc_fence_after();
     bool part1_ready = Cfg::WPARTS == 1;
@@ -353,18 +333,12 @@ __device__ __forceinline__ void stack_mma_issuer(const TcConvArgs& a, uint32_t t
             const uint64_t bdesc = bdesc_st + static_cast<uint64_t>((g * Cfg::BLK_BYTES) >> 4);
             const uint64_t adesc = adesc_st + static_cast<uint64_t>(T * g);
             const uint32_t accum = (!first || g != 0) ? 1u : 0u;
-            if constexpr (CS > 1) {
-              mma_bf16_ss_2cta(acc0, adesc, bdesc, idesc, accum);
-              if (two) mma_bf16_ss_2cta(acc1, adesc + 8, bdesc, idesc, accum);
-            } else {
-              // (with g = 0 skipped, g = 1 of the first stage is the MMA that overwrites the accumulator)
-              if (!(skip0 && g == 0)) mma_bf16_ss(acc0, adesc, bdesc, idesc, (!first || g > (skip0 ? 1 : 0)) ? 1u : 0u);
-              if (two) mma_bf16_ss(acc1, adesc + 8, bdesc, idesc, accum);
-            }
+            // (with g = 0 skipped, g = 1 of the first stage is the MMA that overwrites the accumulator)
+            if (!(skip0 && g == 0)) mma_bf16_ss(acc0, adesc, bdesc, idesc, (!first || g > (skip0 ? 1 : 0)) ? 1u : 0u);
+            if (two) mma_bf16_ss(acc1, adesc + 8, bdesc, idesc, accum);
           }
           // release the weight stage when these MMAs have read it
-          if constexpr (CS > 1) tc_commit_2cta(bar_w_empty + 8 * st, kMask);
-          else tc_commit(bar_w_empty + 8 * st);
+          tc_commit(bar_w_empty + 8 * st);
         }
         w_ready = __all_sync(0xffffffffu, probe);
         if (++st == Cfg::WSTAGES) { st = 0; ph ^= 1; }
@@ -384,10 +358,10 @@ __device__ __forceinline__ void stack_mma_issuer(const TcConvArgs& a, uint32_t t
           for (int dy = 0; dy < Cfg::S; ++dy)
             issue_stage(a_tile0 + static_cast<uint64_t>((dy * RP) >> 4), (ws | dy) == 0);
           // chunk planes 0-1 are not read again by this unit: hand them to the window producer already
-          if (last_set && last_pass && leader && valid) tc_commit(bar_win_empty);
+          if (last_set && last_pass && leader) tc_commit(bar_win_empty);
           if (!part1_ready) {        // planes 2-3 of this unit were loading under the stages above
             if constexpr (PROF) t0 = clock64();
-            if (valid) mbar_wait_warp(bar_win_full + 8, vit & 1);
+            mbar_wait_warp(bar_win_full + 8, vit & 1);
             if constexpr (PROF) t_win += clock64() - t0;
             tc_fence_after();
             part1_ready = true;
@@ -395,7 +369,7 @@ __device__ __forceinline__ void stack_mma_issuer(const TcConvArgs& a, uint32_t t
           for (int i = 0; i < Cfg::S / 2; ++i) issue_stage(dB + static_cast<uint64_t>((2 * i * RP) >> 4), false);
           issue_stage(dC, false);
           issue_stage(dD, false);
-          if (last_set && last_pass && leader && valid) tc_commit(bar_win_empty + 8);
+          if (last_set && last_pass && leader) tc_commit(bar_win_empty + 8);
         }
       } else {
         // stage order: (weight set,) filter row dy, then k-step q
@@ -409,25 +383,16 @@ __device__ __forceinline__ void stack_mma_issuer(const TcConvArgs& a, uint32_t t
           }
       }
       if (leader) {
-        if constexpr (CS > 1) {
-          tc_commit_2cta(bar_acc_full + 8 * s0, kMask);
-          if (two) tc_commit_2cta(bar_acc_full + 8 * s1, kMask);
-        } else {
-          tc_commit(bar_acc_full + 8 * s0);
-          if (two) tc_commit(bar_acc_full + 8 * s1);
-        }
+        tc_commit(bar_acc_full + 8 * s0);
+        if (two) tc_commit(bar_acc_full + 8 * s1);
       }
       tc += two ? 2 : 1;
     }
-    // release the window (the two-part schedule released its parts inside the last pass): in pair mode both
-    // CTAs' windows were read by these MMAs
+    // release the window (the two-part schedule released its parts inside the last pass)
     if constexpr (Cfg::WPARTS == 1) {
-      if (leader && valid) {
-        if constexpr (CS > 1) tc_commit_2cta(bar_win_empty, kMask);
-        else tc_commit(bar_win_empty);
-      }
+      if (leader) tc_commit(bar_win_empty);
     }
-    if (valid) ++vit;
+    ++vit;
   }
   if (PROF && a.prof && leader) {
     long long* o = a.prof + static_cast<size_t>(blockIdx.x) * 8;
@@ -448,12 +413,12 @@ __device__ __forceinline__ void stack_mma_issuer(const TcConvArgs& a, uint32_t t
 // 31 % of the H2 kernel's samples, profiles/r02_ncu_source_stalls_stack_k25_v39_v40.txt).
 template <class Cfg, class Epi, int CN, bool PROF, bool PART = false>
 __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0, uint32_t tmem_base, uint32_t bar_acc_full,
-                                               uint32_t bar_acc_empty, uint32_t crank, int iters, int NT,
+                                               uint32_t bar_acc_empty, int iters, int NT,
                                                int units_per_frame, int warp, int lane, bool profile,
                                                uint8_t* smem_raw, uint32_t gate_a, uint32_t gate_w,
                                                uint32_t bar_gate) {
   using namespace sm100;
-  constexpr int KC = Cfg::KC, T = Cfg::T, CS = Cfg::CS, KP = Cfg::KP;
+  constexpr int KC = Cfg::KC, T = Cfg::T, KP = Cfg::KP;
   const bool gated = Epi::kGate && a.do_gate;
   uint32_t gate_uses = 0;
   constexpr int NCH = (CN + 7) / 8 * 8;            // channels handed to the fused epilogue (8-aligned)
@@ -461,19 +426,17 @@ __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0
   const int m = ew * 32 + lane;
   const int prow = m >> 3, pcol = m & 7;
   uint32_t tc = 0;
-  const uint32_t lead_acc_empty = (CS > 1) ? mapa_cluster(bar_acc_empty, 0) : 0u;
   long long e_wait = 0, e_begin = 0, e0 = 0, e_tm = 0, e_fin = 0, e_gw = 0, e_gm = 0;
   if constexpr (PROF) e_begin = clock64();
   for (int it = 0; it < iters; ++it) {
     const int u = it * static_cast<int>(gridDim.x) + static_cast<int>(blockIdx.x);
-    const bool valid = u < a.num_units;
-    if (CS == 1 && !valid) break;      // idle tail: every role of a single CTA stops at the same iteration
+    if (u >= a.num_units) break;      // idle tail: every role of the CTA stops at the same iteration
     const int nl = u / units_per_frame;
     const int r = u - nl * units_per_frame;
     const int n = a.n0 + nl;
     const int uy = r / a.units_x, ux = r - uy * a.units_x;
     const int y = uy * kTileRows + prow;
-    if (a.wait_flags && valid) {
+    if (a.wait_flags) {
       // chained launch: this frame's tensors are ready once all its units finished in the previous launch
       if (lane == 0)
         while (ld_acquire_gpu(a.wait_flags + n) < a.flag_target) {}
@@ -487,7 +450,7 @@ __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0
       const uint32_t slot = tc & 3;
       // this thread's output pixel; its global inputs are fetched while the MMAs still run
       const int x = ux * 64 + 8 * (j - 1) + pcol;
-      const bool store = valid && j >= 1 && y < a.H && x < a.W;
+      const bool store = j >= 1 && y < a.H && x < a.W;
       const size_t pin = static_cast<size_t>(y) * a.W + x;
       typename Epi::template Pre<NCH> pre;
       if (store) Epi::template load<NCH, CN>(a, n, pin, C0, pre);
@@ -556,9 +519,7 @@ __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0
       const bool gate_follows = gated && j >= 1;
       if (!gate_follows) {
         tc_fence_before();
-        // accumulator drained: MMAs may reuse it (pair mode: the leader's barrier counts both CTAs)
-        if (CS > 1 && crank != 0) mbar_arrive_cluster(lead_acc_empty + 8 * slot);
-        else mbar_arrive(bar_acc_empty + 8 * slot);
+        mbar_arrive(bar_acc_empty + 8 * slot);      // accumulator drained: MMAs may reuse it
       }
       // the fused math + stores: ONE inlined copy serves both paths (the new state also stays in registers for the gate)
       float hv[NCH];
@@ -639,13 +600,12 @@ __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0
           }
         }
         tc_fence_before();
-        if (CS > 1 && crank != 0) mbar_arrive_cluster(lead_acc_empty + 8 * slot);
-        else mbar_arrive(bar_acc_empty + 8 * slot);
+        mbar_arrive(bar_acc_empty + 8 * slot);
         if (store) Epi::template gate<NCH, CN>(a, n, pin, C0, gacc, hv);
         if constexpr (PROF) { const long long t = clock64(); e_gm += t - e0; e0 = t; }
       }
     }
-    if (a.done_flags && valid) {
+    if (a.done_flags) {
       // all epilogue stores of this unit are issued: publish them, then count the unit as done
       asm volatile("bar.sync 2, %0;" ::"n"(Cfg::NEPI) : "memory");
       if (threadIdx.x == 128) {
@@ -667,13 +627,12 @@ __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0
 }
 
 // F: 16-bit operand format (op_format.cuh); Epi writes the next launch's operands in the same format.
-template <int KP, int T, int KC, int CS, class Epi, bool PROF = false, int WSETS = 1, bool PART = false,
-          bool GX3 = false, class F = OpBf16>
-__global__ void __launch_bounds__((StackCfg<KP, T, KC, CS, GX3, F>::NTHREADS), 1)
-hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ CUtensorMap w_map,
-                   const TcConvArgs a) {
+template <int KP, int T, int KC, class Epi, bool PROF = false, int WSETS = 1, bool PART = false, bool GX3 = false,
+          class F = OpBf16>
+__global__ void __launch_bounds__((StackCfg<KP, T, KC, GX3, F>::NTHREADS), 1)
+hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) {
   using namespace sm100;
-  using Cfg = StackCfg<KP, T, KC, CS, GX3, F>;
+  using Cfg = StackCfg<KP, T, KC, GX3, F>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t win = base;
@@ -696,7 +655,6 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
   // uniform branches and the MMA issuer's addresses can live in uniform registers
   const int warp = __shfl_sync(0xffffffffu, static_cast<int>(threadIdx.x >> 5), 0);
   const int lane = threadIdx.x & 31;
-  const uint32_t crank = (CS > 1) ? cluster_ctarank() : 0u;
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < 2; ++i) {
@@ -709,17 +667,13 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
     }
     for (int i = 0; i < 4; ++i) {
       mbar_init(bar_acc_full + 8 * i, 1);
-      mbar_init(bar_acc_empty + 8 * i, Cfg::NEPI * CS);     // all epilogue threads (pair mode: of both CTAs, at the leader)
+      mbar_init(bar_acc_empty + 8 * i, Cfg::NEPI);     // all epilogue threads
     }
     mbar_init(bar_gate, 1);
-    tma_prefetch_desc(&w_map);
     fence_barrier_init();
     tma_prefetch_desc(&in_map);
   }
-  if (warp == 2) {
-    if constexpr (CS > 1) tmem_alloc_2cta<512>(tmem_slot);
-    else tmem_alloc<512>(tmem_slot);
-  }
+  if (warp == 2) tmem_alloc<512>(tmem_slot);
   if (warp >= 4) {
     // Per-channel parameter vectors -> shared memory.  With ~220 KB of the SM's SRAM carved out as shared
     // memory the L1 is a few KB, so every per-tile __ldg of these vectors was an L2 round trip on the
@@ -741,12 +695,10 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
   }
   tc_fence_before();
   __syncthreads();
-  if constexpr (CS > 1) cluster_sync_all();     // peers' barriers exist before any remote arrive
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot_ptr;
   grid_launch_dependents();      // a chained next launch may take SMs as they free up (no effect otherwise)
 
-  // every CTA runs the same number of iterations (cluster members share the weight stream)
   const int iters = (a.num_units + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
   const int units_per_frame = a.units_x * a.units_y;
   const int wseg = a.W < 64 ? a.W : 64;
@@ -754,22 +706,16 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
   const int npairs = (NT + 1) / 2;
 
   if (warp == 0) {
-    // ---------------- weight producer: this CTA's share of every stage ----------------
+    // ---------------- weight producer ----------------
     if (lane == 0) {
       uint32_t st = 0, ph = 0;
       const uint8_t* wsrc = reinterpret_cast<const uint8_t*>(a.wpk);
-      const uint32_t lead_w_full = (CS > 1) ? mapa_cluster(bar_w_full, 0) : 0u;
       for (int it = 0; it < iters; ++it) {
-        if (CS == 1 && it * static_cast<int>(gridDim.x) + static_cast<int>(blockIdx.x) >= a.num_units) break;
+        if (it * static_cast<int>(gridDim.x) + static_cast<int>(blockIdx.x) >= a.num_units) break;
         for (int pr = 0; pr < npairs; ++pr)
           for (int sg = 0; sg < Cfg::PASS_STAGES * WSETS; ++sg) {
             mbar_wait(bar_w_empty + 8 * st, ph ^ 1);
-            if constexpr (CS > 1) {
-              // both halves complete their bytes on the leader's barrier
-              if (crank == 0) mbar_arrive_expect_tx(bar_w_full + 8 * st, 2 * Cfg::STAGE_BYTES);
-              tma_load_2d_2cta(w_buf + st * Cfg::STAGE_BYTES, &w_map, lead_w_full + 8 * st, 0,
-                               (sg * CS + static_cast<int>(crank)) * Cfg::STAGE_ROWS);
-            } else if ((a.dbg_flags & 1) && (it | pr | (sg >= Cfg::WSTAGES))) {
+            if ((a.dbg_flags & 1) && (it | pr | (sg >= Cfg::WSTAGES))) {
               mbar_arrive(bar_w_full + 8 * st);      // development: reuse the resident (stale) stage
             } else {
               mbar_arrive_expect_tx(bar_w_full + 8 * st, Cfg::STAGE_BYTES);
@@ -784,7 +730,6 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
     // ---------------- window producer: one TMA box per unit ----------------
     if (lane == 0) {
       int vit = 0;
-      const uint32_t lead_win_full = (CS > 1) ? mapa_cluster(bar_win_full, 0) : 0u;
       for (int it = 0; it < iters; ++it) {
         const int u = it * static_cast<int>(gridDim.x) + static_cast<int>(blockIdx.x);
         if (u >= a.num_units) continue;
@@ -797,28 +742,18 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
           fence_proxy_async_global();
         }
         mbar_wait(bar_win_empty, (vit & 1) ^ 1);
-        if constexpr (CS > 1) {
-          // the leader's barrier collects the bytes of both windows (the peer's unit is u + 1)
-          if (crank == 0)
-            mbar_arrive_expect_tx(bar_win_full, Cfg::WIN_BYTES * ((u + 1 < a.num_units) ? 2 : 1));
-          tma_load_4d_2cta(win, &in_map, lead_win_full, 2 * (ux * 64 + Cfg::MIN_COL),
-                           uy * kTileRows - Cfg::PAD + Cfg::ACT_PAD, 0, n);
-        } else {
-          mbar_arrive_expect_tx(bar_win_full, Cfg::PART_BYTES);
-          tma_load_4d(win, &in_map, bar_win_full, 2 * (ux * 64 + Cfg::MIN_COL),
-                      uy * kTileRows - Cfg::PAD + Cfg::ACT_PAD, 0, n);
-          if constexpr (Cfg::WPARTS == 2) {
-            mbar_wait(bar_win_empty + 8, (vit & 1) ^ 1);
-            mbar_arrive_expect_tx(bar_win_full + 8, Cfg::PART_BYTES);
-            tma_load_4d(win + Cfg::PART_BYTES, &in_map, bar_win_full + 8, 2 * (ux * 64 + Cfg::MIN_COL),
-                        uy * kTileRows - Cfg::PAD + Cfg::ACT_PAD, Cfg::PART_CHUNKS, n);
-          }
+        mbar_arrive_expect_tx(bar_win_full, Cfg::PART_BYTES);
+        tma_load_4d(win, &in_map, bar_win_full, 2 * (ux * 64 + Cfg::MIN_COL),
+                    uy * kTileRows - Cfg::PAD + Cfg::ACT_PAD, 0, n);
+        if constexpr (Cfg::WPARTS == 2) {
+          mbar_wait(bar_win_empty + 8, (vit & 1) ^ 1);
+          mbar_arrive_expect_tx(bar_win_full + 8, Cfg::PART_BYTES);
+          tma_load_4d(win + Cfg::PART_BYTES, &in_map, bar_win_full + 8, 2 * (ux * 64 + Cfg::MIN_COL),
+                      uy * kTileRows - Cfg::PAD + Cfg::ACT_PAD, Cfg::PART_CHUNKS, n);
         }
         ++vit;
       }
     }
-  } else if (warp == 1 && crank != 0) {
-    // peer CTA of a pair: its MMAs are issued by the leader
   } else if (warp == 1) {
     // ---------------- MMA issuer (convergent warp, one elected lane issues) ----------------
     const long long clk0 = a.clk_out ? clock64() : 0;
@@ -836,7 +771,7 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
     ae.rho_t = par + 5 * KP;
     // ---------------- epilogue: NGRP warpgroups, 8-channel chunks each, the last one takes the rest ----------
 #define HGRU_STACK_EPI(C0_, CN_)                                                                                 \
-  stack_epilogue<Cfg, Epi, CN_, PROF, PART>(ae, C0_, tmem_base, bar_acc_full, bar_acc_empty, crank, iters, NT,          \
+  stack_epilogue<Cfg, Epi, CN_, PROF, PART>(ae, C0_, tmem_base, bar_acc_full, bar_acc_empty, iters, NT,                 \
                                             units_per_frame, warp, lane, warp < 8, smem_raw, gate_a, gate_w, bar_gate)
     // all groups but the last take 8 channels and share one copy of the code
     constexpr int kLastGrp = Cfg::NGRP - 1;
@@ -848,11 +783,9 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_cons
 
   tc_fence_before();
   __syncthreads();
-  if constexpr (CS > 1) cluster_sync_all();     // no CTA exits while a peer may still signal it
   if (warp == 2) {
     tc_fence_after();
-    if constexpr (CS > 1) tmem_dealloc_2cta<512>(tmem_base);
-    else tmem_dealloc<512>(tmem_base);
+    tmem_dealloc<512>(tmem_base);
   }
 }
 

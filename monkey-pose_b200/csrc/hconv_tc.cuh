@@ -148,11 +148,9 @@ struct TcConvArgs {
   const int* wait_flags;
   int* done_flags;
   int flag_target;
-  // Frame groups: a launch covers frames [n0, n0 + N) of the tensors (N = frames of this launch; tensor strides do
-  // not depend on it).  `pdl` asks for a programmatic dependent launch although there is nothing to wait for (the
-  // first launch of a frame group follows the last launch of the previous, independent, group).
+  // A launch covers frames [n0, n0 + N) of the tensors (N = frames of this launch; tensor strides do not depend on
+  // it): the stem convs run chunk by chunk behind the upload of the crops.
   int n0;
-  int pdl;
   // Optional in-kernel SM clock measurement (nvidia-smi keeps reporting the nominal clock while the kernel runs at
   // its power-limited one): the MMA issuer of CTA b stores {clock64 cycles, %globaltimer nanoseconds} it spent in
   // its loop at clk_out[2b], clk_out[2b + 1].  nullptr = off.

@@ -178,7 +178,6 @@ struct hgru_plan_s {
   DevBuf flags;                     // launch chaining: [2T][N] per-frame completion counters (stacked kernel)
   DevBuf clk;                       // in-kernel clock samples of the last conv launch: [CTA][2] (cycles, ns)
   bool chain = false;
-  int group_frames = 0;             // chained launches walk the batch in groups of this many frames (0 = whole batch)
   CUtensorMap mapA, mapH1;          // SxS halo-window boxes (horizontal convs)
   CUtensorMap mapA_lo, mapH1_lo;    // bf16x3 on the stacked kernel: the lo halves are tensors of their own
   size_t lo_off = 0;                // ... lo_off elements behind the hi tensors
@@ -207,27 +206,14 @@ struct hgru_plan_s {
 
 enum { V_IB = 0, V_OB, V_BETA, V_NU, V_GAMMA, V_KAPPA, V_OMEGA, V_LBIAS };
 
-// development switch (environment variable set to 1)
-static bool dev_switch(const char* name) {
-  const char* e = getenv(name);
-  return e && e[0] == '1';
-}
-
 static int hgru_plan_init(hgru_plan_s* p, int N, int H, int W, int k, int S, int T, int mode) {
   if (N < 1 || H < 1 || W < 1 || k < 1 || T < 1) return fail(HGRU_E_INVALID, "hgru_plan_create: non-positive shape");
   if (S < 1 || (S % 2) == 0 || S > 15) return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: S must be odd and <= 15");
   if (mode != HGRU_MODE_FP32 && mode != HGRU_MODE_BF16 && mode != HGRU_MODE_BF16X3 && mode != HGRU_MODE_FP16)
     return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: unknown mode");
-  if (mode == HGRU_MODE_FP16) {
-    // fp16 operands exist for the 15x15 kernels only: tap-stacked (k <= 32) and fused paired-tap (k <= 64)
-    if (S != 15 || k > 64) return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: fp16 mode supports S = 15 and k <= 64");
-    // development switches that select a kernel without an fp16 variant
-    const bool wide = k > 32;
-    const char* sw = dev_switch("HGRU_SIMT_INIT") ? "HGRU_SIMT_INIT"
-                     : (wide && dev_switch("HGRU_NO_FUSE64")) ? "HGRU_NO_FUSE64"
-                     : (!wide && dev_switch("HGRU_FP32_HG")) ? "HGRU_FP32_HG" : nullptr;
-    if (sw) return fail(HGRU_E_UNSUPPORTED, std::string("hgru_plan_create: fp16 mode has no kernel for ") + sw + "=1");
-  }
+  // fp16 operands exist for the 15x15 kernels only: tap-stacked (k <= 32) and fused paired-tap (k <= 64)
+  if (mode == HGRU_MODE_FP16 && (S != 15 || k > 64))
+    return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: fp16 mode supports S = 15 and k <= 64");
   p->N = N; p->H = H; p->W = W; p->k = k; p->S = S; p->T = T; p->mode = mode;
   p->KP = round_up(k, 16);
   if (mode != HGRU_MODE_FP32 && p->KP == 48) p->KP = 64;      // tensor-core kernels exist for 16 / 32 / 64 padded channels
@@ -251,8 +237,7 @@ static int hgru_plan_init(hgru_plan_s* p, int N, int H, int W, int k, int S, int
       return rc;
   } else if (mode == HGRU_MODE_BF16X3) {
     StackGeom sg;
-    const char* ns = getenv("HGRU_X3_NO_STACK");      // development switch: the hconv_tc SPLIT3 kernel at every width
-    if (stack_geometry(S, p->KP, k, &sg) && !(ns && ns[0] == '1')) {
+    if (stack_geometry(S, p->KP, k, &sg)) {
       // Narrow layers: the tap-stacked kernel, two launches per conv.  The first reads the a_lo operand against w_hi
       // and leaves fp32 sums in C; the second reads a_hi against the weight sets w_hi and w_lo (accumulated in TMEM),
       // adds C and runs the integration epilogue -- the launch with the heavy epilogue is the one with twice the MMAs
@@ -308,20 +293,13 @@ static int hgru_plan_init(hgru_plan_s* p, int N, int H, int W, int k, int S, int
     p->stacked = stack_geometry(S, p->KP, k, &sg);
     int box_cols = g.box_cols, box_rows = g.box_rows, box_chunks = 2;
     size_t wbytes = tapb * S * S;
-    {
-      const char* nf = getenv("HGRU_NO_FUSE64");      // development switch: the unfused four-launch pipeline
-      p->fused_tc = !p->stacked && S == 15 && p->KP == 64 && !(nf && nf[0] == '1');
-    }
+    p->fused_tc = !p->stacked && S == 15 && p->KP == 64;
     if (p->fused_tc) wbytes = sizeof(__nv_bfloat16) * ksteps * 15 * 8 * 2 * 128 * 8;      // paired-tap blocks
     if (p->stacked || p->fused_tc) {
       // consecutive conv launches are chained through per-frame counters (HGRU_NO_CHAIN=1: plain stream order)
       const char* nc = getenv("HGRU_NO_CHAIN");
       p->chain = !(nc && nc[0] == '1');
       if (p->chain && (rc = p->flags.alloc(sizeof(int) * 2 * static_cast<size_t>(T) * N))) return rc;
-      // Group-major order (time-major inside a frame group): all 2T launches of one group of frames before the next
-      // group, so that a group's state (X, H1, H2, G2 and the two bf16 operands) can stay in L2 across timesteps.
-      const char* gf = getenv("HGRU_GROUP_FRAMES");
-      if (gf && p->chain) p->group_frames = atoi(gf);
     }
     if (p->stacked) {
       p->stack_T = sg.T;
@@ -493,24 +471,13 @@ static int launch_init_tc(int KP, const float* h0, const hgru::TcConvArgs& a, cu
 }
 
 static int hgru_init_state_bf16(hgru_plan_s* p, const float* H2_init_nhwc, cudaStream_t st) {
-  static const bool simt_init = [] { const char* e = getenv("HGRU_SIMT_INIT"); return e && e[0] == '1'; }();
-  if (!simt_init) {      // (development switch: HGRU_SIMT_INIT=1 runs the exact-fp32 SIMT gate below)
-    // tensor-core version: the 1x1 gate conv as one UMMA tile per 128 pixels (bf16 operands like every later gate)
-    hgru::TcConvArgs a{};
-    a.N = p->N; a.H = p->H; a.W = p->W; a.KP = p->KP; a.kreal = p->k; a.act_pad = p->act_pad;
-    a.wpk = p->wpk_i.as<__nv_bfloat16>(); a.bias = p->vec(V_IB); a.H2 = p->H2.as<float>();
-    a.out_bf16 = p->actA.as<__nv_bfloat16>();
-    return p->fmt() == FMT_FP16 ? launch_init_tc<hgru::OpFp16>(p->KP, H2_init_nhwc, a, st)
-                                : launch_init_tc<hgru::OpBf16>(p->KP, H2_init_nhwc, a, st);
-  }
-  SMEM_ATTR_ONCE(hgru::init_state_gate_kernel, 100 * 1024);
-  const int KP = p->KP;
-  const size_t smem = sizeof(float) * (KP * KP + hgru::kInitPix * (KP + 1));
-  hgru::init_state_gate_kernel<<<nblk(p->npix, hgru::kInitPix), 256, smem, st>>>(
-      H2_init_nhwc, p->i_r.as<float>(), p->vec(V_IB), p->H2.as<float>(), p->actA.as<__nv_bfloat16>(), p->npix,
-      p->k, KP, p->H * p->W, p->W, p->act_pad);
-  CUDA_TRY(cudaGetLastError());
-  return 0;
+  // the 1x1 gate conv as one UMMA tile per 128 pixels (16-bit operands like every later gate)
+  hgru::TcConvArgs a{};
+  a.N = p->N; a.H = p->H; a.W = p->W; a.KP = p->KP; a.kreal = p->k; a.act_pad = p->act_pad;
+  a.wpk = p->wpk_i.as<__nv_bfloat16>(); a.bias = p->vec(V_IB); a.H2 = p->H2.as<float>();
+  a.out_bf16 = p->actA.as<__nv_bfloat16>();
+  return p->fmt() == FMT_FP16 ? launch_init_tc<hgru::OpFp16>(p->KP, H2_init_nhwc, a, st)
+                              : launch_init_tc<hgru::OpBf16>(p->KP, H2_init_nhwc, a, st);
 }
 
 static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_nhwc, float* H1_trace,
@@ -528,7 +495,6 @@ static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_n
   const bool fused = p->stacked || p->fused_tc;
   // (a weight ring of 5 stages x 3 taps instead of 3 stages x 5 taps for the fused 64-channel kernel measured the
   // same: profiles/r02_bench_k64_fused_ring_5x3taps.json)
-  static const bool fp32_hg = [] { const char* e = getenv("HGRU_FP32_HG"); return e && e[0] == '1'; }();
   // Chained launches (see TcConvArgs::wait_flags): launch l waits per frame on launch l-1's counters instead of on
   // the whole grid.  Not with traces (their copy kernels sit between the launches).
   const bool chain = fused && p->chain && !H1_trace && !H2_trace;
@@ -540,11 +506,6 @@ static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_n
     a.wait_flags = l > 0 ? flags + static_cast<size_t>(l - 1) * p->N : nullptr;
   };
   if (chain) p->timer.begin(st);
-  const int GF = (chain && p->group_frames > 0 && p->group_frames < p->N) ? p->group_frames : p->N;
-  for (int n0 = 0; n0 < p->N; n0 += GF) {
-  base.n0 = n0;
-  base.N = (n0 + GF <= p->N) ? GF : p->N - n0;
-  const bool last_group = n0 + GF >= p->N;
   for (int t = 0; t < p->T; ++t) {
     hgru::TcConvArgs a;
     if (!fused && t > 0) {
@@ -564,11 +525,9 @@ static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_n
     a.gate_wpk = p->wpk_o.as<__nv_bfloat16>(); a.gate_bias = p->vec(V_OB); a.gate_out = p->G.as<float>();
     a.do_gate = fused ? 1 : 0;
     set_flags(a, 2 * t);
-    a.pdl = (chain && t == 0 && n0 > 0) ? 1 : 0;      // follows the previous group's last launch: nothing to wait for
     if (!chain) p->timer.begin(st);
-    // (fused pipeline: H1 and G2 travel to the H2 launch as fp16, EpiH1h / EpiH2h; development switch
-    // HGRU_FP32_HG=1: as fp32 on the stacked kernel, for A/B runs)
-    if ((rc = p->stacked    ? stack_launch(fp32_hg ? EPI_H1 : EPI_H1_HALF, 1, false, KP, p->stack_T, p->fmt(), p->mapA, a, st)
+    // (fused pipeline: H1 and G2 travel to the H2 launch as fp16, EpiH1h / EpiH2h)
+    if ((rc = p->stacked    ? stack_launch(EPI_H1_HALF, 1, false, KP, p->stack_T, p->fmt(), p->mapA, a, st)
               : p->fused_tc ? tc_fused64_launch(EPI_H1_HALF, p->fmt(), p->mapA, a, st)
                             : tc_hconv_launch(EPI_H1, p->S, KP, p->mapA, a, st)))
       return rc;
@@ -592,23 +551,23 @@ static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_n
     a.gate_wpk = p->wpk_i.as<__nv_bfloat16>(); a.gate_bias = p->vec(V_IB);
     a.gate_act_out = p->actA.as<__nv_bfloat16>();
     a.do_gate = (fused && t + 1 < p->T) ? 1 : 0;
-    if (g_timing && t + 1 == p->T && last_group) a.clk_out = p->clk.as<unsigned long long>();   // (grids are <= 1024 CTAs)
+    if (g_timing && t + 1 == p->T) a.clk_out = p->clk.as<unsigned long long>();   // (grids are <= 1024 CTAs)
     if (t + 1 == p->T && p->fc_a) {     // last update also emits the readout's bf16 hi/lo operand
       a.fc_a = p->fc_a; a.fc_scale = p->fc_scale; a.fc_shift = p->fc_shift; a.fc_kpad = p->fc_kpad;
     }
     set_flags(a, 2 * t + 1);
     if (!chain) p->timer.begin(st);
-    if ((rc = p->stacked    ? stack_launch(fp32_hg ? EPI_H2 : EPI_H2_HALF, 1, false, KP, p->stack_T, p->fmt(), p->mapH1, a, st)
+    if ((rc = p->stacked    ? stack_launch(EPI_H2_HALF, 1, false, KP, p->stack_T, p->fmt(), p->mapH1, a, st)
               : p->fused_tc ? tc_fused64_launch(EPI_H2_HALF, p->fmt(), p->mapH1, a, st)
                             : tc_hconv_launch(EPI_H2, p->S, KP, p->mapH1, a, st)))
       return rc;
     if (!chain) p->timer.end(st);
-    else if (t + 1 == p->T && last_group) p->timer.end(st, 2 * p->T);   // chained: one interval around all launches,
-    //                                                                     counted as 2T passes over the whole batch
+    else if (t + 1 == p->T) p->timer.end(st, 2 * p->T);   // chained: one interval around all launches,
+    //                                                       counted as 2T passes over the whole batch
     ++p->launches;
     if (H1_trace) {
       float* dst = H1_trace + static_cast<size_t>(t) * p->npix * p->k;
-      if (fused && !(p->stacked && fp32_hg))      // H1 is an fp16 oct-chunked tensor in the fused pipeline
+      if (fused)      // H1 is an fp16 oct-chunked tensor in the fused pipeline
         hgru::oct_half_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(p->H1.as<__half>(), dst, p->npix, p->k, KP, HW);
       else
         hgru::quad_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(p->H1.as<float>(), dst, p->npix, p->k, KP, HW);
@@ -619,7 +578,6 @@ static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_n
           p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix * p->k, p->npix, p->k, KP, HW);
       ++p->launches;
     }
-  }
   }
   return 0;
 }
@@ -1184,7 +1142,6 @@ int pose_forward_host(pose_plan_t p, const float* depth_host, const float* H2_in
   CUDA_TRY(cudaStreamWaitEvent(p->copy_st, p->ev_begin, 0));
   // frame chunks, one event each: conv_1 of chunk c runs while chunk c+1 is still on the bus
   int nchunks = p->N / pose_plan_s::kUploadChunkFrames;
-  if (const char* e = getenv("HGRU_UPLOAD_CHUNKS")) nchunks = atoi(e);      // development switch (A/B of the overlap)
   nchunks = nchunks < 1 ? 1 : (nchunks > pose_plan_s::kUploadChunks ? pose_plan_s::kUploadChunks : nchunks);
   {
     const int per = (p->N + nchunks - 1) / nchunks;

@@ -469,105 +469,12 @@ split_chunks_to_nhwc_kernel(const __nv_bfloat16* __restrict__ in, float* __restr
 }
 
 // ------------------------------------------------------------------------------------------------
-// Initial state of the tensor-core path in one pass: O_0 (NHWC, k channels; hgru_module.py:884-887)
-//   -> H2 fp32 quad-chunked (zero padded), and the first timestep's gated operand
-//   A = bf16(sigmoid(O_0 *1x1 i_r + i_b) . O_0)  (hgru_module.py:696-711) in the chunked layout.
-// Exact-fp32 SIMT version (block = 256 pixels, i_r in shared memory, thread = 4 pixels x 8 output channels); the
-// production path runs init_state_tc_kernel (gate_tc.cuh) instead -- this one stays behind HGRU_SIMT_INIT=1.
-// ------------------------------------------------------------------------------------------------
-constexpr int kInitPix = 256;     // pixels per block of init_state_gate_kernel (4 per thread)
-__global__ void __launch_bounds__(256)
-init_state_gate_kernel(const float* __restrict__ h0 /*[npix][k] or nullptr = zeros*/,
-                       const float* __restrict__ wg /*[KP][KP]*/, const float* __restrict__ bg,
-                       float* __restrict__ H2q, __nv_bfloat16* __restrict__ actA, size_t npix, int k, int KP,
-                       int HW, int W, int act_pad /* remainder-packed operand layout, see StackCfg::REM */) {
-  extern __shared__ float smem_f[];
-  float* wsm = smem_f;                 // [KP][KP]
-  float* xin = smem_f + KP * KP;       // [kInitPix][KP+1]
-  const int tid = threadIdx.x;
-  const int CG = KP >> 3;
-  const size_t p0 = blockIdx.x * static_cast<size_t>(kInitPix);
-  for (int e = tid; e < KP * KP; e += 256) wsm[e] = wg[e];
-  // the block's pixels are contiguous in h0 ([npix][k]): stream them in flat order, scatter into the padded rows
-  {
-    const size_t base = p0 * k;
-    const int lim = static_cast<int>((p0 + kInitPix < npix ? static_cast<size_t>(kInitPix) : npix - p0) * k);
-    // e / k by multiplication (exact for e < 2^16, k <= 64): an integer division per element made this
-    // load loop a third of the kernel's instructions
-    const unsigned magic = 0xFFFFFFFFu / static_cast<unsigned>(k) + 1u;
-    for (int e = tid; e < kInitPix * k; e += 256) {
-      const int pp = static_cast<int>(__umulhi(static_cast<unsigned>(e), magic)), c = e - pp * k;
-      xin[pp * (KP + 1) + c] = (h0 && e < lim) ? __ldg(h0 + base + e) : 0.f;
-    }
-    const int npad = KP - k;                                     // zero the pad channels
-    for (int pp = tid; pp < kInitPix; pp += 256)
-      for (int c = k; c < k + npad; ++c) xin[pp * (KP + 1) + c] = 0.f;
-  }
-  __syncthreads();
-  // thread = 4 pixels (pq, pq+64, pq+128, pq+192) x one chunk of 8 output channels: every weight read from
-  // shared memory feeds 4 pixels
-  const int pq = tid & 63;
-  for (int cg = tid >> 6; cg < CG; cg += 4) {
-    float acc[4][8];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-      for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
-    for (int ci = 0; ci < k; ++ci) {          // (the pad input channels are zero)
-      const float4 w0 = *reinterpret_cast<const float4*>(wsm + ci * KP + cg * 8);
-      const float4 w1 = *reinterpret_cast<const float4*>(wsm + ci * KP + cg * 8 + 4);
-      const float wv[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const float xv = xin[(pq + 64 * i) * (KP + 1) + ci];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(xv, wv[j], acc[i][j]);
-      }
-    }
-    float bgv[8];
-#pragma unroll
-    for (int j = 0; j < 8; ++j) bgv[j] = (cg * 8 + j < k) ? __ldg(bg + cg * 8 + j) : 0.f;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int pp = pq + 64 * i;
-      const size_t p = p0 + pp;
-      if (p >= npix) continue;
-      const size_t n = p / HW, pin = p - n * HW;
-      F8 hv, mv;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const int c = cg * 8 + j;
-        hv.v[j] = xin[pp * (KP + 1) + c];
-        mv.v[j] = (c < k) ? sigmoidf_(acc[i][j] + bgv[j]) * hv.v[j] : 0.f;
-      }
-      float* o = H2q + ((n * (KP >> 2) + 2 * cg) * HW + pin) * 4;
-      *reinterpret_cast<float4*>(o) = make_float4(hv.v[0], hv.v[1], hv.v[2], hv.v[3]);
-      *reinterpret_cast<float4*>(o + static_cast<size_t>(HW) * 4) = make_float4(hv.v[4], hv.v[5], hv.v[6], hv.v[7]);
-      if (act_pad == 0) {
-        st8_bf16(chunk_ptr(actA, static_cast<int>(n), cg, pin, HW, CG), mv);
-      } else {
-        const int plane = HW + act_pad * W;
-        const size_t pa = pin + static_cast<size_t>(act_pad) * W;
-        if (cg != CG - 1) {
-          st8_bf16(chunk_ptr(actA, static_cast<int>(n), cg, pa, plane, CG), mv);
-        } else {
-          // last chunk = row-packed plane of channel KP - 8: element j of the pixel j rows above
-          __nv_bfloat16* oa = chunk_ptr(actA, static_cast<int>(n), cg, pa, plane, CG);
-          const __nv_bfloat16 v = __float2bfloat16(mv.v[0]);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) oa[j - static_cast<ptrdiff_t>(j) * W * 8] = v;
-        }
-      }
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
 // Exact fp32 1x1 gate on the quad-chunked state layout (bf16x3 mode; hgru_module.py:696-711, 729-740):
 //   g = sigmoid(in *1x1 wg + bg);  out_g (quad fp32) = g              when out_g  != nullptr   (G2)
 //                                  out_act = bf16 hi | lo of g . in   when out_act != nullptr  (gated operand)
-// Same tiling as init_state_gate_kernel: 256 pixels per block, thread = 4 pixels x 8 output channels.
+// 256 pixels per block (i_r in shared memory), thread = 4 pixels x 8 output channels.
 // ------------------------------------------------------------------------------------------------
+constexpr int kInitPix = 256;     // pixels per block of gate_quad_split_kernel (4 per thread)
 // `lo_off` > 0: the operand goes to TWO tensors in the tap-stacked kernel's layout instead (hi at out_act, lo lo_off
 // elements behind it; `act_pad` zero rows on top of every chunk plane of width W, and with act_pad > 0 the last chunk
 // is the row-packed plane P[y][x][j] = v(y + j, x) of channel KP - 8: see StackCfg::REM in hconv_stack.cuh).

@@ -191,78 +191,4 @@ __device__ __forceinline__ void tmem_ld_wait() {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-// ---------------------------------------------------------------- CTA pairs (cta_group::2)
-template <uint32_t kCols>
-__device__ __forceinline__ void tmem_alloc_2cta(uint32_t slot_smem) {   // same warp id in both CTAs
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;"
-               ::"r"(slot_smem), "n"(kCols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-template <uint32_t kCols>
-__device__ __forceinline__ void tmem_dealloc_2cta(uint32_t taddr) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "n"(kCols)
-               : "memory");
-}
-// D[tmem of both CTAs] (+)= A * B with M = 256 over the CTA pair: each CTA supplies its own 128
-// rows of A and half of B's N rows from the same shared-memory offsets; issued by the leader CTA.
-__device__ __forceinline__ void mma_bf16_ss_2cta(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc,
-                                                 uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// commit of the pair's MMAs: arrives on the mbarrier at this offset in every CTA of `mask`
-__device__ __forceinline__ void tc_commit_2cta(uint32_t bar, uint16_t mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(bar), "h"(mask) : "memory");
-}
-// arrive on the mbarrier at the same shared-memory offset in another CTA of the cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t target_cta) {
-  asm volatile(
-      "{\n\t.reg .b32 ra;\n\t"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-      "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
-      ::"r"(bar), "r"(target_cta) : "memory");
-}
-// shared::cluster address of the same shared-memory offset in CTA `target_cta` of the cluster
-__device__ __forceinline__ uint32_t mapa_cluster(uint32_t saddr, uint32_t target_cta) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(target_cta));
-  return r;
-}
-// TMA loads issued by either CTA of a pair: data lands in the issuing CTA's shared memory, the
-// bytes are completed on an mbarrier given by its shared::cluster address (the leader's).
-__device__ __forceinline__ void tma_load_2d_2cta(uint32_t dst, const CUtensorMap* m, uint32_t bar_cluster,
-                                                 int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_2cta(uint32_t dst, const CUtensorMap* m, uint32_t bar_cluster,
-                                                 int c0, int c1, int c2, int c3) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes"
-      " [%0], [%1, {%3, %4, %5, %6}], [%2];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-      : "memory");
-}
-// arrive on an mbarrier given by its shared::cluster address
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar_cluster) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_cluster) : "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
 }  // namespace sm100

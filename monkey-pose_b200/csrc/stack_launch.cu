@@ -17,9 +17,9 @@ bool stack_geometry(int S, int KP, int k, StackGeom* g) {
   g->box_cols = 64 + g->T * (g->NG - 1) + 8;
   g->box_rows = hgru::kTileRows + 14;
   // KC = 25: remainder-packed K schedule (hgru::StackCfg::REM) -- 24 weight stages, 7 pad rows per plane
-  const bool rem = hgru::StackCfg<32, 5, 25, 1>::REM && g->KC == 25;
-  g->stages = rem ? hgru::StackCfg<32, 5, 25, 1>::PASS_STAGES : 15 * g->ksteps;
-  g->act_pad = rem ? hgru::StackCfg<32, 5, 25, 1>::ACT_PAD : 0;
+  const bool rem = hgru::StackCfg<32, 5, 25>::REM && g->KC == 25;
+  g->stages = rem ? hgru::StackCfg<32, 5, 25>::PASS_STAGES : 15 * g->ksteps;
+  g->act_pad = rem ? hgru::StackCfg<32, 5, 25>::ACT_PAD : 0;
   return true;
 }
 
@@ -32,7 +32,7 @@ void pack_stack(const float* p_r, __nv_bfloat16* dst, int k, const StackGeom& sg
   if (sg.act_pad)
     hgru::pack_weights_stack_rem_kernel<F><<<nblk(ts), 256, 0, st>>>(p_r, o, k, sg.T, sg.KC, sg.NG, lo_part);
   else
-    hgru::pack_weights_stack_kernel<F><<<nblk(ts), 256, 0, st>>>(p_r, o, k, sg.ksteps, sg.T, sg.KC, sg.NG, 1, lo_part);
+    hgru::pack_weights_stack_kernel<F><<<nblk(ts), 256, 0, st>>>(p_r, o, k, sg.ksteps, sg.T, sg.KC, sg.NG, lo_part);
 }
 
 template <int KP, int T, int KC, class Epi, int WSETS = 1, bool PART = false, class F = hgru::OpBf16>
@@ -41,8 +41,8 @@ int launch_stack(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t st) {
   // -- except at 32 channels, where the two staging tiles do not fit next to a 3-stage weight ring: that
   // configuration keeps its gates in the exact SIMT kernel.
   constexpr bool GX3 = PART && !(KP == 32 && T == 4);
-  using Cfg = hgru::StackCfg<KP, T, KC, 1, GX3, F>;
-  auto kern = hgru::hconv_stack_kernel<KP, T, KC, 1, Epi, false, WSETS, PART, GX3, F>;
+  using Cfg = hgru::StackCfg<KP, T, KC, GX3, F>;
+  auto kern = hgru::hconv_stack_kernel<KP, T, KC, Epi, false, WSETS, PART, GX3, F>;
   SMEM_ATTR_ONCE(kern, Cfg::SMEM_BYTES);
   a.units_x = (a.W + 63) / 64;
   a.units_y = (a.H + hgru::kTileRows - 1) / hgru::kTileRows;
@@ -58,8 +58,8 @@ int launch_stack(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t st) {
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = (a.wait_flags || a.pdl) ? 1 : 0;
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, map, map, a));     // (w_map is only read in pair mode)
+  cfg.attrs = at; cfg.numAttrs = a.wait_flags ? 1 : 0;
+  CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, map, a));
   return 0;
 }
 
@@ -94,9 +94,8 @@ int stack_launch(EpiKind epi, int wsets, bool part, int KP, int T, OpFormat fmt,
     switch (epi) {
       case EPI_H1_HALF: return dispatch_stack<hgru::EpiH1h>(KP, T, map, a, st);      // fused bf16 pipeline
       case EPI_H2_HALF: return dispatch_stack<hgru::EpiH2h>(KP, T, map, a, st);
-      case EPI_H1: return dispatch_stack<hgru::EpiH1>(KP, T, map, a, st);            // (HGRU_FP32_HG=1 A/B runs)
-      case EPI_H2: return dispatch_stack<hgru::EpiH2>(KP, T, map, a, st);
       case EPI_PARTIAL: return dispatch_stack<hgru::EpiPartial>(KP, T, map, a, st);  // bf16x3, first launch of a conv
+      default: break;
     }
   } else if (part && wsets == 2) {                                                   // bf16x3, second launch
     if (epi == EPI_H1) return dispatch_stack<hgru::EpiH1, 2, true>(KP, T, map, a, st);

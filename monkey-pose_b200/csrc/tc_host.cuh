@@ -47,21 +47,6 @@ inline int make_act_tensor_map(CUtensorMap* map, const void* base, int N, int CG
   return r == CUDA_SUCCESS ? 0 : static_cast<int>(r);
 }
 
-// Tensor map over a packed byte array viewed as rows of 256 bytes; box = `box_rows` consecutive rows
-// (one weight-ring stage).  Used where a load must signal a peer CTA's mbarrier (cta_group::2 TMA).
-inline int make_rows256_map(CUtensorMap* map, const void* base, size_t total_bytes, int box_rows) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) return -1;
-  cuuint64_t gdim[2] = {256, static_cast<cuuint64_t>(total_bytes / 256)};
-  cuuint64_t gstr[1] = {256};
-  cuuint32_t box[2] = {256, static_cast<cuuint32_t>(box_rows)};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? 0 : static_cast<int>(r);
-}
-
 // Tensor map over a K-major bf16 matrix [rows][K] (row pitch K*2 bytes, K % 8 == 0) with boxes of
 // (64 K-elements = 128 bytes) x box_rows and the 128-byte swizzle: the canonical SW128 UMMA tile.
 inline int make_kmajor_bf16_map(CUtensorMap* map, const void* base, size_t rows, size_t K, int box_rows) {

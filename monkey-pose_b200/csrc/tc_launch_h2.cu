@@ -29,10 +29,10 @@ int launch_tc(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t st) {
   TC_CASE(Epi_, S_, 32, 2, 8, G32_)       \
   TC_CASE(Epi_, S_, 16, 1, 8, G32_)
 
-// the horizontal convs with the fused integration epilogues
+// the horizontal convs with the fused integration epilogues, S < 15 (15 x 15 runs on the tap-stacked kernel or, at
+// 64 channels, on the fused one below)
 template <class Epi>
 int dispatch_tc_hconv(int S, int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st) {
-  TC_CASES_S(Epi, 15, 5, 15)
   TC_CASES_S(Epi, 7, 7, 7)
   TC_CASES_S(Epi, 5, 5, 5)
   TC_CASES_S(Epi, 3, 9, 9)
@@ -62,17 +62,16 @@ int launch_tc_fused64(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t s
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = (a.wait_flags || a.pdl) ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = a.wait_flags ? 1 : 0;
   CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, map, a));
   return 0;
 }
 
-// bf16x3 mode: the 15x15 horizontal convs on hi/lo operand splits
+// bf16x3 mode at 64 channels: the 15x15 horizontal convs on hi/lo operand splits (narrower layers run it on the
+// tap-stacked kernel)
 template <class Epi>
 int dispatch_tc_hconv_x3(int S, int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st) {
   if (S == 15 && KP == 64) return launch_tc<15, 4, 64, 1, 3, Epi, true>(map, a, st);   // (wide stages: 3 taps each)
-  if (S == 15 && KP == 32) return launch_tc<15, 2, 32, 4, 5, Epi, true>(map, a, st);
-  if (S == 15 && KP == 16) return launch_tc<15, 1, 16, 8, 5, Epi, true>(map, a, st);
   return fail(HGRU_E_UNSUPPORTED, "bf16x3 conv: unsupported (S, padded channels)");
 }
 

@@ -188,32 +188,6 @@ def test_chained_launches_equal_stream_ordered_launches(monkeypatch):
     assert torch.equal(outs[True][1], outs[False][1])
 
 
-@pytest.mark.parametrize("channels,group", [(25, 37), (25, 64), (64, 19), (32, 50)])
-def test_group_major_order_equals_whole_batch_order(monkeypatch, channels, group):
-    """HGRU_GROUP_FRAMES (read when the plan is created): the chained launches walk the batch in frame groups, all 2T
-    launches of a group before the next group (so a group's state can stay in L2 across timesteps).  Frames are
-    independent, so the predictions must be bit for bit those of the whole-batch order; 150 frames: ragged last group."""
-    N, hw, T, S, F = (150 if channels < 64 else 40), 64, 3, 15, 32
-    P = init.pose_params(channels=channels, S=S, T=T, hw=hw, fc_hidden=F, out=69, seed=3, stress=4.0, random_bn=True)
-    depth = torch.as_tensor(init.synthetic_depth(N, seed=0, size=2 * hw)).cuda()
-    h0 = init.hidden_init((N, hw, hw, channels), seed=5)
-    outs = []
-    for g in (None, group):
-        if g is None:
-            monkeypatch.delenv("HGRU_GROUP_FRAMES", raising=False)
-        else:
-            monkeypatch.setenv("HGRU_GROUP_FRAMES", str(g))
-        m = mp.model()
-        m.channels, m.timesteps, m.fc_hidden, m.compute_mode, m.hidden_state = channels, T, F, "bf16", h0
-        m.load_params(P)
-        reps = [m.build(depth, 69).clone() for _ in range(3)]
-        torch.cuda.synchronize()
-        assert all(torch.equal(r, reps[0]) for r in reps[1:])
-        outs.append((reps[0], m.activation("hgru"), m.gpu_launches))
-    assert torch.equal(outs[0][0], outs[1][0]) and torch.equal(outs[0][1], outs[1][1])
-    assert outs[1][2] > outs[0][2]          # more, smaller launches
-
-
 @pytest.mark.parametrize("shape", [(5, 40, 24, 25, 15, 3), (3, 33, 70, 25, 15, 2), (40, 64, 64, 32, 15, 3),
                                    (9, 18, 66, 16, 15, 2)])
 def test_chained_layer_equals_traced_layer_on_ragged_shapes(shape):

@@ -158,6 +158,23 @@ def test_product_build_defines_no_development_switch():
     assert {"HGRU_STACK_NO_REM", "HGRU_STACK_NGRP4", "HGRU_DBG_NO_GLOBAL"} <= switches
 
 
+def test_library_reads_only_the_chaining_switch_from_the_environment():
+    """The one run-time switch of the library is HGRU_NO_CHAIN=1 (plain stream order between the conv launches, the
+    reference order of the chaining test).  Every getenv() argument in the library's sources (not the devtools) is
+    collected, a non-literal one as its expression, so a switch read through a helper is caught too."""
+    import os
+    import re
+    csrc = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "monkey-pose_b200", "csrc")
+    names = set()
+    for root, dirs, files in os.walk(csrc):
+        dirs[:] = [d for d in dirs if d != "devtools"]
+        for fn in files:
+            if fn.endswith((".cu", ".cuh", ".inl", ".h", ".cpp")):
+                src = open(os.path.join(root, fn)).read()
+                names |= {a.strip().strip('"') for a in re.findall(r"\bgetenv\(([^)]*)\)", src)}
+    assert names == {"HGRU_NO_CHAIN"}
+
+
 def test_circuit_step_methods_mirror_the_reference_signatures():
     """ContextualCircuit exposes the reference's per-timestep methods (hgru_module.py:505-861) with the same argument
     names and order; they need CUDA tensors (no CPU fallback)."""
