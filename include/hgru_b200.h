@@ -13,7 +13,11 @@
  *     stream-ordered unless stated otherwise;
  *   - every function returns 0 on success, non-zero on failure (HGRU_E_*); the message of the
  *     last failure on the calling thread is available from hgru_last_error(); nothing aborts;
- *   - one plan per GPU; a plan is not re-entrant (use it from one thread / stream at a time).
+ *   - one plan per GPU; a plan is not re-entrant (use it from one thread / stream at a time);
+ *   - a plan's N is its capacity: the *_forward_batch entry points run any batch of 1 <= n <= N frames on it (the
+ *     reference's placeholders have a run-time batch dimension), every tensor argument then has n frames, and the
+ *     result equals that of a plan created for n frames, bit for bit.  The plain *_forward calls are the n = N case.
+ *     An n outside [1, N] returns HGRU_E_INVALID before any CUDA call.
  */
 #ifndef HGRU_B200_H_
 #define HGRU_B200_H_
@@ -76,6 +80,9 @@ HGRU_API int hgru_set_params(hgru_plan_t plan, const float* p_r_dev, const float
  * H1_trace / H2_trace: NULL or [T,N,H,W,k] buffers receiving I / O after every timestep. */
 HGRU_API int hgru_forward(hgru_plan_t plan, const float* X_dev, const float* H2_init_dev, float* H2_out_dev,
                  float* H1_trace_dev, float* H2_trace_dev, void* stream);
+/* The same over n frames (1 <= n <= N): X, H2_init, H2_out [n,H,W,k], traces [T,n,H,W,k]. */
+HGRU_API int hgru_forward_batch(hgru_plan_t plan, int n, const float* X_dev, const float* H2_init_dev,
+                                float* H2_out_dev, float* H1_trace_dev, float* H2_trace_dev, void* stream);
 
 HGRU_API size_t hgru_plan_workspace_bytes(hgru_plan_t plan);
 /* number of kernels the last hgru_forward launched */
@@ -115,6 +122,12 @@ HGRU_API int pose_forward(pose_plan_t plan, const float* depth_dev, const float*
  * on return.  H2_init stays a device pointer (it is state, not per-frame input). */
 HGRU_API int pose_forward_host(pose_plan_t plan, const float* depth_host, const float* H2_init_dev,
                       float* out_host, void* stream);
+/* pose_forward / pose_forward_host over n frames (1 <= n <= N): depth [n,2HW,2HW,1], H2_init [n,HW,HW,C], out [n,O];
+ * only n frames are uploaded and read back.  No re-allocation and no re-packing of the parameters. */
+HGRU_API int pose_forward_batch(pose_plan_t plan, int n, const float* depth_dev, const float* H2_init_dev,
+                                float* out_dev, void* stream);
+HGRU_API int pose_forward_host_batch(pose_plan_t plan, int n, const float* depth_host, const float* H2_init_dev,
+                                     float* out_host, void* stream);
 
 /* aux['hidden_init'] = 'identity' (hgru_module.py:876-878: O_0 = X, the hGRU's own input): when on, H2_init_dev
  * of the forward calls is ignored and the initial state is conv3 of the same forward.  Off by default. */
@@ -122,10 +135,11 @@ HGRU_API int pose_set_hidden_init(pose_plan_t plan, int identity);
 
 /* Intermediate activations of the last pose_forward, by the reference's attribute names
  * ("pool1","conv2","conv3","hgru","fc1"; hgru_pose.py:50-105), copied into dst_dev in the
- * reference's layout ([N,HW,HW,C] / [N,F]).  For parity tests. */
+ * reference's layout ([n,HW,HW,C] / [n,F], n = the last forward's frames).  For parity tests. */
 HGRU_API int pose_get_activation(pose_plan_t plan, const char* name, float* dst_dev, void* stream);
 
 HGRU_API size_t pose_plan_workspace_bytes(pose_plan_t plan);
+/* kernels the last pose_forward* launched */
 HGRU_API int pose_plan_launch_count(pose_plan_t plan);
 /* average device time (ms) of the horizontal-conv kernels in the last pose_forward/hgru_forward
  * when timing was enabled with hgru_enable_kernel_timing(plan-independent switch) */
@@ -308,7 +322,11 @@ HGRU_API int attn_plan_destroy(attn_plan_t plan);
 HGRU_API int attn_set_params(attn_plan_t plan, const attn_params_t* params, float bn_epsilon, void* stream);
 /* frames [N,H,W] fp32 (depth / image_max_depth, as the caller feeds the reference graph) -> out [N,O] */
 HGRU_API int attn_forward(attn_plan_t plan, const float* frames_dev, float* out_dev, void* stream);
-/* name in {"resized","pool1",...,"pool5","fc1"}: dense fp32 NHWC copy of an intermediate tensor */
+/* The same over n frames (1 <= n <= N): frames [n,H,W], out [n,O].  Each layer's K split is the one a plan created
+ * for n frames takes, so the result depends on the batch only, not on the capacity. */
+HGRU_API int attn_forward_batch(attn_plan_t plan, int n, const float* frames_dev, float* out_dev, void* stream);
+/* name in {"resized","pool1",...,"pool5","fc1"}: dense fp32 NHWC copy of an intermediate tensor of the last
+ * forward (its n frames) */
 HGRU_API int attn_get_activation(attn_plan_t plan, const char* name, float* dst_dev, void* stream);
 HGRU_API size_t attn_plan_workspace_bytes(attn_plan_t plan);
 HGRU_API int attn_plan_launch_count(attn_plan_t plan);

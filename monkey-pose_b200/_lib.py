@@ -49,6 +49,7 @@ SIGNATURES = {
     "hgru_plan_destroy": (_I, [_P]),
     "hgru_set_params": (_I, [_P] + [_P] * 12 + [_P]),
     "hgru_forward": (_I, [_P, _P, _P, _P, _P, _P, _P]),
+    "hgru_forward_batch": (_I, [_P, _I, _P, _P, _P, _P, _P, _P]),
     "hgru_plan_workspace_bytes": (ctypes.c_size_t, [_P]),
     "hgru_plan_launch_count": (_I, [_P]),
     "pose_plan_create": (_I, [_I, _I, _I, _I, _I, _I, _I, _I, ctypes.POINTER(_P)]),
@@ -56,6 +57,8 @@ SIGNATURES = {
     "pose_set_params": (_I, [_P, ctypes.POINTER(PoseParams), ctypes.c_float, _P]),
     "pose_forward": (_I, [_P, _P, _P, _P, _P]),
     "pose_forward_host": (_I, [_P, _P, _P, _P, _P]),
+    "pose_forward_batch": (_I, [_P, _I, _P, _P, _P, _P]),
+    "pose_forward_host_batch": (_I, [_P, _I, _P, _P, _P, _P]),
     "pose_set_hidden_init": (_I, [_P, _I]),
     "pose_get_activation": (_I, [_P, ctypes.c_char_p, _P, _P]),
     "pose_plan_workspace_bytes": (ctypes.c_size_t, [_P]),
@@ -95,6 +98,7 @@ SIGNATURES = {
     "attn_plan_destroy": (_I, [_P]),
     "attn_set_params": (_I, [_P, ctypes.POINTER(AttnParams), ctypes.c_float, _P]),
     "attn_forward": (_I, [_P, _P, _P, _P]),
+    "attn_forward_batch": (_I, [_P, _I, _P, _P, _P]),
     "attn_get_activation": (_I, [_P, ctypes.c_char_p, _P, _P]),
     "attn_plan_workspace_bytes": (ctypes.c_size_t, [_P]),
     "attn_plan_launch_count": (_I, [_P]),

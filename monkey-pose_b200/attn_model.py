@@ -41,6 +41,7 @@ class attn_model_struct(LayerOps):
         self.dropout_seed = 1234
         self._plan = None
         self._plan_key = None
+        self._plan_capacity = 0                      # frames the plan was created for: it runs every batch up to that
         self._dev_params = None
 
     def __getitem__(self, name):
@@ -123,8 +124,9 @@ class attn_model_struct(LayerOps):
         if self._dev_params is None:
             self._dev_params = self._materialise(int(output_shape))
         P, widths, F = self._dev_params
-        key = (N, H, W, widths, F, int(output_shape), depth.device.index)
-        if self._plan_key != key:
+        # a plan runs any batch up to its capacity (attn_forward_batch); a larger batch re-creates it at that size
+        key = (H, W, widths, F, int(output_shape), depth.device.index)
+        if self._plan_key != key or N > self._plan_capacity:
             if self._plan is not None:
                 lib.attn_plan_destroy(self._plan)
                 self._plan = None
@@ -132,7 +134,7 @@ class attn_model_struct(LayerOps):
             wa = (ctypes.c_int * 5)(*widths)
             _lib.check(lib.attn_plan_create(N, H, W, wa, F, int(output_shape), ctypes.byref(plan)),
                        "attn_plan_create")
-            self._plan, self._plan_key = plan, key
+            self._plan, self._plan_key, self._plan_capacity = plan, key, N
             q = _lib.AttnParams()
             for i, (name, _) in enumerate(init.ATTN_CONV):
                 q.conv_filters[i] = P[name + "_filters"].data_ptr()
@@ -145,7 +147,8 @@ class attn_model_struct(LayerOps):
             _lib.check(lib.attn_set_params(plan, ctypes.byref(q), float(self._BATCH_NORM_EPSILON), _stream()),
                        "attn_set_params")
         out = torch.empty((N, int(output_shape)), device=depth.device, dtype=torch.float32)
-        _lib.check(lib.attn_forward(self._plan, depth.data_ptr(), out.data_ptr(), _stream()), "attn_forward")
+        _lib.check(lib.attn_forward_batch(self._plan, N, depth.data_ptr(), out.data_ptr(), _stream()),
+                   "attn_forward_batch")
         self.gpu_launches = int(lib.attn_plan_launch_count(self._plan))
         self._shapes = {"resized": (N, 128, 128, 1), "fc1": (N, F)}
         for i, c in enumerate(widths):

@@ -39,6 +39,13 @@ int fail(int code, const std::string& msg) {
 
 using namespace hgru_host;
 
+// the frame count of a *_batch forward: 1 <= n <= N, the capacity the plan was created with
+static int check_batch(const char* fn, int n, int N) {
+  if (n >= 1 && n <= N) return 0;
+  return fail(HGRU_E_INVALID, std::string(fn) + ": n = " + std::to_string(n) + " is outside [1, " + std::to_string(N) +
+                                  "], the plan's capacity");
+}
+
 namespace {
 
 struct DevBuf {
@@ -165,8 +172,9 @@ struct KernelTimer {
 // hGRU plan
 // =================================================================================================
 struct hgru_plan_s {
-  int N, H, W, k, KP, CG, S, T, mode;
-  size_t npix, nelem;        // pixels, padded elements
+  int N, H, W, k, KP, CG, S, T, mode;   // N: capacity, the frames every buffer and tensor map is sized for
+  size_t npix, nelem;        // pixels, padded elements (of N frames)
+  int n = 0;                 // frames of the current (or last) forward, 1 <= n <= N: the first n frames of every buffer
   bool params_set = false;
   int launches = 0;
   // parameters (zero padded to KP)
@@ -197,6 +205,8 @@ struct hgru_plan_s {
   bool op16() const { return mode == HGRU_MODE_BF16 || mode == HGRU_MODE_FP16; }
   OpFormat fmt() const { return mode == HGRU_MODE_FP16 ? FMT_FP16 : FMT_BF16; }
   float* vec(int i) const { return vecs.as<float>() + static_cast<size_t>(i) * KP; }
+  size_t npix_n() const { return static_cast<size_t>(n) * H * W; }      // pixels, padded elements of n frames
+  size_t nelem_n() const { return npix_n() * KP; }
   size_t workspace() const {
     return p_r.bytes + i_r.bytes + o_r.bytes + vecs.bytes + rho.bytes + wpk.bytes + wpk_i.bytes +
            wpk_o.bytes + Xp.bytes + H2.bytes + H1.bytes + C.bytes + G.bytes + A.bytes + actA.bytes +
@@ -214,7 +224,7 @@ static int hgru_plan_init(hgru_plan_s* p, int N, int H, int W, int k, int S, int
   // fp16 operands exist for the 15x15 kernels only: tap-stacked (k <= 32) and fused paired-tap (k <= 64)
   if (mode == HGRU_MODE_FP16 && (S != 15 || k > 64))
     return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: fp16 mode supports S = 15 and k <= 64");
-  p->N = N; p->H = H; p->W = W; p->k = k; p->S = S; p->T = T; p->mode = mode;
+  p->N = N; p->n = N; p->H = H; p->W = W; p->k = k; p->S = S; p->T = T; p->mode = mode;
   p->KP = round_up(k, 16);
   if (mode != HGRU_MODE_FP32 && p->KP == 48) p->KP = 64;      // tensor-core kernels exist for 16 / 32 / 64 padded channels
   // exact path: the 1x1 gate kernel keeps the k x k matrix and a 64-pixel tile in <= 64 KB of shared memory
@@ -403,30 +413,30 @@ static int hgru_set_params_impl(hgru_plan_s* p, const float* p_r, const float* i
 // ---- fp32 path: SIMT kernels, unfused (the <= 1e-4 anchor) --------------------------------------
 static int hgru_run_fp32(hgru_plan_s* p, const float* Xp, float* H1_trace, float* H2_trace, cudaStream_t st) {
   const int KP = p->KP, HW = p->H * p->W;
-  const size_t nchunks = p->nelem / 8;
+  const size_t nchunks = p->nelem_n() / 8;
   const size_t gate_smem = sizeof(float) * (KP * KP + 64 * (KP + 1));
   SMEM_ATTR_ONCE(hgru::gate1x1_kernel, 64 * 1024);
   int rc;
   for (int t = 0; t < p->T; ++t) {
     // circuit_input (hgru_module.py:692-724): G1, gated copy, C1 = conv + lateral_bias (:657)
-    hgru::gate1x1_kernel<<<nblk(p->npix, 64), 256, gate_smem, st>>>(
-        p->H2.as<float>(), p->i_r.as<float>(), p->vec(V_IB), nullptr, p->A.as<float>(), nullptr, p->npix, KP,
+    hgru::gate1x1_kernel<<<nblk(p->npix_n(), 64), 256, gate_smem, st>>>(
+        p->H2.as<float>(), p->i_r.as<float>(), p->vec(V_IB), nullptr, p->A.as<float>(), nullptr, p->npix_n(), KP,
         p->k, HW);
     p->timer.begin(st);
     if ((rc = dispatch_simt_conv(p->S, p->A.as<float>(), p->p_r.as<float>(), p->vec(V_LBIAS), nullptr, nullptr,
-                                 p->C.as<float>(), p->N, p->H, p->W, KP, KP, 0, st)))
+                                 p->C.as<float>(), p->n, p->H, p->W, KP, KP, 0, st)))
       return rc;
     p->timer.end(st);
     // input_integration (:795-804)
     hgru::h1_kernel<<<nblk(nchunks), 256, 0, st>>>(Xp, p->H2.as<float>(), p->C.as<float>(), p->vec(V_BETA),
                                                   p->vec(V_NU), p->H1.as<float>(), nullptr, nchunks, KP, p->k, HW);
     // circuit_output (:726-756): G2, C2
-    hgru::gate1x1_kernel<<<nblk(p->npix, 64), 256, gate_smem, st>>>(
-        p->H1.as<float>(), p->o_r.as<float>(), p->vec(V_OB), p->G.as<float>(), nullptr, nullptr, p->npix, KP,
+    hgru::gate1x1_kernel<<<nblk(p->npix_n(), 64), 256, gate_smem, st>>>(
+        p->H1.as<float>(), p->o_r.as<float>(), p->vec(V_OB), p->G.as<float>(), nullptr, nullptr, p->npix_n(), KP,
         p->k, HW);
     p->timer.begin(st);
     if ((rc = dispatch_simt_conv(p->S, p->H1.as<float>(), p->p_r.as<float>(), p->vec(V_LBIAS), nullptr, nullptr,
-                                 p->C.as<float>(), p->N, p->H, p->W, KP, KP, 0, st)))
+                                 p->C.as<float>(), p->n, p->H, p->W, KP, KP, 0, st)))
       return rc;
     p->timer.end(st);
     // output_integration + rho (:806-823, 847-849)
@@ -435,13 +445,13 @@ static int hgru_run_fp32(hgru_plan_s* p, const float* Xp, float* H1_trace, float
                                                   p->rho.as<float>(), t, p->H2.as<float>(), nchunks, KP, p->k);
     p->launches += 6;
     if (H1_trace) {
-      hgru::unpad_channels_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(
-          p->H1.as<float>(), H1_trace + static_cast<size_t>(t) * p->npix * p->k, p->npix, p->k, KP);
+      hgru::unpad_channels_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
+          p->H1.as<float>(), H1_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP);
       ++p->launches;
     }
     if (H2_trace) {
-      hgru::unpad_channels_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(
-          p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix * p->k, p->npix, p->k, KP);
+      hgru::unpad_channels_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
+          p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP);
       ++p->launches;
     }
   }
@@ -473,7 +483,7 @@ static int launch_init_tc(int KP, const float* h0, const hgru::TcConvArgs& a, cu
 static int hgru_init_state_bf16(hgru_plan_s* p, const float* H2_init_nhwc, cudaStream_t st) {
   // the 1x1 gate conv as one UMMA tile per 128 pixels (16-bit operands like every later gate)
   hgru::TcConvArgs a{};
-  a.N = p->N; a.H = p->H; a.W = p->W; a.KP = p->KP; a.kreal = p->k; a.act_pad = p->act_pad;
+  a.N = p->n; a.H = p->H; a.W = p->W; a.KP = p->KP; a.kreal = p->k; a.act_pad = p->act_pad;
   a.wpk = p->wpk_i.as<__nv_bfloat16>(); a.bias = p->vec(V_IB); a.H2 = p->H2.as<float>();
   a.out_bf16 = p->actA.as<__nv_bfloat16>();
   return p->fmt() == FMT_FP16 ? launch_init_tc<hgru::OpFp16>(p->KP, H2_init_nhwc, a, st)
@@ -485,7 +495,7 @@ static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_n
   const int KP = p->KP, HW = p->H * p->W;
   int rc;
   hgru::TcConvArgs base{};
-  base.N = p->N; base.H = p->H; base.W = p->W; base.KP = KP; base.kreal = p->k;
+  base.N = p->n; base.H = p->H; base.W = p->W; base.KP = KP; base.kreal = p->k;
   base.act_pad = p->act_pad;
   // initial state O_0 (NHWC or zeros) -> H2 (quad-chunked fp32) + the first gated operand, one pass (unless the
   // caller already ran it: the pose plan overlaps it with the upload of the crops)
@@ -566,16 +576,16 @@ static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_n
     //                                                       counted as 2T passes over the whole batch
     ++p->launches;
     if (H1_trace) {
-      float* dst = H1_trace + static_cast<size_t>(t) * p->npix * p->k;
+      float* dst = H1_trace + static_cast<size_t>(t) * p->npix_n() * p->k;
       if (fused)      // H1 is an fp16 oct-chunked tensor in the fused pipeline
-        hgru::oct_half_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(p->H1.as<__half>(), dst, p->npix, p->k, KP, HW);
+        hgru::oct_half_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(p->H1.as<__half>(), dst, p->npix_n(), p->k, KP, HW);
       else
-        hgru::quad_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(p->H1.as<float>(), dst, p->npix, p->k, KP, HW);
+        hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(p->H1.as<float>(), dst, p->npix_n(), p->k, KP, HW);
       ++p->launches;
     }
     if (H2_trace) {
-      hgru::quad_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(
-          p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix * p->k, p->npix, p->k, KP, HW);
+      hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
+          p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
       ++p->launches;
     }
   }
@@ -593,12 +603,12 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
   SMEM_ATTR_ONCE(hgru::gate_quad_split_kernel, 100 * 1024);
   const size_t gsmem = sizeof(float) * (KP * KP + hgru::kInitPix * (KP + 1));
   if (H2_init_nhwc)
-    hgru::nhwc_to_quad_kernel<<<nblk(p->nelem / 4), 256, 0, st>>>(H2_init_nhwc, p->H2.as<float>(), p->npix, p->k, KP, HW);
+    hgru::nhwc_to_quad_kernel<<<nblk(p->nelem_n() / 4), 256, 0, st>>>(H2_init_nhwc, p->H2.as<float>(), p->npix_n(), p->k, KP, HW);
   else
-    CUDA_TRY(cudaMemsetAsync(p->H2.p, 0, p->H2.bytes, st));
+    CUDA_TRY(cudaMemsetAsync(p->H2.p, 0, p->nelem_n() * sizeof(float), st));
   ++p->launches;
   hgru::TcConvArgs base{};
-  base.N = p->N; base.H = p->H; base.W = p->W; base.KP = KP; base.kreal = p->k;
+  base.N = p->n; base.H = p->H; base.W = p->W; base.KP = KP; base.kreal = p->k;
   base.split_out = 1;
   if (p->stacked) {
     // ---- narrow layers: the tap-stacked kernel, two launches per conv (see hgru_plan_init) ----
@@ -616,8 +626,8 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
     };
     auto gate_in = [&]() {
       // circuit_input gate (hgru_module.py:696-711), exact fp32: operand A = split(sigmoid(H2 *1x1 i_r + i_b) . H2)
-      hgru::gate_quad_split_kernel<<<nblk(p->npix, hgru::kInitPix), 256, gsmem, st>>>(
-          p->H2.as<float>(), p->i_r.as<float>(), p->vec(V_IB), nullptr, p->actA.as<__nv_bfloat16>(), p->npix, p->k,
+      hgru::gate_quad_split_kernel<<<nblk(p->npix_n(), hgru::kInitPix), 256, gsmem, st>>>(
+          p->H2.as<float>(), p->i_r.as<float>(), p->vec(V_IB), nullptr, p->actA.as<__nv_bfloat16>(), p->npix_n(), p->k,
           KP, HW, p->lo_off, p->W, p->act_pad);
       ++p->launches;
     };
@@ -643,8 +653,8 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
       if (!chain) p->timer.end(st);
       if (!fused_gate) {
         // circuit_output gate (:729-740): G2 = sigmoid(H1 *1x1 o_r + o_b), exact fp32
-        hgru::gate_quad_split_kernel<<<nblk(p->npix, hgru::kInitPix), 256, gsmem, st>>>(
-            p->H1.as<float>(), p->o_r.as<float>(), p->vec(V_OB), p->G.as<float>(), nullptr, p->npix, p->k, KP, HW);
+        hgru::gate_quad_split_kernel<<<nblk(p->npix_n(), hgru::kInitPix), 256, gsmem, st>>>(
+            p->H1.as<float>(), p->o_r.as<float>(), p->vec(V_OB), p->G.as<float>(), nullptr, p->npix_n(), p->k, KP, HW);
         ++p->launches;
       }
       // C2 conv (:746-750, 657) + output_integration + rho (:806-823, 847-849) -> H2 in place
@@ -671,13 +681,13 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
       else if (t + 1 == p->T) p->timer.end(st, 2 * p->T);      // chained: one interval, counted as 2T convs
       p->launches += 4;
       if (H1_trace) {
-        hgru::quad_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(
-            p->H1.as<float>(), H1_trace + static_cast<size_t>(t) * p->npix * p->k, p->npix, p->k, KP, HW);
+        hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
+            p->H1.as<float>(), H1_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
         ++p->launches;
       }
       if (H2_trace) {
-        hgru::quad_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(
-            p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix * p->k, p->npix, p->k, KP, HW);
+        hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
+            p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
         ++p->launches;
       }
     }
@@ -685,8 +695,8 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
   }
   for (int t = 0; t < p->T; ++t) {
     // circuit_input gate (hgru_module.py:696-711): operand A = split(sigmoid(H2 *1x1 i_r + i_b) . H2)
-    hgru::gate_quad_split_kernel<<<nblk(p->npix, hgru::kInitPix), 256, gsmem, st>>>(
-        p->H2.as<float>(), p->i_r.as<float>(), p->vec(V_IB), nullptr, p->actA.as<__nv_bfloat16>(), p->npix, p->k,
+    hgru::gate_quad_split_kernel<<<nblk(p->npix_n(), hgru::kInitPix), 256, gsmem, st>>>(
+        p->H2.as<float>(), p->i_r.as<float>(), p->vec(V_IB), nullptr, p->actA.as<__nv_bfloat16>(), p->npix_n(), p->k,
         KP, HW);
     // C1 conv (:714-718, 657) + input_integration (:795-804) -> H1 (fp32 + hi/lo operand)
     hgru::TcConvArgs a = base;
@@ -697,8 +707,8 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
     if ((rc = tc_x3_launch(EPI_H1, p->S, KP, p->mapA, a, st))) return rc;
     p->timer.end(st);
     // circuit_output gate (:729-740): G2 = sigmoid(H1 *1x1 o_r + o_b), exact fp32
-    hgru::gate_quad_split_kernel<<<nblk(p->npix, hgru::kInitPix), 256, gsmem, st>>>(
-        p->H1.as<float>(), p->o_r.as<float>(), p->vec(V_OB), p->G.as<float>(), nullptr, p->npix, p->k, KP, HW);
+    hgru::gate_quad_split_kernel<<<nblk(p->npix_n(), hgru::kInitPix), 256, gsmem, st>>>(
+        p->H1.as<float>(), p->o_r.as<float>(), p->vec(V_OB), p->G.as<float>(), nullptr, p->npix_n(), p->k, KP, HW);
     // C2 conv (:746-750, 657) + output_integration + rho (:806-823, 847-849) -> H2 in place
     a = base;
     a.wpk = p->wpk.as<__nv_bfloat16>(); a.bias = p->vec(V_LBIAS); a.H1 = p->H1.as<float>();
@@ -713,13 +723,13 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
     p->timer.end(st);
     p->launches += 4;
     if (H1_trace) {
-      hgru::quad_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(
-          p->H1.as<float>(), H1_trace + static_cast<size_t>(t) * p->npix * p->k, p->npix, p->k, KP, HW);
+      hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
+          p->H1.as<float>(), H1_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
       ++p->launches;
     }
     if (H2_trace) {
-      hgru::quad_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(
-          p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix * p->k, p->npix, p->k, KP, HW);
+      hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
+          p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
       ++p->launches;
     }
   }
@@ -729,15 +739,15 @@ static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init
 // API boundary <-> internal state layout (fp32 mode: channel-padded NHWC; bf16 modes: quad-chunked)
 static void state_from_nhwc(const hgru_plan_s* p, const float* in, float* out, cudaStream_t st) {
   if (p->mode != HGRU_MODE_FP32)
-    hgru::nhwc_to_quad_kernel<<<nblk(p->nelem / 4), 256, 0, st>>>(in, out, p->npix, p->k, p->KP, p->H * p->W);
+    hgru::nhwc_to_quad_kernel<<<nblk(p->nelem_n() / 4), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP, p->H * p->W);
   else
-    hgru::pad_channels_kernel<<<nblk(p->nelem), 256, 0, st>>>(in, out, p->npix, p->k, p->KP);
+    hgru::pad_channels_kernel<<<nblk(p->nelem_n()), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP);
 }
 static void state_to_nhwc(const hgru_plan_s* p, const float* in, float* out, cudaStream_t st) {
   if (p->mode != HGRU_MODE_FP32)
-    hgru::quad_to_nhwc_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(in, out, p->npix, p->k, p->KP, p->H * p->W);
+    hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP, p->H * p->W);
   else
-    hgru::unpad_channels_kernel<<<nblk(p->npix * p->k), 256, 0, st>>>(in, out, p->npix, p->k, p->KP);
+    hgru::unpad_channels_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP);
 }
 
 // The recurrence on padded buffers: X = Xp, state in p->H2 (in/out).
@@ -753,7 +763,7 @@ static int hgru_run_padded(hgru_plan_s* p, const float* Xp, const float* H2_init
     rc = hgru_run_bf16x3(p, Xp, H2_init_nhwc, H1_trace, H2_trace, st);
   } else {
     if (H2_init_nhwc) state_from_nhwc(p, H2_init_nhwc, p->H2.as<float>(), st);
-    else CUDA_TRY(cudaMemsetAsync(p->H2.p, 0, p->H2.bytes, st));
+    else CUDA_TRY(cudaMemsetAsync(p->H2.p, 0, p->nelem_n() * sizeof(float), st));
     rc = hgru_run_fp32(p, Xp, H1_trace, H2_trace, st);
   }
   if (rc) return rc;
@@ -811,17 +821,21 @@ static void pose_plan_free(pose_plan_s* p) {
   for (auto b : all) b->release();
 }
 
-static int pose_forward_impl(pose_plan_s* p, const float* depth, const float* H2_init, float* out, cudaStream_t st,
-                             const cudaEvent_t* chunk_ready = nullptr, int nchunks = 1) {
+// A forward over the first n frames of the plan (n <= N; buffers, tensor maps and the chaining counters keep the
+// capacity N as their size and stride).  Every per-forward size derives from n, so the result equals that of a plan
+// created for n frames, bit for bit.
+static int pose_forward_impl(pose_plan_s* p, int n, const float* depth, const float* H2_init, float* out,
+                             cudaStream_t st, const cudaEvent_t* chunk_ready = nullptr, int nchunks = 1) {
   if (!p->params_set) return fail(HGRU_E_STATE, "pose_forward before pose_set_params");
   if (!depth || !out) return fail(HGRU_E_INVALID, "pose_forward: null pointer");
   hgru_plan_s* h = &p->hg;
-  const int N = p->N, HW = p->HW, KP = p->KP, C = p->C;
+  h->n = n;
+  const int HW = p->HW, KP = p->KP, C = p->C;
   const bool tc = p->mode != HGRU_MODE_FP32;      // stem + fc_1 on tensor cores (hi/lo splits) in both bf16 modes
   int rc;
   p->launches = 0;
   if (p->h0_identity && !p->h0_tmp.p) {
-    if (int r = p->h0_tmp.alloc(static_cast<size_t>(N) * HW * HW * C * sizeof(float))) return r;
+    if (int r = p->h0_tmp.alloc(static_cast<size_t>(p->N) * HW * HW * C * sizeof(float))) return r;
   }
   if (h->op16() && !p->h0_identity) {
     // the hGRU's initial-state pass does not depend on the crops: run it first (under their upload, when the
@@ -842,7 +856,7 @@ static int pose_forward_impl(pose_plan_s* p, const float* depth, const float* H2
   // output is X of the hGRU).  Frames are independent, so with a chunked upload (pose_forward_host) the stem of a
   // chunk runs as soon as the chunk has landed, under the upload of the next one; per-frame results do not depend
   // on the chunking.
-  const int per = (N + nchunks - 1) / nchunks;
+  const int per = (n + nchunks - 1) / nchunks;
   const size_t pix = static_cast<size_t>(HW) * HW;
   auto conv1 = [&](int n0, int nn) {
     float* o32 = tc ? nullptr : p->pool1.as<float>() + static_cast<size_t>(n0) * pix * KP;
@@ -868,7 +882,7 @@ static int pose_forward_impl(pose_plan_s* p, const float* depth, const float* H2
     return tc_stem_launch(KP, p->map_conv2, a, st);
   };
   for (int c = 0; c < nchunks; ++c) {
-    const int n0 = c * per, nn = (n0 + per <= N ? per : N - n0);
+    const int n0 = c * per, nn = (n0 + per <= n ? per : n - n0);
     if (nn <= 0) break;
     if (chunk_ready) CUDA_TRY(cudaStreamWaitEvent(st, chunk_ready[c], 0));
     conv1(n0, nn);
@@ -876,10 +890,10 @@ static int pose_forward_impl(pose_plan_s* p, const float* depth, const float* H2
   }
   if (!tc) {
     if ((rc = dispatch_simt_conv(3, p->pool1.as<float>(), p->w2.as<float>(), p->b2.as<float>(), p->bn_scale(1),
-                                 p->bn_shift(1), p->conv2.as<float>(), N, HW, HW, KP, KP, 1, st)))
+                                 p->bn_shift(1), p->conv2.as<float>(), n, HW, HW, KP, KP, 1, st)))
       return rc;
     if ((rc = dispatch_simt_conv(3, p->conv2.as<float>(), p->w3.as<float>(), p->b3.as<float>(), p->bn_scale(2),
-                                 p->bn_shift(2), h->Xp.as<float>(), N, HW, HW, KP, KP, 1, st)))
+                                 p->bn_shift(2), h->Xp.as<float>(), n, HW, HW, KP, KP, 1, st)))
       return rc;
     p->launches += 2;
   }
@@ -901,22 +915,22 @@ static int pose_forward_impl(pose_plan_s* p, const float* depth, const float* H2
   const int K = HW * HW * C;
   int nsplit = p->nsplit;
   if (p->fc1_tc) {
-    hgru::GemmArgs g{N, p->F, K, p->fc_kpad, p->fc_kbps, p->part.as<float>(), 0, 0, 0, 0, 0, 0};
-    dim3 grid((p->F + hgru::kGemmBN - 1) / hgru::kGemmBN, (N + hgru::kGemmBM - 1) / hgru::kGemmBM, p->fc_splits);
+    hgru::GemmArgs g{n, p->F, K, p->fc_kpad, p->fc_kbps, p->part.as<float>(), 0, 0, 0, 0, 0, 0};
+    dim3 grid((p->F + hgru::kGemmBN - 1) / hgru::kGemmBN, (n + hgru::kGemmBM - 1) / hgru::kGemmBM, p->fc_splits);
     hgru::gemm_tc_splitk_kernel<hgru::kGemmBN><<<grid, 256, hgru::kGemmSmemBytes, st>>>(p->map_fc_a, p->map_fc_a, p->map_fc_b, g);
     nsplit = p->fc_splits;
     ++p->launches;
   } else {
     const int kslice = round_up((K + p->nsplit - 1) / p->nsplit, 16);
-    dim3 g1((p->F + 63) / 64, (N + 63) / 64, p->nsplit);
+    dim3 g1((p->F + 63) / 64, (n + 63) / 64, p->nsplit);
     hgru::fc1_splitk_kernel<<<g1, 256, 0, st>>>(h->H2.as<float>(), p->fc1_w.as<float>(), p->bn_scale(3),
-                                                p->bn_shift(3), p->part.as<float>(), N, K, p->F, C, KP, kslice);
+                                                p->bn_shift(3), p->part.as<float>(), n, K, p->F, C, KP, kslice);
     ++p->launches;
   }
   // + bias, relu (:92), BN (:95-103), fc_out (:104)
-  hgru::fc_tail_kernel<<<N, 256, sizeof(float) * (p->F + hgru::kFcTailScratch), st>>>(
+  hgru::fc_tail_kernel<<<n, 256, sizeof(float) * (p->F + hgru::kFcTailScratch), st>>>(
       p->part.as<float>(), nsplit, p->fc1_b.as<float>(), p->bn_scale(4), p->bn_shift(4),
-      p->fc2_w.as<float>(), p->fc2_b.as<float>(), p->fc1.as<float>(), out, N, p->F, p->O);
+      p->fc2_w.as<float>(), p->fc2_b.as<float>(), p->fc1.as<float>(), out, n, p->F, p->O);
   ++p->launches;      // (one per kernel: the count is checked against the ncu launch list)
   CUDA_TRY(cudaGetLastError());
   return 0;
@@ -971,8 +985,16 @@ int hgru_set_params(hgru_plan_t plan, const float* p_r, const float* i_r, const 
 int hgru_forward(hgru_plan_t p, const float* X, const float* H2_init, float* H2_out, float* H1_trace,
                  float* H2_trace, void* stream) {
   if (!p) return fail(HGRU_E_INVALID, "hgru_forward: null plan");
+  return hgru_forward_batch(p, p->N, X, H2_init, H2_out, H1_trace, H2_trace, stream);
+}
+
+int hgru_forward_batch(hgru_plan_t p, int n, const float* X, const float* H2_init, float* H2_out, float* H1_trace,
+                       float* H2_trace, void* stream) {
+  if (!p) return fail(HGRU_E_INVALID, "hgru_forward_batch: null plan");
+  if (int rc = check_batch("hgru_forward_batch", n, p->N)) return rc;
   if (!X || !H2_out) return fail(HGRU_E_INVALID, "hgru_forward: null tensor pointer");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  p->n = n;
   state_from_nhwc(p, X, p->Xp.as<float>(), st);
   int rc = hgru_run_padded(p, p->Xp.as<float>(), H2_init, H1_trace, H2_trace, st);
   if (rc) return rc;
@@ -1124,11 +1146,24 @@ int pose_set_params(pose_plan_t p, const pose_params_t* q, float eps, void* stre
 
 int pose_forward(pose_plan_t p, const float* depth, const float* H2_init, float* out, void* stream) {
   if (!p) return fail(HGRU_E_INVALID, "pose_forward: null plan");
-  return pose_forward_impl(p, depth, H2_init, out, static_cast<cudaStream_t>(stream));
+  return pose_forward_impl(p, p->N, depth, H2_init, out, static_cast<cudaStream_t>(stream));
+}
+
+int pose_forward_batch(pose_plan_t p, int n, const float* depth, const float* H2_init, float* out, void* stream) {
+  if (!p) return fail(HGRU_E_INVALID, "pose_forward_batch: null plan");
+  if (int rc = check_batch("pose_forward_batch", n, p->N)) return rc;
+  return pose_forward_impl(p, n, depth, H2_init, out, static_cast<cudaStream_t>(stream));
 }
 
 int pose_forward_host(pose_plan_t p, const float* depth_host, const float* H2_init, float* out_host, void* stream) {
   if (!p) return fail(HGRU_E_INVALID, "pose_forward_host: null plan");
+  return pose_forward_host_batch(p, p->N, depth_host, H2_init, out_host, stream);
+}
+
+int pose_forward_host_batch(pose_plan_t p, int n, const float* depth_host, const float* H2_init, float* out_host,
+                            void* stream) {
+  if (!p) return fail(HGRU_E_INVALID, "pose_forward_host_batch: null plan");
+  if (int rc = check_batch("pose_forward_host_batch", n, p->N)) return rc;
   if (!depth_host || !out_host) return fail(HGRU_E_INVALID, "pose_forward_host: null pointer");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   // upload on the plan's copy stream (ordered after the work already queued on `st`), so that the copy engine
@@ -1141,22 +1176,22 @@ int pose_forward_host(pose_plan_t p, const float* depth_host, const float* H2_in
   CUDA_TRY(cudaEventRecord(p->ev_begin, st));
   CUDA_TRY(cudaStreamWaitEvent(p->copy_st, p->ev_begin, 0));
   // frame chunks, one event each: conv_1 of chunk c runs while chunk c+1 is still on the bus
-  int nchunks = p->N / pose_plan_s::kUploadChunkFrames;
+  int nchunks = n / pose_plan_s::kUploadChunkFrames;
   nchunks = nchunks < 1 ? 1 : (nchunks > pose_plan_s::kUploadChunks ? pose_plan_s::kUploadChunks : nchunks);
   {
-    const int per = (p->N + nchunks - 1) / nchunks;
+    const int per = (n + nchunks - 1) / nchunks;
     const size_t frame = static_cast<size_t>(4) * p->HW * p->HW;      // floats per 2HW x 2HW crop
     for (int c = 0; c < nchunks; ++c) {
-      const int n0 = c * per, nn = (n0 + per <= p->N ? per : p->N - n0);
+      const int n0 = c * per, nn = (n0 + per <= n ? per : n - n0);
       if (nn > 0)
         CUDA_TRY(cudaMemcpyAsync(p->depth.as<float>() + n0 * frame, depth_host + n0 * frame, nn * frame * sizeof(float),
                                  cudaMemcpyHostToDevice, p->copy_st));
       CUDA_TRY(cudaEventRecord(p->ev_chunk[c], p->copy_st));
     }
   }
-  int rc = pose_forward_impl(p, p->depth.as<float>(), H2_init, p->out.as<float>(), st, p->ev_chunk, nchunks);
+  int rc = pose_forward_impl(p, n, p->depth.as<float>(), H2_init, p->out.as<float>(), st, p->ev_chunk, nchunks);
   if (rc) return rc;
-  CUDA_TRY(cudaMemcpyAsync(out_host, p->out.p, p->out.bytes, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaMemcpyAsync(out_host, p->out.p, sizeof(float) * n * p->O, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(cudaStreamSynchronize(st));
   return 0;
 }
@@ -1175,8 +1210,8 @@ int pose_get_activation(pose_plan_t p, const char* name, float* dst, void* strea
   if ((is_pool1 || is_conv2) && p->mode != HGRU_MODE_FP32) {
     // tensor-core stem: the activation lives as bf16 hi | lo chunk planes
     const hgru_plan_s* h = &p->hg;
-    hgru::split_chunks_to_nhwc_kernel<<<nblk(h->npix * h->k), 256, 0, st>>>(
-        (is_pool1 ? p->act_pool1 : p->act_conv2).as<__nv_bfloat16>(), dst, h->npix, h->k, h->KP / 8, h->H * h->W);
+    hgru::split_chunks_to_nhwc_kernel<<<nblk(h->npix_n() * h->k), 256, 0, st>>>(
+        (is_pool1 ? p->act_pool1 : p->act_conv2).as<__nv_bfloat16>(), dst, h->npix_n(), h->k, h->KP / 8, h->H * h->W);
     CUDA_TRY(cudaGetLastError());
     return 0;
   }
@@ -1185,7 +1220,7 @@ int pose_get_activation(pose_plan_t p, const char* name, float* dst, void* strea
   else if (!strcmp(name, "conv3")) src = p->hg.Xp.as<float>();
   else if (!strcmp(name, "hgru")) src = p->hg.H2.as<float>();
   else if (!strcmp(name, "fc1")) {
-    CUDA_TRY(cudaMemcpyAsync(dst, p->fc1.p, p->fc1.bytes, cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(dst, p->fc1.p, sizeof(float) * p->hg.n * p->F, cudaMemcpyDeviceToDevice, st));
     return 0;
   } else return fail(HGRU_E_INVALID, std::string("pose_get_activation: unknown name ") + name);
   state_to_nhwc(&p->hg, src, dst, st);
@@ -1498,7 +1533,7 @@ int attn_plan_create(int N, int H, int W, const int* widths, int fc_hidden, int 
   for (int i = 0; i < 5; ++i)
     if (widths[i] < 8 || widths[i] % 8) return fail(HGRU_E_UNSUPPORTED, "attn_plan_create: widths must be multiples of 8");
   attn_plan_s* p = new attn_plan_s();
-  p->N = N; p->H = H; p->W = W; p->F = fc_hidden; p->O = O;
+  p->N = N; p->n = N; p->H = H; p->W = W; p->F = fc_hidden; p->O = O;
   for (int i = 0; i < 5; ++i) p->w[i] = widths[i];
   const int rc = attn_plan_build(p);
   if (rc) {
@@ -1524,20 +1559,27 @@ int attn_set_params(attn_plan_t plan, const attn_params_t* params, float bn_epsi
 
 int attn_forward(attn_plan_t plan, const float* frames_dev, float* out_dev, void* stream) {
   if (!plan) return fail(HGRU_E_INVALID, "attn_forward: null plan");
-  return attn_forward_impl(plan, frames_dev, out_dev, static_cast<cudaStream_t>(stream));
+  return attn_forward_impl(plan, plan->N, frames_dev, out_dev, static_cast<cudaStream_t>(stream));
+}
+
+int attn_forward_batch(attn_plan_t plan, int n, const float* frames_dev, float* out_dev, void* stream) {
+  if (!plan) return fail(HGRU_E_INVALID, "attn_forward_batch: null plan");
+  if (int rc = check_batch("attn_forward_batch", n, plan->N)) return rc;
+  return attn_forward_impl(plan, n, frames_dev, out_dev, static_cast<cudaStream_t>(stream));
 }
 
 int attn_get_activation(attn_plan_t plan, const char* name, float* dst, void* stream) {
   if (!plan || !name || !dst) return fail(HGRU_E_INVALID, "attn_get_activation: null pointer");
   const std::string n(name);
   const void* src = nullptr;
-  size_t bytes = 0;
+  size_t bytes = 0;      // (of the capacity N; the copy takes the last forward's n frames)
   if (n == "resized") { src = plan->resized.p; bytes = plan->resized.bytes; }
   else if (n == "fc1") { src = plan->fc1.p; bytes = plan->fc1.bytes; }
   else if (n.size() == 5 && n.compare(0, 4, "pool") == 0 && n[4] >= '1' && n[4] <= '5') {
     src = plan->pool[n[4] - '1'].p; bytes = plan->pool[n[4] - '1'].bytes;
   }
   if (!src) return fail(HGRU_E_INVALID, "attn_get_activation: unknown tensor name '" + n + "'");
+  bytes = bytes / plan->N * plan->n;
   CUDA_TRY(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream)));
   return 0;
 }

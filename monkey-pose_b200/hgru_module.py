@@ -58,8 +58,9 @@ def auxilliary_variables():
     }
 
 
-# Plans own their workspace (gigabytes at batch 256), so only the most recently used few shapes stay alive.
-_PLAN_CACHE = {}          # key -> plan handle, in least-recently-used order (dicts keep insertion order)
+# Plans own their workspace (gigabytes at batch 256), so only the most recently used few shapes stay alive.  A plan
+# serves every batch up to its capacity (hgru_forward_batch), so the batch size is not part of the key.
+_PLAN_CACHE = {}          # key -> (plan handle, capacity), in least-recently-used order (dicts keep insertion order)
 PLAN_CACHE_SIZE = 4
 
 
@@ -67,26 +68,32 @@ def clear_plan_cache():
     """Destroy every cached layer plan and free its device workspace."""
     lib = _lib.load()
     torch.cuda.synchronize()
-    for plan in _PLAN_CACHE.values():
+    for plan, _ in _PLAN_CACHE.values():
         lib.hgru_plan_destroy(plan)
     _PLAN_CACHE.clear()
 
 
 def _get_plan(N, H, W, k, S, T, mode):
-    key = (torch.cuda.current_device(), N, H, W, k, S, T, mode)
-    plan = _PLAN_CACHE.pop(key, None)
-    if plan is None:
+    """A plan of this shape that runs N frames: the cached one when its capacity is at least N, else a new plan for
+    N frames, which replaces a smaller cached one."""
+    key = (torch.cuda.current_device(), H, W, k, S, T, mode)
+    entry = _PLAN_CACHE.pop(key, None)
+    lib = _lib.load()
+    if entry is not None and entry[1] < N:
+        torch.cuda.synchronize()                            # (its last forward may still be running)
+        lib.hgru_plan_destroy(entry[0])
+        entry = None
+    if entry is None:
         import ctypes
-        lib = _lib.load()
         while len(_PLAN_CACHE) >= PLAN_CACHE_SIZE:          # evict the least recently used plan
             old = next(iter(_PLAN_CACHE))
             torch.cuda.synchronize()                        # (its last forward may still be running)
-            lib.hgru_plan_destroy(_PLAN_CACHE.pop(old))
+            lib.hgru_plan_destroy(_PLAN_CACHE.pop(old)[0])
         h = ctypes.c_void_p()
         _lib.check(lib.hgru_plan_create(N, H, W, k, S, T, mode, ctypes.byref(h)), "hgru_plan_create")
-        plan = h
-    _PLAN_CACHE[key] = plan          # (re)insert as most recently used
-    return plan
+        entry = (h, N)
+    _PLAN_CACHE[key] = entry          # (re)insert as most recently used
+    return entry[0]
 
 
 def _stream():
@@ -517,9 +524,9 @@ class ContextualCircuit(object):
         if trace:
             I_tr = torch.empty((self.timesteps,) + tuple(self.X.shape), device=self.X.device)
             O_tr = torch.empty_like(I_tr)
-        _lib.check(lib.hgru_forward(plan, self.X.data_ptr(), O0.data_ptr(), O.data_ptr(),
-                                    I_tr.data_ptr() if trace else None,
-                                    O_tr.data_ptr() if trace else None, st), "hgru_forward")
+        _lib.check(lib.hgru_forward_batch(plan, self.n, self.X.data_ptr(), O0.data_ptr(), O.data_ptr(),
+                                          I_tr.data_ptr() if trace else None,
+                                          O_tr.data_ptr() if trace else None, st), "hgru_forward_batch")
         self.I_steps, self.O_steps = I_tr, O_tr
         self.gpu_launches = lib.hgru_plan_launch_count(plan)
         if self.return_weights:

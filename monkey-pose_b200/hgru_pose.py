@@ -95,8 +95,9 @@ class model(LayerOps):
         self.dropout_seed = 1234      # train_mode=True: seed of the counter-based dropout mask
         self._plan = None
         self._plan_key = None
+        self._plan_capacity = 0       # frames the plan was created for: it runs every batch up to that size
         self._dev_params = None
-        self._h0_cache = None         # (key, device tensor) of the seeded O_0 draw
+        self._h0_cache = None         # (key, device tensor) of the seeded O_0 draw, at the plan's capacity
         self._lazy = {}
 
     def __getattr__(self, name):
@@ -275,15 +276,18 @@ class model(LayerOps):
             return self._build_layerwise(depth, output_shape, train_mode)
         lib = _lib.load()
         mode = _lib.MODES[self.compute_mode]
-        key = (torch.cuda.current_device(), N, hw, self.channels, S, self.timesteps, self.fc_hidden,
-               int(output_shape), mode)
-        if self._plan is None or key != self._plan_key:
+        # The plan key leaves out the batch: a plan runs any batch up to its capacity (pose_forward_batch) with no
+        # re-allocation and no re-packing of the weights.  A larger batch re-creates it at that size; capacity never
+        # shrinks.
+        key = (torch.cuda.current_device(), hw, self.channels, S, self.timesteps, self.fc_hidden, int(output_shape),
+               mode)
+        if self._plan is None or key != self._plan_key or N > self._plan_capacity:
             if self._plan is not None:
                 lib.pose_plan_destroy(self._plan)
             h = ctypes.c_void_p()
             _lib.check(lib.pose_plan_create(N, hw, self.channels, S, self.timesteps, self.fc_hidden,
                                             int(output_shape), mode, ctypes.byref(h)), "pose_plan_create")
-            self._plan, self._plan_key, self._dev_params = h, key, None
+            self._plan, self._plan_key, self._plan_capacity, self._dev_params = h, key, N, None
         st = _stream()
         if self._dev_params is None:
             P = self._materialise(int(depth.shape[-1]), hw, int(output_shape))
@@ -305,11 +309,13 @@ class model(LayerOps):
             if tuple(h0.shape) != (N, hw, hw, self.channels):
                 raise ValueError("hidden_state must be [N,%d,%d,%d]" % (hw, hw, self.channels))
         elif self.aux.get('hidden_init', 'random') == 'random':
-            # the seeded O_0 draw is made once per shape and kept on the device (268 MB at N = 256, 64 channels)
-            hkey = (torch.cuda.current_device(), N, hw, self.channels, self.seed)
+            # the seeded O_0 draw is made once per shape at the plan's capacity and kept on the device (268 MB at
+            # N = 256, 64 channels).  The generator fills in C order, so its first N frames are the draw of N frames.
+            cap = self._plan_capacity
+            hkey = (torch.cuda.current_device(), cap, hw, self.channels, self.seed)
             if self._h0_cache is None or self._h0_cache[0] != hkey:
-                self._h0_cache = (hkey, _as_dev(init.hidden_init((N, hw, hw, self.channels), seed=self.seed + 7)))
-            h0 = self._h0_cache[1]
+                self._h0_cache = (hkey, _as_dev(init.hidden_init((cap, hw, hw, self.channels), seed=self.seed + 7)))
+            h0 = self._h0_cache[1] if N == cap else self._h0_cache[1][:N]
         elif self.aux.get('hidden_init') not in ('zeros', 'identity'):
             raise RuntimeError("hidden_init must be 'random', 'zeros' or 'identity'")      # hgru_module.py:891-892
         # 'identity': O_0 = X = conv3 of this forward (hgru_module.py:876-878), taken inside the library
@@ -319,11 +325,12 @@ class model(LayerOps):
         h0_ptr = h0.data_ptr() if h0 is not None else None
         if depth.is_cuda:
             out = torch.empty((N, int(output_shape)), device=depth.device, dtype=torch.float32)
-            _lib.check(lib.pose_forward(self._plan, depth.data_ptr(), h0_ptr, out.data_ptr(), st), "pose_forward")
+            _lib.check(lib.pose_forward_batch(self._plan, N, depth.data_ptr(), h0_ptr, out.data_ptr(), st),
+                       "pose_forward_batch")
         else:
             out = torch.empty((N, int(output_shape)), dtype=torch.float32, pin_memory=True)
-            _lib.check(lib.pose_forward_host(self._plan, depth.data_ptr(), h0_ptr, out.data_ptr(), st),
-                       "pose_forward_host")
+            _lib.check(lib.pose_forward_host_batch(self._plan, N, depth.data_ptr(), h0_ptr, out.data_ptr(), st),
+                       "pose_forward_host_batch")
         self.gpu_launches = lib.pose_plan_launch_count(self._plan)
         act = (N, hw, hw, self.channels)
         self._act = {"pool1": _Lazy(self, "pool1", act), "conv2": _Lazy(self, "conv2", act),
