@@ -73,7 +73,7 @@ int run_case(int N, int H, int W, int k, int grid_override, int iters) {
   if (hgru::make_act_tensor_map(&map, d_act, N, CG, HA, W, Cfg::COLS, Cfg::ROWS, Cfg::PART_CHUNKS)) { printf("map fail\n"); return 1; }
   hgru::TcConvArgs a{};
   a.N = N; a.H = H; a.W = W; a.KP = KP; a.kreal = k; a.act_pad = PADR;
-  a.units_x = (W + 63) / 64; a.units_y = (H + 15) / 16; a.num_units = N * a.units_x * a.units_y;
+  a.units_x = (W + 63) / 64; a.units_y = (H + 15) / 16; a.num_units = N * a.units_x * a.units_y; a.unit_tiles = Cfg::MAXNTO;
   a.wpk = d_wpk; a.bias = d_bias; a.out = d_out;
   auto kern = hgru::hconv_stack_kernel<KP, T, KC, hgru::EpiBias>;
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
@@ -147,7 +147,7 @@ void time_real_epilogue(const char* name, int N, int H, int W, int k, int gate =
   hgru::make_act_tensor_map(&map, act, N, CG, HA, W, Cfg::COLS, Cfg::ROWS, Cfg::PART_CHUNKS);
   hgru::TcConvArgs a{};
   a.N = N; a.H = H; a.W = W; a.KP = KP; a.kreal = k; a.act_pad = Cfg::ACT_PAD;
-  a.units_x = (W + 63) / 64; a.units_y = (H + 15) / 16; a.num_units = N * a.units_x * a.units_y;
+  a.units_x = (W + 63) / 64; a.units_y = (H + 15) / 16; a.num_units = N * a.units_x * a.units_y; a.unit_tiles = Cfg::MAXNTO;
   a.wpk = wpk; a.bias = vec; a.v0 = vec + KP; a.v1 = vec + 2 * KP; a.v2 = vec + 3 * KP; a.rho_t = vec + 4 * KP;
   a.X = X; a.H1 = H1; a.G = G; a.H2 = H2; a.out = H1; a.out_bf16 = actout;
   a.gate_wpk = wpk; a.gate_bias = vec; a.gate_out = G; a.gate_act_out = actout; a.do_gate = gate; a.dbg_flags = dbg;

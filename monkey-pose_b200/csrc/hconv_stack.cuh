@@ -20,6 +20,13 @@
 // weights (288 KB at k = 25 with the remainder-packed schedule) stream through a ring (5 stages at k = 25) once per
 // tile pair.  Tap group 0 of a row's first carry tile only reads zero-filled window columns and is not issued.
 //
+// Narrow units (TcConvArgs::unit_tiles = 1): 16 rows x 8 columns = 1 carry tile + 1 output tile, one tile pair, for
+// batches too small to fill the SMs with wide units.  The window, its TMA box and the weight schedule are those of
+// the wide unit (the unused columns cost nothing at such batch sizes).  A narrow unit's carry tile is an output tile
+// of a wide unit: it gets every tap group (unless it starts at image column 0, where the wide unit's carry tile
+// skips group 0 too) through the same stage sequence, so its accumulator, the carry taken from it and every output
+// are bitwise those of the wide unit -- a frame's result does not depend on the unit width.
+//
 // Launch chaining: the launches of one forward depend on each other only frame by frame (a unit needs the four
 // units of its frame from the previous launch), so instead of grid-wide stream order each unit's epilogue counts
 // itself done in a per-launch, per-frame counter (TcConvArgs::done_flags) and the next launch -- started early by
@@ -449,7 +456,7 @@ __device__ __forceinline__ void stack_epilogue(const TcConvArgs& a, const int C0
     for (int j = 0; j < NT; ++j, ++tc) {
       const uint32_t slot = tc & 3;
       // this thread's output pixel; its global inputs are fetched while the MMAs still run
-      const int x = ux * 64 + 8 * (j - 1) + pcol;
+      const int x = ux * (8 * a.unit_tiles) + 8 * (j - 1) + pcol;
       const bool store = j >= 1 && y < a.H && x < a.W;
       const size_t pin = static_cast<size_t>(y) * a.W + x;
       typename Epi::template Pre<NCH> pre;
@@ -701,7 +708,8 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs 
 
   const int iters = (a.num_units + static_cast<int>(gridDim.x) - 1) / static_cast<int>(gridDim.x);
   const int units_per_frame = a.units_x * a.units_y;
-  const int wseg = a.W < 64 ? a.W : 64;
+  const int ucols = 8 * a.unit_tiles;              // image columns per unit
+  const int wseg = a.W < ucols ? a.W : ucols;
   const int NT = 1 + (wseg + 7) / 8;               // carry tile + output tiles, uniform over units
   const int npairs = (NT + 1) / 2;
 
@@ -743,12 +751,12 @@ hconv_stack_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs 
         }
         mbar_wait(bar_win_empty, (vit & 1) ^ 1);
         mbar_arrive_expect_tx(bar_win_full, Cfg::PART_BYTES);
-        tma_load_4d(win, &in_map, bar_win_full, 2 * (ux * 64 + Cfg::MIN_COL),
+        tma_load_4d(win, &in_map, bar_win_full, 2 * (ux * ucols + Cfg::MIN_COL),
                     uy * kTileRows - Cfg::PAD + Cfg::ACT_PAD, 0, n);
         if constexpr (Cfg::WPARTS == 2) {
           mbar_wait(bar_win_empty + 8, (vit & 1) ^ 1);
           mbar_arrive_expect_tx(bar_win_full + 8, Cfg::PART_BYTES);
-          tma_load_4d(win + Cfg::PART_BYTES, &in_map, bar_win_full + 8, 2 * (ux * 64 + Cfg::MIN_COL),
+          tma_load_4d(win + Cfg::PART_BYTES, &in_map, bar_win_full + 8, 2 * (ux * ucols + Cfg::MIN_COL),
                       uy * kTileRows - Cfg::PAD + Cfg::ACT_PAD, Cfg::PART_CHUNKS, n);
         }
         ++vit;

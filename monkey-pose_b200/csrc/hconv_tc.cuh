@@ -21,7 +21,7 @@
 // reused by all S*S taps.
 //
 // CTA = 8 warps: w0 weight producer, w1 MMA issuer, w2 TMEM allocator, w3 input producer,
-// w4..7 epilogue (TMEM -> registers -> global).  Persistent over "units" (16 x 8*TILES_X pixels
+// w4..7 epilogue (TMEM -> registers -> global).  Persistent over "units" (16 x 8*UT pixels
 // of one frame); two TMEM accumulator sets so unit u's epilogue overlaps unit u+1's MMAs.
 #pragma once
 #include <cuda_bf16.h>
@@ -47,7 +47,10 @@ constexpr int kTileRows = 16;   // M tile = 16 rows x 8 cols of pixels
 // the epilogue as tcgen05.mma on a shared-memory staging tile of the new state (as in hconv_stack.cuh), and the
 // launches of a forward are chained through per-frame completion counters (TcConvArgs::wait_flags / done_flags):
 // two launches per timestep instead of four, no grid-wide stream order between them.
-template <int S, int KSTEPS, int CO_PAD, int TILES_X, int G, int WSTAGES, bool SPLIT3 = false, bool FUSE = false>
+// UT: tiles per unit, TILES_X (the window's width in tiles) or fewer: the narrow units of the fused 64-channel kernel,
+// for batches too small to fill the SMs with wide units.  Its window and TMA box stay those of TILES_X.
+template <int S, int KSTEPS, int CO_PAD, int TILES_X, int G, int WSTAGES, bool SPLIT3 = false, bool FUSE = false,
+          int UT = TILES_X>
 struct TcConvCfg {
   static constexpr int kParts = SPLIT3 ? 2 * KSTEPS : KSTEPS;      // window parts (TMA boxes / barriers)
   static constexpr int kWSteps = SPLIT3 ? 2 * KSTEPS : KSTEPS;     // weight k-steps (SPLIT3: wide a_hi pass, a_lo pass)
@@ -75,7 +78,8 @@ struct TcConvCfg {
   static constexpr int kStageBytes = kPairTap ? 2 * kPairBlockBytes : G * kTapBytesWide;
   static constexpr int kStagesPerKstep = kPairTap ? S * 4 : kTaps / G;
   static constexpr int kAccN = SPLIT3 ? 2 * CO_PAD : CO_PAD; // accumulator columns per tile
-  static constexpr int kAccCols = TILES_X * kAccN;          // TMEM columns per accumulator set
+  static constexpr int kUnitTiles = UT;
+  static constexpr int kAccCols = UT * kAccN;               // TMEM columns per accumulator set
   static constexpr int kGateABytes = FUSE ? (CO_PAD / 8) * 128 * 16 : 0;   // staging tile of the new state (bf16, K-major)
   static constexpr int kGateWBytes = FUSE ? KSTEPS * 2 * CO_PAD * 16 : 0;   // packed 1x1 gate weights
   static constexpr int kGateBytes = kGateABytes + kGateWBytes;
@@ -86,6 +90,7 @@ struct TcConvCfg {
   static_assert(kSmemBytes <= 232448, "shared memory per CTA");
   static_assert(kPairTap || kTaps % G == 0, "taps per stage must divide S*S");
   static_assert(!kPairTap || (S == 15 && CO_PAD == 64 && TILES_X == 4 && !SPLIT3), "paired-tap schedule: 64 channels, 15x15");
+  static_assert(UT >= 1 && UT <= TILES_X && (kPairTap || UT == TILES_X), "narrow units: paired-tap schedule only");
   static_assert(2 * kAccCols <= 512, "two accumulator sets must fit TMEM");
   static_assert(CO_PAD % 16 == 0 && CO_PAD >= 16 && kAccN <= 256, "UMMA N constraint (M=128)");
   static_assert(kChunkPitch % 16 == 0 && (kChunkPitch >> 4) < 16384, "LBO range");
@@ -155,6 +160,8 @@ struct TcConvArgs {
   // its power-limited one): the MMA issuer of CTA b stores {clock64 cycles, %globaltimer nanoseconds} it spent in
   // its loop at clk_out[2b], clk_out[2b + 1].  nullptr = off.
   unsigned long long* clk_out;
+  // Tap-stacked kernel: output tiles (8 columns each) per unit, StackCfg::MAXNTO or 1 (chosen by launch_stack).
+  int unit_tiles;
 };
 
 __device__ __forceinline__ unsigned long long global_timer_ns() {
@@ -712,12 +719,13 @@ struct EpiGateIn {
 };
 
 // F: format of the 16-bit operands (op_format.cuh); fp16 exists for the FUSE path (its Epi writes the same format).
+// UT: tiles per unit (TcConvCfg).
 template <int S, int KSTEPS, int CO_PAD, int TILES_X, int G, int WSTAGES, class Epi, bool SPLIT3 = false,
-          bool FUSE = false, class F = OpBf16>
+          bool FUSE = false, class F = OpBf16, int UT = TILES_X>
 __global__ void __launch_bounds__(256, 1)
 hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) {
   using namespace sm100;
-  using Cfg = TcConvCfg<S, KSTEPS, CO_PAD, TILES_X, G, WSTAGES, SPLIT3, FUSE>;
+  using Cfg = TcConvCfg<S, KSTEPS, CO_PAD, TILES_X, G, WSTAGES, SPLIT3, FUSE, UT>;
   constexpr int NP = Cfg::kParts, NW = Cfg::kWSteps;
   static_assert(!FUSE || !SPLIT3, "the fused-gate epilogue serves the plain bf16 path");
   static_assert(FUSE || F::kIdescFmt == OpBf16::kIdescFmt, "16-bit operand formats other than bf16: FUSE path only");
@@ -815,7 +823,7 @@ hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) 
         const int n = a.n0 + nl;
         const int uy = r / a.units_x, ux = r - uy * a.units_x;
         const int y0 = uy * kTileRows - Cfg::kPad;
-        const int x0 = ux * (8 * TILES_X) - Cfg::kPad;
+        const int x0 = ux * (8 * UT) - Cfg::kPad;
         if constexpr (FUSE) {
           if (a.wait_flags) {
             // chained launch: this frame's operand is complete once all its units finished in the previous launch
@@ -882,17 +890,19 @@ hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) 
                 // tap 7 alone, every tile: the first instructions of a unit (they overwrite the accumulators)
                 const uint32_t accum = (wq | dy) != 0;
 #pragma unroll
-                for (int t = 0; t < 4; ++t)
+                for (int t = 0; t < UT; ++t)
                   if (leader) mma_bf16_ss(acc + t * 64, a_row + static_cast<uint64_t>(8 * t + 7), b_blk, idesc_n, accum);
               } else {
                 const int pdx = blk - 1;      // rows 0-63 of the block: tap pdx + 8, rows 64-127: tap pdx
                 if (leader) {
-                  // tile 0 has no left neighbour for its low taps, tile 3 no right neighbour for its high taps
+                  // tile 0 has no left neighbour for its low taps, the last tile no right neighbour for its high
+                  // taps.  Every tile gets tap pdx, then tap pdx + 8, whatever UT: the same K order in every unit.
                   mma_bf16_ss(acc, a_row + static_cast<uint64_t>(pdx), b_blk + (1024 >> 4), idesc_n, 1u);
 #pragma unroll
-                  for (int t = 1; t < 4; ++t)
+                  for (int t = 1; t < UT; ++t)
                     mma_bf16_ss(acc + (t - 1) * 64, a_row + static_cast<uint64_t>(8 * t + pdx), b_blk, idesc_p, 1u);
-                  mma_bf16_ss(acc + 3 * 64, a_row + static_cast<uint64_t>(24 + pdx + 8), b_blk, idesc_n, 1u);
+                  mma_bf16_ss(acc + (UT - 1) * 64, a_row + static_cast<uint64_t>(8 * (UT - 1) + pdx + 8), b_blk, idesc_n,
+                              1u);
                 }
               }
             }
@@ -910,7 +920,7 @@ hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) 
             const uint64_t adesc_tap = adesc_q + tap_off;
             const uint32_t accum = (wq | sg | g) != 0;
 #pragma unroll
-            for (int t = 0; t < TILES_X; ++t) {
+            for (int t = 0; t < UT; ++t) {
               if (leader) mma_bf16_ss(acc + t * Cfg::kAccN, adesc_tap + static_cast<uint64_t>(t * 8), bdesc, idesc, accum);
             }
             // next tap: dx+1, wrapping to the next filter row
@@ -955,8 +965,8 @@ hconv_tc_kernel(const __grid_constant__ CUtensorMap in_map, const TcConvArgs a) 
       mbar_wait(bar_acc_full + 8 * s, (it >> 1) & 1);
       tc_fence_after();
 #pragma unroll 1
-      for (int t = 0; t < TILES_X; ++t) {
-        const int x = ux * (8 * TILES_X) + t * 8 + pcol;
+      for (int t = 0; t < UT; ++t) {
+        const int x = ux * (8 * UT) + t * 8 + pcol;
         const bool ok = (y < a.H) && (x < a.W);
         const uint32_t taddr =
             tmem_base + (static_cast<uint32_t>(ew * 32) << 16) + s * Cfg::kAccCols + t * Cfg::kAccN;

@@ -57,6 +57,16 @@ inline int sm_count(int* out) {
   return 0;
 }
 
+// Unit width of the hGRU conv launches (tap-stacked and fused 64-channel kernels).  Narrow units give a small batch
+// more CTAs at the price of more tensor-core work per output pixel; the width changes no value, so it is picked for
+// speed alone, from the launch's frame count, and all conv launches of a forward get the same one (the per-frame
+// chaining counters count units).  Estimated launch time = waves (units over SMs, rounded up) x tensor-core
+// instructions per unit; narrow only when strictly cheaper, so full batches keep the wide units.
+inline bool narrow_units_faster(int units_wide, int work_wide, int units_narrow, int work_narrow, int sms) {
+  const long long waves_wide = (units_wide + sms - 1) / sms, waves_narrow = (units_narrow + sms - 1) / sms;
+  return waves_narrow * work_narrow < waves_wide * work_wide;
+}
+
 inline unsigned nblk(size_t n, int b = 256) { return static_cast<unsigned>((n + b - 1) / b); }
 inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 

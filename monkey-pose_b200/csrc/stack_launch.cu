@@ -44,11 +44,16 @@ int launch_stack(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t st) {
   using Cfg = hgru::StackCfg<KP, T, KC, GX3, F>;
   auto kern = hgru::hconv_stack_kernel<KP, T, KC, Epi, false, WSETS, PART, GX3, F>;
   SMEM_ATTR_ONCE(kern, Cfg::SMEM_BYTES);
-  a.units_x = (a.W + 63) / 64;
-  a.units_y = (a.H + hgru::kTileRows - 1) / hgru::kTileRows;
-  a.num_units = a.N * a.units_x * a.units_y;
   int sms = 0, rc = sm_count(&sms);
   if (rc) return rc;
+  // wide units (8 output tiles) or narrow ones (1); work = tiles per unit, the carry tile included
+  a.units_y = (a.H + hgru::kTileRows - 1) / hgru::kTileRows;
+  const int wide_x = (a.W + 8 * Cfg::MAXNTO - 1) / (8 * Cfg::MAXNTO), narrow_x = (a.W + 7) / 8;
+  const int wide_tiles = 1 + ((a.W < 8 * Cfg::MAXNTO ? a.W : 8 * Cfg::MAXNTO) + 7) / 8;
+  const bool narrow = narrow_units_faster(a.N * wide_x * a.units_y, wide_tiles, a.N * narrow_x * a.units_y, 2, sms);
+  a.unit_tiles = narrow ? 1 : Cfg::MAXNTO;
+  a.units_x = narrow ? narrow_x : wide_x;
+  a.num_units = a.N * a.units_x * a.units_y;
   const int grid = a.num_units < sms ? a.num_units : sms;
   a.flag_target = a.units_x * a.units_y;
   // A launch that waits on the previous launch's per-frame counters is chained to it (programmatic dependent

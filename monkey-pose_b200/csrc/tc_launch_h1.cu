@@ -45,17 +45,16 @@ int dispatch_tc_hconv(int S, int KP, const CUtensorMap& map, const hgru::TcConvA
 // 64 channels, 15x15 (the reference's own width): the same kernel with the 1x1 gate convs issued from its epilogue
 // and the launches of a forward chained per frame (TcConvCfg FUSE) -- two launches per timestep.  Three weight
 // stages instead of four make room for the gate's staging tile and weights.
-template <class Epi, class F = hgru::OpBf16, int G = 5, int WS = 3>
-int launch_tc_fused64(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t st) {
-  using Cfg = hgru::TcConvCfg<15, 4, 64, 4, G, WS, false, true>;
-  auto kern = hgru::hconv_tc_kernel<15, 4, 64, 4, G, WS, Epi, false, true, F>;
+// UT: tiles per unit, 4 (wide) or 2 (narrow, see launch_tc_fused64).
+template <class Epi, class F, int UT, int G = 5, int WS = 3>
+int launch_tc_fused64_ut(const CUtensorMap& map, hgru::TcConvArgs a, int sms, cudaStream_t st) {
+  using Cfg = hgru::TcConvCfg<15, 4, 64, 4, G, WS, false, true, UT>;
+  auto kern = hgru::hconv_tc_kernel<15, 4, 64, 4, G, WS, Epi, false, true, F, UT>;
   SMEM_ATTR_ONCE(kern, Cfg::kSmemBytes);
-  a.units_x = (a.W + 31) / 32;
+  a.units_x = (a.W + 8 * UT - 1) / (8 * UT);
   a.units_y = (a.H + hgru::kTileRows - 1) / hgru::kTileRows;
   a.num_units = a.N * a.units_x * a.units_y;
   a.flag_target = a.units_x * a.units_y;
-  int sms = 0, rc = sm_count(&sms);
-  if (rc) return rc;
   const int grid = a.num_units < sms ? a.num_units : sms;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid); cfg.blockDim = dim3(256); cfg.dynamicSmemBytes = Cfg::kSmemBytes; cfg.stream = st;
@@ -65,6 +64,16 @@ int launch_tc_fused64(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t s
   cfg.attrs = at; cfg.numAttrs = a.wait_flags ? 1 : 0;
   CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, map, a));
   return 0;
+}
+// Wide units (4 tiles) or narrow ones (2 tiles); work = paired-tap instructions per filter row, 8 UT + 7.
+template <class Epi, class F = hgru::OpBf16>
+int launch_tc_fused64(const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st) {
+  int sms = 0, rc = sm_count(&sms);
+  if (rc) return rc;
+  const int units_y = (a.H + hgru::kTileRows - 1) / hgru::kTileRows;
+  if (narrow_units_faster(a.N * ((a.W + 31) / 32) * units_y, 39, a.N * ((a.W + 15) / 16) * units_y, 23, sms))
+    return launch_tc_fused64_ut<Epi, F, 2>(map, a, sms, st);
+  return launch_tc_fused64_ut<Epi, F, 4>(map, a, sms, st);
 }
 
 // bf16x3 mode at 64 channels: the 15x15 horizontal convs on hi/lo operand splits (narrower layers run it on the
