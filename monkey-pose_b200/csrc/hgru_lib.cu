@@ -21,6 +21,7 @@
 #include "layers.cuh"
 #include "simt_kernels.cuh"
 #include <algorithm>
+#include <array>
 
 #include "attn.cuh"
 #include "tc_host.cuh"
@@ -183,7 +184,7 @@ struct hgru_plan_s {
   DevBuf Xp, H2, H1, C, G, A;
   // bf16 chunked operand copies (tensor-core mode)
   DevBuf actA, actH1, actH2;
-  DevBuf flags;                     // launch chaining: [2T][N] per-frame completion counters (stacked kernel)
+  DevBuf flags;                     // launch chaining: [conv launches per timestep x T][N] per-frame completion counters
   DevBuf clk;                       // in-kernel clock samples of the last conv launch: [CTA][2] (cycles, ns)
   bool chain = false;
   CUtensorMap mapA, mapH1;          // SxS halo-window boxes (horizontal convs)
@@ -197,6 +198,7 @@ struct hgru_plan_s {
   int fc_kpad = 0;
   bool stacked = false;             // narrow layers: tap-stacked kernel (hconv_stack.cuh)
   bool fused_tc = false;            // 64 channels, 15x15: hconv_tc_kernel with epilogue-issued gates, chained (FUSE)
+  bool epi_gates = false;           // the 1x1 gates run in the conv launches' epilogues (else as launches of their own)
   int stack_T = 0;
   int act_pad = 0;                  // pad rows of the bf16 operand planes (remainder-packed layout)
   bool state_ready = false;         // the caller already ran hgru_init_state_bf16 for the coming forward
@@ -207,10 +209,17 @@ struct hgru_plan_s {
   float* vec(int i) const { return vecs.as<float>() + static_cast<size_t>(i) * KP; }
   size_t npix_n() const { return static_cast<size_t>(n) * H * W; }      // pixels, padded elements of n frames
   size_t nelem_n() const { return npix_n() * KP; }
+  // launches per conv: two on the bf16x3 tap-stacked path (EPI_PARTIAL into C, then the launch that adds C), else one
+  int conv_parts() const { return mode == HGRU_MODE_BF16X3 && stacked ? 2 : 1; }
+  // every device buffer: what workspace() counts is what hgru_plan_free releases
+  template <class P> static auto buffers(P* p) {
+    return std::array{&p->p_r, &p->i_r, &p->o_r, &p->vecs, &p->rho, &p->wpk, &p->wpk_i, &p->wpk_o, &p->Xp, &p->H2,
+                      &p->H1, &p->C, &p->G, &p->A, &p->actA, &p->actH1, &p->actH2, &p->flags, &p->clk};
+  }
   size_t workspace() const {
-    return p_r.bytes + i_r.bytes + o_r.bytes + vecs.bytes + rho.bytes + wpk.bytes + wpk_i.bytes +
-           wpk_o.bytes + Xp.bytes + H2.bytes + H1.bytes + C.bytes + G.bytes + A.bytes + actA.bytes +
-           actH1.bytes + actH2.bytes + flags.bytes + clk.bytes;
+    size_t b = 0;
+    for (auto buf : buffers(this)) b += buf->bytes;
+    return b;
   }
 };
 
@@ -245,106 +254,90 @@ static int hgru_plan_init(hgru_plan_s* p, int N, int H, int W, int k, int S, int
     if ((rc = p->A.alloc(act)) || (rc = p->C.alloc(act)) ||
         (rc = p->p_r.alloc(sizeof(float) * S * S * p->KP * p->KP)))
       return rc;
-  } else if (mode == HGRU_MODE_BF16X3) {
-    StackGeom sg;
-    if (stack_geometry(S, p->KP, k, &sg)) {
-      // Narrow layers: the tap-stacked kernel, two launches per conv.  The first reads the a_lo operand against w_hi
-      // and leaves fp32 sums in C; the second reads a_hi against the weight sets w_hi and w_lo (accumulated in TMEM),
-      // adds C and runs the integration epilogue -- the launch with the heavy epilogue is the one with twice the MMAs
-      // to hide it behind.  Operands are two tensors (hi, lo) in the stacked kernel's layout.
-      p->stacked = true;
-      p->stack_T = sg.T;
-      p->act_pad = sg.act_pad;
-      const int HA = H + p->act_pad;
-      const size_t tb = static_cast<size_t>(N) * p->CG * HA * W * 8 * sizeof(__nv_bfloat16);
-      p->lo_off = tb / sizeof(__nv_bfloat16);
-      if ((rc = p->actA.alloc(2 * tb)) || (rc = p->actH1.alloc(2 * tb)) || (rc = p->C.alloc(act))) return rc;
-      CUDA_TRY(cudaMemset(p->actA.p, 0, 2 * tb));
-      CUDA_TRY(cudaMemset(p->actH1.p, 0, 2 * tb));
-      const size_t set = sizeof(__nv_bfloat16) * sg.stages * sg.NG * 2 * 128 * 8;
-      if ((rc = p->wpk.alloc(2 * set))) return rc;
-      // 1x1 gate weights in the SPLIT3 packing ([w_hi | w_lo] wide block + w_hi per 16 input channels)
-      const size_t gw = sizeof(__nv_bfloat16) * 3 * (p->KP / 16) * 2 * p->KP * 8;
-      if ((rc = p->wpk_i.alloc(gw)) || (rc = p->wpk_o.alloc(gw))) return rc;
-      {
-        const char* nc = getenv("HGRU_NO_CHAIN");
-        p->chain = !(nc && nc[0] == '1');
-        if (p->chain && (rc = p->flags.alloc(sizeof(int) * 4 * static_cast<size_t>(T) * N))) return rc;
-      }
-      const int box_chunks = sg.act_pad ? p->CG / 2 : p->CG;
-      char* a0 = static_cast<char*>(p->actA.p);
-      char* h0 = static_cast<char*>(p->actH1.p);
-      if (hgru::make_act_tensor_map(&p->mapA, a0, N, p->CG, HA, W, sg.box_cols, sg.box_rows, box_chunks) ||
-          hgru::make_act_tensor_map(&p->mapA_lo, a0 + tb, N, p->CG, HA, W, sg.box_cols, sg.box_rows, box_chunks) ||
-          hgru::make_act_tensor_map(&p->mapH1, h0, N, p->CG, HA, W, sg.box_cols, sg.box_rows, box_chunks) ||
-          hgru::make_act_tensor_map(&p->mapH1_lo, h0 + tb, N, p->CG, HA, W, sg.box_cols, sg.box_rows, box_chunks))
-        return fail(HGRU_E_CUDA, "cuTensorMapEncodeTiled failed");
-      return 0;
-    }
-    TcGeom g;
-    if (!x3_geometry(S, p->KP, &g))
-      return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: bf16x3 mode supports S = 15 and k <= 64");
-    // operands carry hi and lo bf16 halves: 2*CG chunk planes per frame
-    const size_t ab = 2 * p->nelem * sizeof(__nv_bfloat16);
-    if ((rc = p->actA.alloc(ab)) || (rc = p->actH1.alloc(ab))) return rc;
-    const int ksteps = p->KP / 16;
-    if ((rc = p->wpk.alloc(sizeof(__nv_bfloat16) * 3 * ksteps * S * S * 2 * p->KP * 8))) return rc;
-    if (hgru::make_act_tensor_map(&p->mapA, p->actA.p, N, 2 * p->CG, H, W, g.box_cols, g.box_rows) ||
-        hgru::make_act_tensor_map(&p->mapH1, p->actH1.p, N, 2 * p->CG, H, W, g.box_cols, g.box_rows))
-      return fail(HGRU_E_CUDA, "cuTensorMapEncodeTiled failed");
-  } else {
-    TcGeom g;
-    if (!tc_geometry(S, p->KP, &g))
-      return fail(HGRU_E_UNSUPPORTED, "hgru_plan_create: bf16 mode supports S in {1,3,5,7,15} and k <= 64");
-    // (bf16 and fp16 modes; the fp16 mode's shapes were checked above)
-    const int ksteps = p->KP / 16;
-    const size_t tapb = sizeof(__nv_bfloat16) * ksteps * 2 * p->KP * 8;
-    StackGeom sg;
-    p->stacked = stack_geometry(S, p->KP, k, &sg);
-    int box_cols = g.box_cols, box_rows = g.box_rows, box_chunks = 2;
-    size_t wbytes = tapb * S * S;
-    p->fused_tc = !p->stacked && S == 15 && p->KP == 64;
-    if (p->fused_tc) wbytes = sizeof(__nv_bfloat16) * ksteps * 15 * 8 * 2 * 128 * 8;      // paired-tap blocks
-    if (p->stacked || p->fused_tc) {
-      // consecutive conv launches are chained through per-frame counters (HGRU_NO_CHAIN=1: plain stream order)
-      const char* nc = getenv("HGRU_NO_CHAIN");
-      p->chain = !(nc && nc[0] == '1');
-      if (p->chain && (rc = p->flags.alloc(sizeof(int) * 2 * static_cast<size_t>(T) * N))) return rc;
-    }
-    if (p->stacked) {
-      p->stack_T = sg.T;
-      p->act_pad = sg.act_pad;
-      box_cols = sg.box_cols; box_rows = sg.box_rows;
-      box_chunks = sg.act_pad ? p->CG / 2 : p->CG;      // remainder-packed kernel loads the window in two parts
-      wbytes = sizeof(__nv_bfloat16) * sg.stages * sg.NG * 2 * 128 * 8;
-    }
-    // operand planes carry act_pad zero rows on top in the remainder-packed layout; they (and the never
-    // written tail elements of the row-packed plane) must read as zero, so the buffers are cleared once
-    const int HA = H + p->act_pad;
-    const size_t ab = static_cast<size_t>(N) * p->CG * HA * W * 8 * sizeof(__nv_bfloat16);
-    if ((rc = p->actA.alloc(ab)) || (rc = p->actH1.alloc(ab)) || (rc = p->actH2.alloc(ab))) return rc;
-    // (cudaMemset on device memory is asynchronous and the kernels run on non-blocking streams: hgru_plan_init's
-    // caller synchronises the device once after all clears, see plan_clears_done)
-    CUDA_TRY(cudaMemset(p->actA.p, 0, ab));
-    CUDA_TRY(cudaMemset(p->actH1.p, 0, ab));
-    if ((rc = p->wpk.alloc(wbytes)) || (rc = p->wpk_i.alloc(tapb)) || (rc = p->wpk_o.alloc(tapb))) return rc;
+    return 0;
+  }
+  // tensor-core modes: the tap-stacked kernel for narrow 15x15 layers, else hconv_tc_kernel (FUSE at 64 channels in
+  // the bf16 / fp16 modes, SPLIT3 in the bf16x3 mode)
+  const bool x3 = mode == HGRU_MODE_BF16X3;
+  StackGeom sg{};
+  TcGeom g{};
+  p->stacked = stack_geometry(S, p->KP, k, &sg);
+  if (!p->stacked && !(x3 ? x3_geometry(S, p->KP, &g) : tc_geometry(S, p->KP, &g)))
+    return fail(HGRU_E_UNSUPPORTED, x3 ? "hgru_plan_create: bf16x3 mode supports S = 15 and k <= 64"
+                                      : "hgru_plan_create: bf16 mode supports S in {1,3,5,7,15} and k <= 64");
+  p->fused_tc = !x3 && !p->stacked && S == 15 && p->KP == 64;
+  // bf16x3 at 32 channels keeps its gates in the exact SIMT kernel: see launch_stack
+  p->epi_gates = x3 ? p->stacked && !(p->KP == 32 && sg.T == 4) : p->stacked || p->fused_tc;
+  int box_cols = g.box_cols, box_rows = g.box_rows, box_chunks = 2;
+  if (p->stacked) {
+    p->stack_T = sg.T;
+    p->act_pad = sg.act_pad;
+    box_cols = sg.box_cols; box_rows = sg.box_rows;
+    box_chunks = sg.act_pad ? p->CG / 2 : p->CG;      // remainder-packed kernel loads the window in two parts
+  }
+  if (p->stacked || p->fused_tc) {
+    // consecutive conv launches are chained through per-frame counters (HGRU_NO_CHAIN=1: plain stream order)
+    const char* nc = getenv("HGRU_NO_CHAIN");
+    p->chain = !(nc && nc[0] == '1');
+    const size_t launches = 2 * static_cast<size_t>(p->conv_parts()) * T;
+    if (p->chain && (rc = p->flags.alloc(sizeof(int) * launches * N))) return rc;
+  }
+  // 16-bit operand planes.  bf16x3 carries hi and lo halves: on the stacked kernel two tensors, the lo one lo_off
+  // elements behind the hi one (the first launch of a conv reads a_lo, the second a_hi), else 2 * CG chunk planes per
+  // frame.  In the remainder-packed layout the planes carry act_pad zero rows on top; they (and the never written tail
+  // elements of the row-packed plane) must read as zero, so the buffers are cleared once.
+  const int HA = H + p->act_pad;
+  const size_t plane = static_cast<size_t>(N) * p->CG * HA * W * 8 * sizeof(__nv_bfloat16);
+  const size_t ab = x3 ? 2 * plane : plane;
+  if ((rc = p->actA.alloc(ab)) || (rc = p->actH1.alloc(ab)) || (!x3 && (rc = p->actH2.alloc(ab)))) return rc;
+  // (cudaMemset on device memory is asynchronous and the kernels run on non-blocking streams: hgru_plan_init's
+  // caller synchronises the device once after all clears, see plan_clears_done)
+  CUDA_TRY(cudaMemset(p->actA.p, 0, ab));
+  CUDA_TRY(cudaMemset(p->actH1.p, 0, ab));
+  if (p->conv_parts() == 2) {
+    p->lo_off = plane / sizeof(__nv_bfloat16);
+    if ((rc = p->C.alloc(act))) return rc;
+  }
+  // packed weights: the 15x15 (or SxS) conv, and the 1x1 gates where a tensor-core kernel issues them
+  const int ksteps = p->KP / 16;
+  const size_t tapb = sizeof(__nv_bfloat16) * ksteps * 2 * p->KP * 8;      // one tap, 16-bit operands
+  const size_t stack_set = p->stacked ? sizeof(__nv_bfloat16) * sg.stages * sg.NG * 2 * 128 * 8 : 0;
+  size_t wbytes = tapb * S * S, gbytes = tapb;
+  if (x3) {      // SPLIT3: w_hi and w_lo sets on the stacked kernel, [w_hi, w_lo, w_hi] per k-step else
+    wbytes = p->stacked ? 2 * stack_set : 3 * tapb * S * S;
+    gbytes = p->stacked ? 3 * tapb : 0;      // ([w_hi | w_lo] wide block + w_hi per 16 input channels)
+  } else if (p->stacked) {
+    wbytes = stack_set;
+  } else if (p->fused_tc) {
+    wbytes = sizeof(__nv_bfloat16) * ksteps * 15 * 8 * 2 * 128 * 8;      // paired-tap blocks
+  }
+  if ((rc = p->wpk.alloc(wbytes))) return rc;
+  if (gbytes && ((rc = p->wpk_i.alloc(gbytes)) || (rc = p->wpk_o.alloc(gbytes)))) return rc;
+  if (!x3) {
     if ((rc = p->clk.alloc(sizeof(unsigned long long) * 2 * 1024))) return rc;
     CUDA_TRY(cudaMemset(p->clk.p, 0, p->clk.bytes));
+  }
+  // operand windows of the convs (SxS halo boxes) and, for the separate gate kernels, 1x1 boxes
+  char* a0 = static_cast<char*>(p->actA.p);
+  char* h0 = static_cast<char*>(p->actH1.p);
+  const int planes = x3 && !p->stacked ? 2 * p->CG : p->CG;
+  bool bad = hgru::make_act_tensor_map(&p->mapA, a0, N, planes, HA, W, box_cols, box_rows, box_chunks) ||
+             hgru::make_act_tensor_map(&p->mapH1, h0, N, planes, HA, W, box_cols, box_rows, box_chunks);
+  if (p->conv_parts() == 2)
+    bad = bad || hgru::make_act_tensor_map(&p->mapA_lo, a0 + plane, N, planes, HA, W, box_cols, box_rows, box_chunks) ||
+          hgru::make_act_tensor_map(&p->mapH1_lo, h0 + plane, N, planes, HA, W, box_cols, box_rows, box_chunks);
+  if (!x3) {
     TcGeom g1;
     tc_geometry(1, p->KP, &g1);
-    if (hgru::make_act_tensor_map(&p->mapA, p->actA.p, N, p->CG, HA, W, box_cols, box_rows, box_chunks) ||
-        hgru::make_act_tensor_map(&p->mapH1, p->actH1.p, N, p->CG, HA, W, box_cols, box_rows, box_chunks) ||
-        hgru::make_act_tensor_map(&p->mapH1_g, p->actH1.p, N, p->CG, HA, W, g1.box_cols, g1.box_rows) ||
-        hgru::make_act_tensor_map(&p->mapH2_g, p->actH2.p, N, p->CG, HA, W, g1.box_cols, g1.box_rows))
-      return fail(HGRU_E_CUDA, "cuTensorMapEncodeTiled failed");
+    bad = bad || hgru::make_act_tensor_map(&p->mapH1_g, h0, N, p->CG, HA, W, g1.box_cols, g1.box_rows) ||
+          hgru::make_act_tensor_map(&p->mapH2_g, p->actH2.p, N, p->CG, HA, W, g1.box_cols, g1.box_rows);
   }
+  if (bad) return fail(HGRU_E_CUDA, "cuTensorMapEncodeTiled failed");
   return 0;
 }
 
 static void hgru_plan_free(hgru_plan_s* p) {
-  DevBuf* all[] = {&p->p_r, &p->i_r, &p->o_r, &p->vecs, &p->rho, &p->wpk, &p->wpk_i, &p->wpk_o, &p->Xp,
-                   &p->H2, &p->H1, &p->C, &p->G, &p->A, &p->actA, &p->actH1, &p->actH2, &p->flags, &p->clk};
-  for (auto b : all) b->release();
+  for (auto b : hgru_plan_s::buffers(p)) b->release();
 }
 
 // weights of the bf16 / fp16 modes in their operand format F: p_r for the plan's 15x15 kernel, i_r and o_r for the
@@ -410,6 +403,33 @@ static int hgru_set_params_impl(hgru_plan_s* p, const float* p_r, const float* i
   return 0;
 }
 
+// API boundary <-> internal state layout (fp32 mode: channel-padded NHWC; bf16 modes: quad-chunked)
+static void state_from_nhwc(const hgru_plan_s* p, const float* in, float* out, cudaStream_t st) {
+  if (p->mode != HGRU_MODE_FP32)
+    hgru::nhwc_to_quad_kernel<<<nblk(p->nelem_n() / 4), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP, p->H * p->W);
+  else
+    hgru::pad_channels_kernel<<<nblk(p->nelem_n()), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP);
+}
+static void state_to_nhwc(const hgru_plan_s* p, const float* in, float* out, cudaStream_t st) {
+  if (p->mode != HGRU_MODE_FP32)
+    hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP, p->H * p->W);
+  else
+    hgru::unpad_channels_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP);
+}
+
+// H1 or H2 of timestep t -> its trace [T][n][H][W][k], if there is one (half: H1 of the bf16 / fp16 pipeline with
+// epilogue-issued gates, an fp16 oct-chunked tensor)
+static void copy_trace(hgru_plan_s* p, const void* src, bool half, float* trace, int t, cudaStream_t st) {
+  if (!trace) return;
+  float* dst = trace + static_cast<size_t>(t) * p->npix_n() * p->k;
+  if (half)
+    hgru::oct_half_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(static_cast<const __half*>(src), dst,
+                                                                              p->npix_n(), p->k, p->KP, p->H * p->W);
+  else
+    state_to_nhwc(p, static_cast<const float*>(src), dst, st);
+  ++p->launches;
+}
+
 // ---- fp32 path: SIMT kernels, unfused (the <= 1e-4 anchor) --------------------------------------
 static int hgru_run_fp32(hgru_plan_s* p, const float* Xp, float* H1_trace, float* H2_trace, cudaStream_t st) {
   const int KP = p->KP, HW = p->H * p->W;
@@ -444,25 +464,13 @@ static int hgru_run_fp32(hgru_plan_s* p, const float* Xp, float* H1_trace, float
                                                   p->vec(V_GAMMA), p->vec(V_KAPPA), p->vec(V_OMEGA),
                                                   p->rho.as<float>(), t, p->H2.as<float>(), nchunks, KP, p->k);
     p->launches += 6;
-    if (H1_trace) {
-      hgru::unpad_channels_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
-          p->H1.as<float>(), H1_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP);
-      ++p->launches;
-    }
-    if (H2_trace) {
-      hgru::unpad_channels_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
-          p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP);
-      ++p->launches;
-    }
+    copy_trace(p, p->H1.p, false, H1_trace, t, st);
+    copy_trace(p, p->H2.p, false, H2_trace, t, st);
   }
   return 0;
 }
 
-// ---- bf16 path ------------------------------------------------------------------------------------
-// Narrow layers (stacked kernel): two tcgen05 launches per timestep, the 1x1 gate convs run as
-// epilogue-issued MMAs inside them.  Wide layers (k = 64): four launches (gate-in, C1+H1, gate-out,
-// C2+H2).  All integration math happens on TMEM accumulators.
-// Initial state of the bf16 path: O_0 (NHWC, or zeros) -> H2 (quad-chunked fp32) + the first gated operand.
+// Initial state of the bf16 / fp16 path: O_0 (NHWC, or zeros) -> H2 (quad-chunked fp32) + the first gated operand.
 // Touches only H2 / actA, so it can run before (and concurrently with the input copy of) the stem.
 template <int KP, class F>
 static int launch_init_tc(const float* h0, const hgru::TcConvArgs& a, cudaStream_t st) {
@@ -490,264 +498,146 @@ static int hgru_init_state_bf16(hgru_plan_s* p, const float* H2_init_nhwc, cudaS
                               : launch_init_tc<hgru::OpBf16>(p->KP, H2_init_nhwc, a, st);
 }
 
-static int hgru_run_bf16(hgru_plan_s* p, const float* Xp, const float* H2_init_nhwc, float* H1_trace,
-                         float* H2_trace, cudaStream_t st) {
+// The conv launch of one half-step, on the plan's kernel family: c = 0 for C1 + input integration (-> H1), 1 for C2 +
+// output integration (-> H2); partial: the first launch of a bf16x3 conv on the stacked kernel (a_lo * w_hi -> C).
+static int conv_launch(const hgru_plan_s* p, int c, bool partial, const hgru::TcConvArgs& a, cudaStream_t st) {
+  const CUtensorMap& map = c == 0 ? (partial ? p->mapA_lo : p->mapA) : (partial ? p->mapH1_lo : p->mapH1);
+  if (p->stacked && p->mode == HGRU_MODE_BF16X3)
+    return stack_launch(partial ? EPI_PARTIAL : c ? EPI_H2 : EPI_H1, p->KP, p->stack_T, FMT_BF16, map, a, st);
+  // (fused pipeline: H1 and G2 travel to the H2 launch as fp16, EpiH1h / EpiH2h)
+  if (p->stacked) return stack_launch(c ? EPI_H2_HALF : EPI_H1_HALF, p->KP, p->stack_T, p->fmt(), map, a, st);
+  if (p->fused_tc)
+    return c ? tc_fused64_launch<EPI_H2_HALF>(p->fmt(), map, a, st) : tc_fused64_launch<EPI_H1_HALF>(p->fmt(), map, a, st);
+  if (p->mode == HGRU_MODE_BF16X3)
+    return c ? tc_x3_launch<EPI_H2>(p->S, p->KP, map, a, st) : tc_x3_launch<EPI_H1>(p->S, p->KP, map, a, st);
+  return c ? tc_hconv_launch<EPI_H2>(p->S, p->KP, map, a, st) : tc_hconv_launch<EPI_H1>(p->S, p->KP, map, a, st);
+}
+
+// A 1x1 gate as a launch of its own (where the conv epilogues do not issue it): c = 0 for circuit_input
+// (hgru_module.py:696-711), operand A = F(sigmoid(H2 *1x1 i_r + i_b) . H2); c = 1 for circuit_output (:729-740),
+// G2 = sigmoid(H1 *1x1 o_r + o_b).  On tensor cores in the bf16 / fp16 modes, exact fp32 (SIMT) in the bf16x3 mode.
+static int gate_launch(hgru_plan_s* p, int c, const hgru::TcConvArgs& base, cudaStream_t st) {
   const int KP = p->KP, HW = p->H * p->W;
-  int rc;
-  hgru::TcConvArgs base{};
-  base.N = p->n; base.H = p->H; base.W = p->W; base.KP = KP; base.kreal = p->k;
-  base.act_pad = p->act_pad;
-  // initial state O_0 (NHWC or zeros) -> H2 (quad-chunked fp32) + the first gated operand, one pass (unless the
-  // caller already ran it: the pose plan overlaps it with the upload of the crops)
-  if (!p->state_ready && (rc = hgru_init_state_bf16(p, H2_init_nhwc, st))) return rc;
-  p->state_ready = false;
+  int rc = 0;
+  if (p->mode == HGRU_MODE_BF16X3) {
+    SMEM_ATTR_ONCE(hgru::gate_quad_split_kernel, 100 * 1024);
+    const size_t smem = sizeof(float) * (KP * KP + hgru::kInitPix * (KP + 1));
+    const dim3 grid = nblk(p->npix_n(), hgru::kInitPix);
+    if (c == 0)
+      hgru::gate_quad_split_kernel<<<grid, 256, smem, st>>>(p->H2.as<float>(), p->i_r.as<float>(), p->vec(V_IB), nullptr,
+                                                            p->actA.as<__nv_bfloat16>(), p->npix_n(), p->k, KP, HW,
+                                                            p->lo_off, p->W, p->act_pad);
+    else
+      hgru::gate_quad_split_kernel<<<grid, 256, smem, st>>>(p->H1.as<float>(), p->o_r.as<float>(), p->vec(V_OB),
+                                                            p->G.as<float>(), nullptr, p->npix_n(), p->k, KP, HW);
+  } else {
+    hgru::TcConvArgs a = base;
+    if (c == 0) {
+      a.wpk = p->wpk_i.as<__nv_bfloat16>(); a.bias = p->vec(V_IB); a.H2 = p->H2.as<float>();
+      a.out_bf16 = p->actA.as<__nv_bfloat16>();
+      rc = dispatch_gate<hgru::EpiGateIn>(KP, p->actH2.as<__nv_bfloat16>(), a, st);
+    } else {
+      a.wpk = p->wpk_o.as<__nv_bfloat16>(); a.bias = p->vec(V_OB); a.out = p->G.as<float>();
+      rc = dispatch_gate<hgru::EpiGateOut>(KP, p->actH1.as<__nv_bfloat16>(), a, st);
+    }
+  }
   ++p->launches;
-  const bool fused = p->stacked || p->fused_tc;
+  return rc;
+}
+
+// ---- tensor-core paths: bf16, fp16 and bf16x3 ------------------------------------------------------------------
+// Per timestep: [circuit_input gate], C1 conv + input integration -> H1, [circuit_output gate], C2 conv + output
+// integration -> H2, traces.  All integration math happens on TMEM accumulators.  The gates are epilogue-issued MMAs
+// inside the conv launches where the plan has epi_gates, else launches of their own.  bf16x3: every conv operand is a
+// bf16 hi + lo pair and each k-step is three products (hi*hi + hi*w_lo + lo*w_hi); on the stacked kernel the first
+// launch of a conv reads a_lo against w_hi and leaves fp32 sums in C, the second reads a_hi against w_hi and w_lo and
+// adds C -- the launch with the heavy epilogue is the one with twice the MMAs to hide it behind.
+static int hgru_run_tc(hgru_plan_s* p, const float* Xp, const float* H2_init_nhwc, float* H1_trace, float* H2_trace,
+                       cudaStream_t st) {
+  int rc;
+  // initial state O_0 (NHWC or zeros) -> H2 (quad-chunked fp32).  bf16 / fp16: + the first gated operand, in one pass
+  // (unless the caller already ran it: the pose plan overlaps it with the upload of the crops)
+  if (p->op16()) {
+    if (!p->state_ready && (rc = hgru_init_state_bf16(p, H2_init_nhwc, st))) return rc;
+    p->state_ready = false;
+  } else if (H2_init_nhwc) {
+    state_from_nhwc(p, H2_init_nhwc, p->H2.as<float>(), st);
+  } else {
+    CUDA_TRY(cudaMemsetAsync(p->H2.p, 0, p->nelem_n() * sizeof(float), st));
+  }
+  ++p->launches;
+  const bool x3 = p->mode == HGRU_MODE_BF16X3;
+  const int parts = p->conv_parts();
+  hgru::TcConvArgs base{};
+  base.N = p->n; base.H = p->H; base.W = p->W; base.KP = p->KP; base.kreal = p->k;
+  base.act_pad = p->act_pad; base.lo_off = p->lo_off;
+  base.split_out = x3 ? parts : 0;      // bf16x3: hi / lo operand splits, two tensors on the stacked kernel
   // (a weight ring of 5 stages x 3 taps instead of 3 stages x 5 taps for the fused 64-channel kernel measured the
   // same: profiles/r02_bench_k64_fused_ring_5x3taps.json)
   // Chained launches (see TcConvArgs::wait_flags): launch l waits per frame on launch l-1's counters instead of on
-  // the whole grid.  Not with traces (their copy kernels sit between the launches).
-  const bool chain = fused && p->chain && !H1_trace && !H2_trace;
+  // the whole grid.  Not with traces (their copy kernels sit between the launches), and not where a gate is a launch
+  // of its own.
+  const bool chain = p->chain && p->epi_gates && !H1_trace && !H2_trace;
   int* flags = chain ? p->flags.as<int>() : nullptr;
   if (chain) CUDA_TRY(cudaMemsetAsync(flags, 0, p->flags.bytes, st));
-  auto set_flags = [&](hgru::TcConvArgs& a, int l) {
-    if (!chain) return;
-    a.done_flags = flags + static_cast<size_t>(l) * p->N;
-    a.wait_flags = l > 0 ? flags + static_cast<size_t>(l - 1) * p->N : nullptr;
-  };
-  if (chain) p->timer.begin(st);
-  for (int t = 0; t < p->T; ++t) {
-    hgru::TcConvArgs a;
-    if (!fused && t > 0) {
-      // circuit_input gate (hgru_module.py:696-711): operand A = bf16(sigmoid(H2 *1x1 i_r + i_b) . H2)
-      a = base;
-      a.wpk = p->wpk_i.as<__nv_bfloat16>(); a.bias = p->vec(V_IB); a.H2 = p->H2.as<float>();
-      a.out_bf16 = p->actA.as<__nv_bfloat16>();
-      if ((rc = dispatch_gate<hgru::EpiGateIn>(KP, p->actH2.as<__nv_bfloat16>(), a, st))) return rc;
-      ++p->launches;
+  // conv c of timestep t; a: the arguments of its (last) launch
+  auto conv = [&](int t, int c, const hgru::TcConvArgs& a) -> int {
+    // kernel timer: chained, one interval around all launches, counted as 2T passes over the whole batch; else one
+    // interval per conv
+    if (!chain || (t == 0 && c == 0)) p->timer.begin(st);
+    for (int i = 0; i < parts; ++i) {
+      const bool partial = i + 1 < parts;
+      hgru::TcConvArgs la = a;
+      if (partial) {
+        la = base;
+        la.wpk = p->wpk.as<__nv_bfloat16>(); la.out = p->C.as<float>();
+      }
+      if (chain) {
+        const size_t l = static_cast<size_t>(2 * t + c) * parts + i;
+        la.done_flags = flags + l * p->N;
+        la.wait_flags = l > 0 ? flags + (l - 1) * p->N : nullptr;
+      }
+      if (int r = conv_launch(p, c, partial, la, st)) return r;
     }
-    // C1 conv (:714-718, 657) + input_integration (:795-804) -> H1 (fp32 + bf16 operand copy)
-    // [fused: + circuit_output gate (:729-740) -> G2]
-    a = base;
-    a.wpk = p->wpk.as<__nv_bfloat16>(); a.bias = p->vec(V_LBIAS); a.X = Xp; a.H2 = p->H2.as<float>();
-    a.v0 = p->vec(V_BETA); a.v1 = p->vec(V_NU);
+    if (!chain || (t + 1 == p->T && c == 1)) p->timer.end(st, chain ? 2 * p->T : 1);
+    p->launches += parts;
+    return 0;
+  };
+  for (int t = 0; t < p->T; ++t) {
+    // at t = 0 the operand comes from the initial-state pass in the bf16 / fp16 modes
+    if ((t == 0 ? !p->op16() : !p->epi_gates) && (rc = gate_launch(p, 0, base, st))) return rc;
+    // C1 conv (:714-718, 657) + input_integration (:795-804) -> H1 (fp32 + 16-bit operand copy)
+    // [epi_gates: + circuit_output gate (:729-740) -> G2]
+    hgru::TcConvArgs a = base;
+    a.wpk = p->wpk.as<__nv_bfloat16>(); a.partial = parts == 2 ? p->C.as<float>() : nullptr;
+    a.bias = p->vec(V_LBIAS); a.X = Xp; a.H2 = p->H2.as<float>(); a.v0 = p->vec(V_BETA); a.v1 = p->vec(V_NU);
     a.out = p->H1.as<float>(); a.out_bf16 = p->actH1.as<__nv_bfloat16>();
     a.gate_wpk = p->wpk_o.as<__nv_bfloat16>(); a.gate_bias = p->vec(V_OB); a.gate_out = p->G.as<float>();
-    a.do_gate = fused ? 1 : 0;
-    set_flags(a, 2 * t);
-    if (!chain) p->timer.begin(st);
-    // (fused pipeline: H1 and G2 travel to the H2 launch as fp16, EpiH1h / EpiH2h)
-    if ((rc = p->stacked    ? stack_launch(EPI_H1_HALF, 1, false, KP, p->stack_T, p->fmt(), p->mapA, a, st)
-              : p->fused_tc ? tc_fused64_launch(EPI_H1_HALF, p->fmt(), p->mapA, a, st)
-                            : tc_hconv_launch(EPI_H1, p->S, KP, p->mapA, a, st)))
-      return rc;
-    if (!chain) p->timer.end(st);
-    ++p->launches;
-    if (!fused) {
-      // circuit_output gate (:729-740): G2 = sigmoid(H1 *1x1 o_r + o_b)
-      a = base;
-      a.wpk = p->wpk_o.as<__nv_bfloat16>(); a.bias = p->vec(V_OB); a.out = p->G.as<float>();
-      if ((rc = dispatch_gate<hgru::EpiGateOut>(KP, p->actH1.as<__nv_bfloat16>(), a, st))) return rc;
-      ++p->launches;
-    }
+    a.do_gate = p->epi_gates ? 1 : 0;
+    if ((rc = conv(t, 0, a))) return rc;
+    if (!p->epi_gates && (rc = gate_launch(p, 1, base, st))) return rc;
     // C2 conv (:746-750, 657) + output_integration + rho (:806-823, 847-849) -> H2 in place
-    // [fused: + the next timestep's circuit_input gate -> operand A]
+    // [epi_gates: + the next timestep's circuit_input gate -> operand A]
     a = base;
-    a.wpk = p->wpk.as<__nv_bfloat16>(); a.bias = p->vec(V_LBIAS); a.H1 = p->H1.as<float>();
-    a.G = p->G.as<float>(); a.H2 = p->H2.as<float>();
+    a.wpk = p->wpk.as<__nv_bfloat16>(); a.partial = parts == 2 ? p->C.as<float>() : nullptr;
+    a.bias = p->vec(V_LBIAS); a.H1 = p->H1.as<float>(); a.G = p->G.as<float>(); a.H2 = p->H2.as<float>();
     a.v0 = p->vec(V_GAMMA); a.v1 = p->vec(V_KAPPA); a.v2 = p->vec(V_OMEGA);
     a.rho_t = p->rho.as<float>() + t;
-    a.out_bf16 = fused ? nullptr : p->actH2.as<__nv_bfloat16>();
+    a.out_bf16 = p->epi_gates ? nullptr : p->actH2.as<__nv_bfloat16>();      // (the bf16 / fp16 gate kernel's operand)
     a.gate_wpk = p->wpk_i.as<__nv_bfloat16>(); a.gate_bias = p->vec(V_IB);
     a.gate_act_out = p->actA.as<__nv_bfloat16>();
-    a.do_gate = (fused && t + 1 < p->T) ? 1 : 0;
-    if (g_timing && t + 1 == p->T) a.clk_out = p->clk.as<unsigned long long>();   // (grids are <= 1024 CTAs)
-    if (t + 1 == p->T && p->fc_a) {     // last update also emits the readout's bf16 hi/lo operand
-      a.fc_a = p->fc_a; a.fc_scale = p->fc_scale; a.fc_shift = p->fc_shift; a.fc_kpad = p->fc_kpad;
-    }
-    set_flags(a, 2 * t + 1);
-    if (!chain) p->timer.begin(st);
-    if ((rc = p->stacked    ? stack_launch(EPI_H2_HALF, 1, false, KP, p->stack_T, p->fmt(), p->mapH1, a, st)
-              : p->fused_tc ? tc_fused64_launch(EPI_H2_HALF, p->fmt(), p->mapH1, a, st)
-                            : tc_hconv_launch(EPI_H2, p->S, KP, p->mapH1, a, st)))
-      return rc;
-    if (!chain) p->timer.end(st);
-    else if (t + 1 == p->T) p->timer.end(st, 2 * p->T);   // chained: one interval around all launches,
-    //                                                       counted as 2T passes over the whole batch
-    ++p->launches;
-    if (H1_trace) {
-      float* dst = H1_trace + static_cast<size_t>(t) * p->npix_n() * p->k;
-      if (fused)      // H1 is an fp16 oct-chunked tensor in the fused pipeline
-        hgru::oct_half_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(p->H1.as<__half>(), dst, p->npix_n(), p->k, KP, HW);
-      else
-        hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(p->H1.as<float>(), dst, p->npix_n(), p->k, KP, HW);
-      ++p->launches;
-    }
-    if (H2_trace) {
-      hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
-          p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
-      ++p->launches;
-    }
-  }
-  return 0;
-}
-
-// ---- bf16x3 path: fp32-class accuracy on tensor cores (k <= 32) -----------------------------------------
-// Every conv operand is a bf16 hi + lo pair and each k-step is three products (hi*hi + hi*w_lo + lo*w_hi, the
-// SPLIT3 mode of hconv_tc.cuh); the 1x1 gates are exact fp32 (SIMT); state, accumulation and the integration
-// epilogues are the fp32 ones of the bf16 path.  Four launches per timestep.
-static int hgru_run_bf16x3(hgru_plan_s* p, const float* Xp, const float* H2_init_nhwc, float* H1_trace,
-                           float* H2_trace, cudaStream_t st) {
-  const int KP = p->KP, HW = p->H * p->W;
-  int rc;
-  SMEM_ATTR_ONCE(hgru::gate_quad_split_kernel, 100 * 1024);
-  const size_t gsmem = sizeof(float) * (KP * KP + hgru::kInitPix * (KP + 1));
-  if (H2_init_nhwc)
-    hgru::nhwc_to_quad_kernel<<<nblk(p->nelem_n() / 4), 256, 0, st>>>(H2_init_nhwc, p->H2.as<float>(), p->npix_n(), p->k, KP, HW);
-  else
-    CUDA_TRY(cudaMemsetAsync(p->H2.p, 0, p->nelem_n() * sizeof(float), st));
-  ++p->launches;
-  hgru::TcConvArgs base{};
-  base.N = p->n; base.H = p->H; base.W = p->W; base.KP = KP; base.kreal = p->k;
-  base.split_out = 1;
-  if (p->stacked) {
-    // ---- narrow layers: the tap-stacked kernel, two launches per conv (see hgru_plan_init) ----
-    base.split_out = 2; base.lo_off = p->lo_off; base.act_pad = p->act_pad;
-    // Launches are chained per frame like the bf16 path's (4 per timestep here); not with traces, and not where the
-    // gates are separate SIMT launches (32 channels, see launch_stack).
-    const bool fused_gate = !(KP == 32 && p->stack_T == 4);
-    const bool chain = fused_gate && p->chain && !H1_trace && !H2_trace;
-    int* flags = chain ? p->flags.as<int>() : nullptr;
-    if (chain) CUDA_TRY(cudaMemsetAsync(flags, 0, p->flags.bytes, st));
-    auto set_flags = [&](hgru::TcConvArgs& a, int l) {
-      if (!chain) return;
-      a.done_flags = flags + static_cast<size_t>(l) * p->N;
-      a.wait_flags = l > 0 ? flags + static_cast<size_t>(l - 1) * p->N : nullptr;
-    };
-    auto gate_in = [&]() {
-      // circuit_input gate (hgru_module.py:696-711), exact fp32: operand A = split(sigmoid(H2 *1x1 i_r + i_b) . H2)
-      hgru::gate_quad_split_kernel<<<nblk(p->npix_n(), hgru::kInitPix), 256, gsmem, st>>>(
-          p->H2.as<float>(), p->i_r.as<float>(), p->vec(V_IB), nullptr, p->actA.as<__nv_bfloat16>(), p->npix_n(), p->k,
-          KP, HW, p->lo_off, p->W, p->act_pad);
-      ++p->launches;
-    };
-    gate_in();      // first timestep; with fused gates the later ones come from the H2 launch's epilogue
-    if (chain) p->timer.begin(st);
-    for (int t = 0; t < p->T; ++t) {
-      if (!fused_gate && t > 0) gate_in();
-      // C1 conv (:714-718, 657): a_lo * w_hi -> C, then a_hi * (w_hi, w_lo) + C + input_integration (:795-804) -> H1
-      // [fused: + circuit_output gate (:729-740) on hi/lo splits of H1 -> G2]
-      if (!chain) p->timer.begin(st);
-      hgru::TcConvArgs a = base;
-      a.wpk = p->wpk.as<__nv_bfloat16>(); a.out = p->C.as<float>();
-      set_flags(a, 4 * t);
-      if ((rc = stack_launch(EPI_PARTIAL, 1, false, KP, p->stack_T, FMT_BF16, p->mapA_lo, a, st))) return rc;
-      a = base;
-      a.wpk = p->wpk.as<__nv_bfloat16>(); a.partial = p->C.as<float>();
-      a.bias = p->vec(V_LBIAS); a.X = Xp; a.H2 = p->H2.as<float>(); a.v0 = p->vec(V_BETA); a.v1 = p->vec(V_NU);
-      a.out = p->H1.as<float>(); a.out_bf16 = p->actH1.as<__nv_bfloat16>();
-      a.gate_wpk = p->wpk_o.as<__nv_bfloat16>(); a.gate_bias = p->vec(V_OB); a.gate_out = p->G.as<float>();
-      a.do_gate = fused_gate ? 1 : 0;
-      set_flags(a, 4 * t + 1);
-      if ((rc = stack_launch(EPI_H1, 2, true, KP, p->stack_T, FMT_BF16, p->mapA, a, st))) return rc;
-      if (!chain) p->timer.end(st);
-      if (!fused_gate) {
-        // circuit_output gate (:729-740): G2 = sigmoid(H1 *1x1 o_r + o_b), exact fp32
-        hgru::gate_quad_split_kernel<<<nblk(p->npix_n(), hgru::kInitPix), 256, gsmem, st>>>(
-            p->H1.as<float>(), p->o_r.as<float>(), p->vec(V_OB), p->G.as<float>(), nullptr, p->npix_n(), p->k, KP, HW);
-        ++p->launches;
-      }
-      // C2 conv (:746-750, 657) + output_integration + rho (:806-823, 847-849) -> H2 in place
-      // [fused: + the next timestep's circuit_input gate -> operand A (hi, lo)]
-      if (!chain) p->timer.begin(st);
-      a = base;
-      a.wpk = p->wpk.as<__nv_bfloat16>(); a.out = p->C.as<float>();
-      set_flags(a, 4 * t + 2);
-      if ((rc = stack_launch(EPI_PARTIAL, 1, false, KP, p->stack_T, FMT_BF16, p->mapH1_lo, a, st))) return rc;
-      a = base;
-      a.wpk = p->wpk.as<__nv_bfloat16>(); a.partial = p->C.as<float>();
-      a.bias = p->vec(V_LBIAS); a.H1 = p->H1.as<float>(); a.G = p->G.as<float>(); a.H2 = p->H2.as<float>();
-      a.v0 = p->vec(V_GAMMA); a.v1 = p->vec(V_KAPPA); a.v2 = p->vec(V_OMEGA);
-      a.rho_t = p->rho.as<float>() + t;
-      a.gate_wpk = p->wpk_i.as<__nv_bfloat16>(); a.gate_bias = p->vec(V_IB);
-      a.gate_act_out = p->actA.as<__nv_bfloat16>();
-      a.do_gate = (fused_gate && t + 1 < p->T) ? 1 : 0;
-      if (t + 1 == p->T && p->fc_a) {
+    a.do_gate = (p->epi_gates && t + 1 < p->T) ? 1 : 0;
+    if (t + 1 == p->T) {
+      if (g_timing) a.clk_out = p->clk.as<unsigned long long>();      // (bf16 / fp16; grids are <= 1024 CTAs)
+      if (p->fc_a) {      // the last update also emits the readout's bf16 hi/lo operand
         a.fc_a = p->fc_a; a.fc_scale = p->fc_scale; a.fc_shift = p->fc_shift; a.fc_kpad = p->fc_kpad;
       }
-      set_flags(a, 4 * t + 3);
-      if ((rc = stack_launch(EPI_H2, 2, true, KP, p->stack_T, FMT_BF16, p->mapH1, a, st))) return rc;
-      if (!chain) p->timer.end(st);
-      else if (t + 1 == p->T) p->timer.end(st, 2 * p->T);      // chained: one interval, counted as 2T convs
-      p->launches += 4;
-      if (H1_trace) {
-        hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
-            p->H1.as<float>(), H1_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
-        ++p->launches;
-      }
-      if (H2_trace) {
-        hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
-            p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
-        ++p->launches;
-      }
     }
-    return 0;
-  }
-  for (int t = 0; t < p->T; ++t) {
-    // circuit_input gate (hgru_module.py:696-711): operand A = split(sigmoid(H2 *1x1 i_r + i_b) . H2)
-    hgru::gate_quad_split_kernel<<<nblk(p->npix_n(), hgru::kInitPix), 256, gsmem, st>>>(
-        p->H2.as<float>(), p->i_r.as<float>(), p->vec(V_IB), nullptr, p->actA.as<__nv_bfloat16>(), p->npix_n(), p->k,
-        KP, HW);
-    // C1 conv (:714-718, 657) + input_integration (:795-804) -> H1 (fp32 + hi/lo operand)
-    hgru::TcConvArgs a = base;
-    a.wpk = p->wpk.as<__nv_bfloat16>(); a.bias = p->vec(V_LBIAS); a.X = Xp; a.H2 = p->H2.as<float>();
-    a.v0 = p->vec(V_BETA); a.v1 = p->vec(V_NU);
-    a.out = p->H1.as<float>(); a.out_bf16 = p->actH1.as<__nv_bfloat16>();
-    p->timer.begin(st);
-    if ((rc = tc_x3_launch(EPI_H1, p->S, KP, p->mapA, a, st))) return rc;
-    p->timer.end(st);
-    // circuit_output gate (:729-740): G2 = sigmoid(H1 *1x1 o_r + o_b), exact fp32
-    hgru::gate_quad_split_kernel<<<nblk(p->npix_n(), hgru::kInitPix), 256, gsmem, st>>>(
-        p->H1.as<float>(), p->o_r.as<float>(), p->vec(V_OB), p->G.as<float>(), nullptr, p->npix_n(), p->k, KP, HW);
-    // C2 conv (:746-750, 657) + output_integration + rho (:806-823, 847-849) -> H2 in place
-    a = base;
-    a.wpk = p->wpk.as<__nv_bfloat16>(); a.bias = p->vec(V_LBIAS); a.H1 = p->H1.as<float>();
-    a.G = p->G.as<float>(); a.H2 = p->H2.as<float>();
-    a.v0 = p->vec(V_GAMMA); a.v1 = p->vec(V_KAPPA); a.v2 = p->vec(V_OMEGA);
-    a.rho_t = p->rho.as<float>() + t;
-    if (t + 1 == p->T && p->fc_a) {
-      a.fc_a = p->fc_a; a.fc_scale = p->fc_scale; a.fc_shift = p->fc_shift; a.fc_kpad = p->fc_kpad;
-    }
-    p->timer.begin(st);
-    if ((rc = tc_x3_launch(EPI_H2, p->S, KP, p->mapH1, a, st))) return rc;
-    p->timer.end(st);
-    p->launches += 4;
-    if (H1_trace) {
-      hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
-          p->H1.as<float>(), H1_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
-      ++p->launches;
-    }
-    if (H2_trace) {
-      hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(
-          p->H2.as<float>(), H2_trace + static_cast<size_t>(t) * p->npix_n() * p->k, p->npix_n(), p->k, KP, HW);
-      ++p->launches;
-    }
+    if ((rc = conv(t, 1, a))) return rc;
+    copy_trace(p, p->H1.p, p->op16() && p->epi_gates, H1_trace, t, st);
+    copy_trace(p, p->H2.p, false, H2_trace, t, st);
   }
   return 0;
-}
-
-// API boundary <-> internal state layout (fp32 mode: channel-padded NHWC; bf16 modes: quad-chunked)
-static void state_from_nhwc(const hgru_plan_s* p, const float* in, float* out, cudaStream_t st) {
-  if (p->mode != HGRU_MODE_FP32)
-    hgru::nhwc_to_quad_kernel<<<nblk(p->nelem_n() / 4), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP, p->H * p->W);
-  else
-    hgru::pad_channels_kernel<<<nblk(p->nelem_n()), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP);
-}
-static void state_to_nhwc(const hgru_plan_s* p, const float* in, float* out, cudaStream_t st) {
-  if (p->mode != HGRU_MODE_FP32)
-    hgru::quad_to_nhwc_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP, p->H * p->W);
-  else
-    hgru::unpad_channels_kernel<<<nblk(p->npix_n() * p->k), 256, 0, st>>>(in, out, p->npix_n(), p->k, p->KP);
 }
 
 // The recurrence on padded buffers: X = Xp, state in p->H2 (in/out).
@@ -757,10 +647,8 @@ static int hgru_run_padded(hgru_plan_s* p, const float* Xp, const float* H2_init
   p->launches = 0;
   p->timer.reset();
   int rc;
-  if (p->op16()) {
-    rc = hgru_run_bf16(p, Xp, H2_init_nhwc, H1_trace, H2_trace, st);
-  } else if (p->mode == HGRU_MODE_BF16X3) {
-    rc = hgru_run_bf16x3(p, Xp, H2_init_nhwc, H1_trace, H2_trace, st);
+  if (p->mode != HGRU_MODE_FP32) {
+    rc = hgru_run_tc(p, Xp, H2_init_nhwc, H1_trace, H2_trace, st);
   } else {
     if (H2_init_nhwc) state_from_nhwc(p, H2_init_nhwc, p->H2.as<float>(), st);
     else CUDA_TRY(cudaMemsetAsync(p->H2.p, 0, p->nelem_n() * sizeof(float), st));
@@ -799,11 +687,16 @@ struct pose_plan_s {
   float* bn_scale(int i) const { return bn.as<float>() + static_cast<size_t>(i) * 2 * bnw; }
   float* bn_shift(int i) const { return bn_scale(i) + bnw; }
   int bnw = 0;
+  // every device buffer besides the hGRU plan's: what workspace() counts is what pose_plan_free releases
+  template <class P> static auto buffers(P* p) {
+    return std::array{&p->depth, &p->pool1, &p->conv2, &p->w1, &p->b1, &p->w2, &p->b2, &p->w3, &p->b3,
+                      &p->fc1_w, &p->fc1_b, &p->fc2_w, &p->fc2_b, &p->bn, &p->part, &p->fc1, &p->out,
+                      &p->act_pool1, &p->act_conv2, &p->wpk2, &p->wpk3, &p->fc1_wt, &p->fc1_a, &p->h0_tmp};
+  }
   size_t workspace() const {
-    return hg.workspace() + depth.bytes + pool1.bytes + conv2.bytes + w1.bytes + b1.bytes + w2.bytes +
-           b2.bytes + w3.bytes + b3.bytes + fc1_w.bytes + fc1_b.bytes + fc2_w.bytes + fc2_b.bytes +
-           bn.bytes + part.bytes + fc1.bytes + out.bytes + act_pool1.bytes + act_conv2.bytes +
-           wpk2.bytes + wpk3.bytes + fc1_wt.bytes + fc1_a.bytes + h0_tmp.bytes;
+    size_t b = hg.workspace();
+    for (auto buf : buffers(this)) b += buf->bytes;
+    return b;
   }
 };
 
@@ -815,10 +708,7 @@ static void pose_plan_free(pose_plan_s* p) {
   if (p->side_st) cudaStreamDestroy(p->side_st);
   if (p->ev_fork) cudaEventDestroy(p->ev_fork);
   if (p->ev_init) cudaEventDestroy(p->ev_init);
-  DevBuf* all[] = {&p->depth, &p->pool1, &p->conv2, &p->w1, &p->b1, &p->w2, &p->b2, &p->w3, &p->b3,
-                   &p->fc1_w, &p->fc1_b, &p->fc2_w, &p->fc2_b, &p->bn, &p->part, &p->fc1, &p->out,
-                   &p->act_pool1, &p->act_conv2, &p->wpk2, &p->wpk3, &p->fc1_wt, &p->fc1_a, &p->h0_tmp};
-  for (auto b : all) b->release();
+  for (auto b : pose_plan_s::buffers(p)) b->release();
 }
 
 // A forward over the first n frames of the plan (n <= N; buffers, tensor maps and the chaining counters keep the

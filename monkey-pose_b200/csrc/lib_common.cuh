@@ -70,7 +70,7 @@ inline bool narrow_units_faster(int units_wide, int work_wide, int units_narrow,
 inline unsigned nblk(size_t n, int b = 256) { return static_cast<unsigned>((n + b - 1) / b); }
 inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 
-// ---- launch geometries (must match the template instances in tc_launch_*.cu / stack_launch.cu) ----
+// ---- launch geometries (must match the template instances in tc_launch.cuh / stack_launch.cu) ----
 struct TcGeom { int tiles_x, box_cols, box_rows; };
 bool tc_geometry(int S, int KP, TcGeom* g);        // plain bf16 hconv_tc_kernel
 bool stem_geometry(int KP, TcGeom* g);             // 3x3 stem convs (SPLIT3)
@@ -82,16 +82,37 @@ bool stack_geometry(int S, int KP, int k, StackGeom* g);
 // format of the hGRU convs' 16-bit operands and weights (hgru::OpBf16 / hgru::OpFp16): bf16 mode / fp16 mode
 enum OpFormat { FMT_BF16 = 0, FMT_FP16 = 1 };
 enum EpiKind { EPI_H1 = 0, EPI_H2 = 1, EPI_H1_HALF = 2, EPI_H2_HALF = 3, EPI_PARTIAL = 4 };
-// hconv_stack_kernel<..., Epi, WSETS, PART>: tap-stacked 15x15 conv (k <= 32); FMT_FP16 exists for EPI_H*_HALF
-int stack_launch(EpiKind epi, int wsets, bool part, int KP, int T, OpFormat fmt, const CUtensorMap& map,
-                 const hgru::TcConvArgs& a, cudaStream_t st);
+// hconv_stack_kernel: tap-stacked 15x15 conv (k <= 32).  EPI_H*_HALF: the fused bf16 / fp16 pipeline; EPI_PARTIAL and
+// EPI_H1 / EPI_H2: the first and second launch of a bf16x3 conv (bf16 only)
+int stack_launch(EpiKind epi, int KP, int T, OpFormat fmt, const CUtensorMap& map, const hgru::TcConvArgs& a,
+                 cudaStream_t st);
 // its weight packing: HWIO fp32 -> the stacked (or remainder-packed) 16-bit stage layout; lo_part = the remainder
 int stack_pack_weights(const float* p_r, __nv_bfloat16* dst, int k, const StackGeom& sg, int lo_part, OpFormat fmt,
                        cudaStream_t st);
-// hconv_tc_kernel: plain (EPI_H1 / EPI_H2), FUSE at 64 channels (EPI_H1_HALF / EPI_H2_HALF), SPLIT3 stem, SPLIT3 x3
-int tc_hconv_launch(EpiKind epi, int S, int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
-int tc_fused64_launch(EpiKind epi, OpFormat fmt, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
-int tc_stem_launch(int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
-int tc_x3_launch(EpiKind epi, int S, int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
+// hconv_tc_kernel, one launcher per kernel family (tc_launch.cuh).  E is the epilogue: tc_launch_h1.cu instantiates
+// EPI_H1 / EPI_H1_HALF, tc_launch_h2.cu EPI_H2 / EPI_H2_HALF.
+template <EpiKind E>      // plain, S < 15: EPI_H1 / EPI_H2
+int tc_hconv_launch(int S, int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
+template <EpiKind E>      // FUSE, 15x15 at 64 channels: EPI_H1_HALF / EPI_H2_HALF
+int tc_fused64_launch(OpFormat fmt, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
+template <EpiKind E>      // SPLIT3, bf16x3 at 15x15 / 64 channels: EPI_H1 / EPI_H2
+int tc_x3_launch(int S, int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);
+int tc_stem_launch(int KP, const CUtensorMap& map, const hgru::TcConvArgs& a, cudaStream_t st);   // SPLIT3 stem
+
+// Launches a conv kernel (map, a).  A launch that waits on the previous launch's per-frame counters (a.wait_flags) is
+// chained to it (programmatic dependent launch): its CTAs take SMs as the previous launch's CTAs exit instead of
+// waiting for the whole grid.
+template <class Kern>
+int launch_chainable(Kern kern, int grid, int block, int smem, const CUtensorMap& map, const hgru::TcConvArgs& a,
+                     cudaStream_t st) {
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = smem; cfg.stream = st;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at; cfg.numAttrs = a.wait_flags ? 1 : 0;
+  CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, map, a));
+  return 0;
+}
 
 }  // namespace hgru_host

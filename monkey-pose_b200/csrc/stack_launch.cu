@@ -56,16 +56,7 @@ int launch_stack(const CUtensorMap& map, hgru::TcConvArgs a, cudaStream_t st) {
   a.num_units = a.N * a.units_x * a.units_y;
   const int grid = a.num_units < sms ? a.num_units : sms;
   a.flag_target = a.units_x * a.units_y;
-  // A launch that waits on the previous launch's per-frame counters is chained to it (programmatic dependent
-  // launch): its CTAs take SMs as the previous launch's CTAs exit instead of waiting for the whole grid.
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(Cfg::NTHREADS); cfg.dynamicSmemBytes = Cfg::SMEM_BYTES; cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = a.wait_flags ? 1 : 0;
-  CUDA_TRY(cudaLaunchKernelEx(&cfg, kern, map, a));
-  return 0;
+  return launch_chainable(kern, grid, Cfg::NTHREADS, Cfg::SMEM_BYTES, map, a, st);
 }
 
 template <class Epi, int WSETS = 1, bool PART = false, class F = hgru::OpBf16>
@@ -86,25 +77,20 @@ int stack_pack_weights(const float* p_r, __nv_bfloat16* dst, int k, const StackG
   return 0;
 }
 
-int stack_launch(EpiKind epi, int wsets, bool part, int KP, int T, OpFormat fmt, const CUtensorMap& map,
-                 const hgru::TcConvArgs& a, cudaStream_t st) {
+int stack_launch(EpiKind epi, int KP, int T, OpFormat fmt, const CUtensorMap& map, const hgru::TcConvArgs& a,
+                 cudaStream_t st) {
   if (fmt == FMT_FP16) {      // fp16 mode: the fused pipeline's two launches per timestep
-    if (!part && wsets == 1 && epi == EPI_H1_HALF)
-      return dispatch_stack<hgru::EpiH1hF16, 1, false, hgru::OpFp16>(KP, T, map, a, st);
-    if (!part && wsets == 1 && epi == EPI_H2_HALF)
-      return dispatch_stack<hgru::EpiH2hF16, 1, false, hgru::OpFp16>(KP, T, map, a, st);
+    if (epi == EPI_H1_HALF) return dispatch_stack<hgru::EpiH1hF16, 1, false, hgru::OpFp16>(KP, T, map, a, st);
+    if (epi == EPI_H2_HALF) return dispatch_stack<hgru::EpiH2hF16, 1, false, hgru::OpFp16>(KP, T, map, a, st);
     return fail(HGRU_E_UNSUPPORTED, "stacked conv: no fp16 variant of this kernel");
   }
-  if (!part && wsets == 1) {
-    switch (epi) {
-      case EPI_H1_HALF: return dispatch_stack<hgru::EpiH1h>(KP, T, map, a, st);      // fused bf16 pipeline
-      case EPI_H2_HALF: return dispatch_stack<hgru::EpiH2h>(KP, T, map, a, st);
-      case EPI_PARTIAL: return dispatch_stack<hgru::EpiPartial>(KP, T, map, a, st);  // bf16x3, first launch of a conv
-      default: break;
-    }
-  } else if (part && wsets == 2) {                                                   // bf16x3, second launch
-    if (epi == EPI_H1) return dispatch_stack<hgru::EpiH1, 2, true>(KP, T, map, a, st);
-    if (epi == EPI_H2) return dispatch_stack<hgru::EpiH2, 2, true>(KP, T, map, a, st);
+  switch (epi) {
+    case EPI_H1_HALF: return dispatch_stack<hgru::EpiH1h>(KP, T, map, a, st);      // fused bf16 pipeline
+    case EPI_H2_HALF: return dispatch_stack<hgru::EpiH2h>(KP, T, map, a, st);
+    case EPI_PARTIAL: return dispatch_stack<hgru::EpiPartial>(KP, T, map, a, st);  // bf16x3, first launch of a conv
+    // bf16x3, second launch: both weight sets, plus the first launch's sums
+    case EPI_H1: return dispatch_stack<hgru::EpiH1, 2, true>(KP, T, map, a, st);
+    case EPI_H2: return dispatch_stack<hgru::EpiH2, 2, true>(KP, T, map, a, st);
   }
   return fail(HGRU_E_UNSUPPORTED, "stacked conv: no such kernel variant");
 }

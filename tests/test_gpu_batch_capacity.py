@@ -402,3 +402,45 @@ def test_streamed_forward_ragged_last_batch_keeps_the_plan(monkeypatch):
         out, made = calls.during(lambda: m.build(b, O))
         assert torch.equal(g, out) and made == {"pose_plan_create": 0}
     assert m._plan_capacity == 5
+
+
+# Launches of one forward, by path: (mode, k, S) -> (per timestep, besides).  hgru_forward_batch without traces; the
+# traces add two copies per timestep.  Besides the recurrence, hgru_forward_batch counts 3 and a pose forward 5 (the
+# stem's three, fc_1 and the fc tail).
+#   bf16 / fp16 at 15x15: the two conv launches (gates in their epilogues), + the initial-state pass
+#   bf16 at S = 7: gate-in (not at t = 0: the initial-state pass makes that operand), C1, gate-out, C2
+#   bf16x3 at k = 25: two launches per conv; + the initial state and the first gate-in
+#   bf16x3 at k = 32: the same with the two gates as SIMT launches of every timestep
+#   bf16x3 at k = 64, fp32: gate-in, C1, gate-out, C2 (fp32: + the integrations; no initial-state launch counted)
+LAUNCHES = {("bf16", 25, 15): (2, 4), ("bf16", 32, 15): (2, 4), ("bf16", 64, 15): (2, 4), ("bf16", 25, 7): (4, 3),
+            ("fp16", 25, 15): (2, 4), ("fp16", 64, 15): (2, 4),
+            ("bf16x3", 25, 15): (4, 5), ("bf16x3", 32, 15): (6, 4), ("bf16x3", 64, 15): (4, 4),
+            ("fp32", 25, 15): (6, 3)}
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("T_", [1, 3])
+@pytest.mark.parametrize("mode,k,S_", list(LAUNCHES))
+def test_launch_counts_per_path(mode, k, S_, T_):
+    """The absolute launch counts hgru_plan_launch_count and pose_plan_launch_count report, with and without the
+    H1 / H2 traces (which also turn the chaining off)."""
+    per_step, fixed = LAUNCHES[(mode, k, S_)]
+    lib = _lib.load()
+    n, H, W = 2, 20, 36
+    rng = np.random.default_rng(8)
+    X = torch.as_tensor(rng.uniform(-1, 1, size=(n, H, W, k)).astype(np.float32)).cuda()
+    params = {name: torch.as_tensor(np.asarray(v, np.float32)).cuda()
+              for name, v in init.hgru_params(k, S_, T_, seed=9).items()}
+    plan = _hgru_plan(n, H, W, k, S_, T_, mode, params)
+    try:
+        assert _hgru_run(plan, n, X, None, False, T_)[2] == fixed + per_step * T_
+        assert _hgru_run(plan, n, X, None, True, T_)[2] == fixed + (per_step + 2) * T_
+    finally:
+        lib.hgru_plan_destroy(plan)
+    m = mp.model()
+    m.channels, m.timesteps, m.SSF, m.SSN, m.fc_hidden, m.compute_mode = k, T_, S_, S_, F, mode
+    m.aux = dict(m.aux, hidden_init="zeros")
+    m.load_params(init.pose_params(channels=k, S=S_, T=T_, hw=HW, fc_hidden=F, out=O, seed=3, random_bn=True))
+    m.build(torch.as_tensor(init.synthetic_depth(n, seed=1, size=2 * HW)).cuda(), O)
+    torch.cuda.synchronize()
+    assert lib.pose_plan_launch_count(m._plan) == fixed + 2 + per_step * T_
