@@ -318,6 +318,13 @@ typedef struct {
   const float* bn[6][4];
 } attn_params_t;
 HGRU_API int attn_plan_create(int N, int H, int W, const int* widths, int fc_hidden, int O, attn_plan_t* out);
+/* The same with the arithmetic of the GEMM layers (aconv_2 .. aconv_5, afc_1; aconv_1, afc_out and everything between
+ * the GEMMs are fp32 in both): HGRU_MODE_BF16X3 (bf16 hi/lo operand splits, three products per k-step, fp32-class
+ * accuracy) is attn_plan_create's plan; HGRU_MODE_FP16 (fp16 operands, 11 significand bits, one product per k-step
+ * at the bf16 rate, fp32 accumulate: <= 2.5e-3 relative on every activation).  fp16 conversions saturate at +-65504,
+ * never inf / NaN.  Any other mode: HGRU_E_UNSUPPORTED. */
+HGRU_API int attn_plan_create_mode(int N, int H, int W, const int* widths, int fc_hidden, int O, int mode,
+                                   attn_plan_t* out);
 HGRU_API int attn_plan_destroy(attn_plan_t plan);
 HGRU_API int attn_set_params(attn_plan_t plan, const attn_params_t* params, float bn_epsilon, void* stream);
 /* frames [N,H,W] fp32 (depth / image_max_depth, as the caller feeds the reference graph) -> out [N,O] */

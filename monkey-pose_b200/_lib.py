@@ -95,6 +95,7 @@ SIGNATURES = {
     "joint_error_count_within_forward": (_I, [_P, _I, ctypes.c_float, _P, _P]),
     "axis1_error_mean_forward": (_I, [_P, _P, _I, _I, _I, _I, _P, _P, _P]),
     "attn_plan_create": (_I, [_I, _I, _I, ctypes.POINTER(_I), _I, _I, ctypes.POINTER(_P)]),
+    "attn_plan_create_mode": (_I, [_I, _I, _I, ctypes.POINTER(_I), _I, _I, _I, ctypes.POINTER(_P)]),
     "attn_plan_destroy": (_I, [_P]),
     "attn_set_params": (_I, [_P, ctypes.POINTER(AttnParams), ctypes.c_float, _P]),
     "attn_forward": (_I, [_P, _P, _P, _P]),

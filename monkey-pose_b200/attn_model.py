@@ -5,12 +5,17 @@
 (:615-633).  `depth` is a torch CUDA tensor [N,H,W,1] (or [N,H,W]) instead of a tf.Tensor; the forward runs in
 libhgru_b200.so (`attn_*` entry points of include/hgru_b200.h) -- there is no CPU fallback.
 
-`train_mode` in (None, False): the fused tensor-core pipeline, inference-mode batch norm (moving statistics).
+`train_mode` in (None, False): the fused tensor-core pipeline, inference-mode batch norm (moving statistics), with the
+GEMM layers (aconv_2 .. aconv_5, afc_1) in `compute_mode`: 'bf16x3' (default: bf16 hi/lo operand splits, three
+products per k-step, fp32-class accuracy, <= 1e-4 relative) or 'fp16' (fp16 operands, one product per k-step at the
+bf16 rate, fp32 accumulation: <= 2.5e-3 relative on every activation).  aconv_1 and afc_out are fp32 in both.
 `train_mode=True` -- what the reference passes both in training (:117) and, as committed, in
 `eval_model_on_real_data` (:360) -- composes the graph layer by layer from the class's own layer methods
 (`monkey_pose_b200.layers.LayerOps`): batch statistics in the six batch norms, dropout keep 0.7 after relu(afc_1)
-with the documented counter-based mask, moving-statistics updates in `updated_moving_stats`.  Forward only.
-Non-reference knobs: `widths`, `fc_hidden` (defaults = the reference's 64..1024 / 1024), `seed`, `dropout_seed`.
+with the documented counter-based mask, moving-statistics updates in `updated_moving_stats`.  Forward only.  It
+keeps its exact fp32 layer path whatever `compute_mode` says.
+Non-reference knobs: `widths`, `fc_hidden` (defaults = the reference's 64..1024 / 1024), `compute_mode`, `seed`,
+`dropout_seed`.
 """
 import ctypes
 
@@ -23,6 +28,7 @@ from .hgru_module import _as_dev, _stream
 from .layers import LayerOps
 
 _BN_FIELDS = ("gamma", "beta", "moving_mean", "moving_variance")
+_MODES = ("bf16x3", "fp16")        # compute_mode -> HGRU_MODE_* through _lib.MODES
 
 
 class attn_model_struct(LayerOps):
@@ -37,12 +43,24 @@ class attn_model_struct(LayerOps):
         # ---- non-reference knobs (defaults reproduce the reference's shapes) ----
         self.widths = (64, 128, 256, 512, 1024)     # :443, :456, :469, :482, :495
         self.fc_hidden = 1024                        # :501 (and hard-coded again at :522)
+        self.compute_mode = 'bf16x3'
         self.seed = 42
         self.dropout_seed = 1234
         self._plan = None
         self._plan_key = None
         self._plan_capacity = 0                      # frames the plan was created for: it runs every batch up to that
         self._dev_params = None
+
+    @property
+    def compute_mode(self):
+        """Arithmetic of the GEMM layers of the inference build: 'bf16x3' (default) or 'fp16'."""
+        return self._compute_mode
+
+    @compute_mode.setter
+    def compute_mode(self, mode):
+        if mode not in _MODES:
+            raise ValueError("attn_model_struct.compute_mode must be one of %s, not %r" % (list(_MODES), mode))
+        self._compute_mode = mode
 
     def __getitem__(self, name):
         return getattr(self, name)
@@ -125,15 +143,20 @@ class attn_model_struct(LayerOps):
             self._dev_params = self._materialise(int(output_shape))
         P, widths, F = self._dev_params
         # a plan runs any batch up to its capacity (attn_forward_batch); a larger batch re-creates it at that size
-        key = (H, W, widths, F, int(output_shape), depth.device.index)
+        key = (H, W, widths, F, int(output_shape), self.compute_mode, depth.device.index)
         if self._plan_key != key or N > self._plan_capacity:
             if self._plan is not None:
                 lib.attn_plan_destroy(self._plan)
                 self._plan = None
             plan = ctypes.c_void_p()
             wa = (ctypes.c_int * 5)(*widths)
-            _lib.check(lib.attn_plan_create(N, H, W, wa, F, int(output_shape), ctypes.byref(plan)),
-                       "attn_plan_create")
+            if self.compute_mode == 'bf16x3':       # attn_plan_create's plan, the entry point callers count on
+                _lib.check(lib.attn_plan_create(N, H, W, wa, F, int(output_shape), ctypes.byref(plan)),
+                           "attn_plan_create")
+            else:
+                _lib.check(lib.attn_plan_create_mode(N, H, W, wa, F, int(output_shape),
+                                                     _lib.MODES[self.compute_mode], ctypes.byref(plan)),
+                           "attn_plan_create_mode")
             self._plan, self._plan_key, self._plan_capacity = plan, key, N
             q = _lib.AttnParams()
             for i, (name, _) in enumerate(init.ATTN_CONV):

@@ -13,30 +13,36 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
+#include "op_format.cuh"
 #include "sm100_ptx.cuh"
 
 namespace hgru {
 
-// Precision: both operands are stored as bf16 hi + lo halves (hi = bf16(x), lo = bf16(x - hi)), the hi parts in
-// columns [0, Kpad) and the lo parts in [Kpad, 2*Kpad) of A and B.  Each k-block is accumulated as three
-// products  A_hi*B_hi + A_lo*B_hi + A_hi*B_lo  (fp32-class accuracy: K = 262 144 bf16 products would
-// otherwise contribute ~2.5e-3 relative error, the largest single error of the bf16 path).  A stage holds
-// the four tiles so B_hi is fetched once for two products; 2 stages x 96 KB.
+// Precision (template parameter Op, op_format.cuh):
+//   OpBf16x3: both operands are stored as bf16 hi + lo halves (hi = bf16(x), lo = bf16(x - hi)), the hi parts in
+//     columns [0, Kpad) and the lo parts in [Kpad, 2*Kpad) of A and B.  Each k-block is accumulated as three products
+//     A_hi*B_hi + A_lo*B_hi + A_hi*B_lo  (fp32-class accuracy: K = 262 144 bf16 products would otherwise contribute
+//     ~2.5e-3 relative error, the largest single error of the bf16 path).  A stage holds the four tiles so B_hi is
+//     fetched once for two products; 2 stages x 96 KB (BN = 256) / 3 x 64 KB (BN = 128).
+//   OpFp16: one fp16 operand per value (11 significand bits, row pitch Kpad), one product per k-step at the bf16
+//     rate; a stage is one A and one B tile, so the same shared memory holds 4 x 48 KB / 7 x 32 KB stages.
 constexpr int kGemmBM = 128, kGemmBN = 256, kGemmBK = 64;
 constexpr int kGemmABytes = kGemmBM * kGemmBK * 2;    // 16 KB
-template <int BN>
+template <int BN, class Op = OpBf16x3>
 struct GemmCfg {
   static_assert(BN == 128 || BN == 256, "N tile");
-  static constexpr int kStages = BN == 256 ? 2 : 3;
+  static constexpr int kParts = Op::kParts;
+  static constexpr int kStages = kParts == 2 ? (BN == 256 ? 2 : 3) : (BN == 256 ? 4 : 7);
   static constexpr int kBBytes = BN * kGemmBK * 2;                       // 32 / 16 KB
-  static constexpr int kStageBytes = 2 * kGemmABytes + 2 * kBBytes;      // A_hi, A_lo, B_hi, B_lo
+  static constexpr int kStageBytes = kParts * (kGemmABytes + kBBytes);   // A_hi, A_lo, B_hi, B_lo / A, B
   static constexpr int kSmemBytes = kStages * kStageBytes + 256 + 1024;
+  static_assert(kSmemBytes <= 227 * 1024, "shared memory");
 };
 constexpr int kGemmSmemBytes = GemmCfg<kGemmBN>::kSmemBytes;
 
 struct GemmArgs {
   int M, Nn, K;          // problem size
-  int Kpad;              // column where the lo halves start (K rounded up to the k-block)
+  int Kpad;              // K rounded up to the k-block: the column where the lo halves start (OpBf16x3)
   int kblocks_per_split; // K blocks (of 64) handled by one z slice
   float* part;           // [splits][M][Nn] fp32
   // implicit-GEMM convolution (CONV = true): A rows are the pixels (n, y, x) of a bf16 NHWC activation, K runs
@@ -56,18 +62,23 @@ __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t saddr) {
   return d;
 }
 
-// BN = 256 (2 stages x 96 KB) for wide outputs; BN = 128 (3 stages x 64 KB) where the output has <= 128 columns,
-// so that half of every MMA is not spent on zero-filled B rows.
+// BN = 256 for wide outputs; BN = 128 where the output has <= 128 columns, so that half of every MMA is not spent on
+// zero-filled B rows.
 // CONV = true: stride-1 SAME convolution as an implicit GEMM -- the A tile of k-block (tap, 64-channel block) is
 // one 4-D TMA box of the NHWC activation shifted by the tap (zero fill = padding); map_a / map_a_lo are the hi
 // and lo activation tensors.  CONV = false: plain GEMM, map_a_lo is ignored (lo halves sit at column Kpad).
-template <int BN, bool CONV = false>
+// map_a_lo is not read when Op has one part.
+template <int BN, bool CONV = false, class Op = OpBf16x3>
 __global__ void __launch_bounds__(256, 1)
 gemm_tc_splitk_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_a_lo,
                       const __grid_constant__ CUtensorMap map_b, const GemmArgs g) {
   using namespace sm100;
-  constexpr int kGemmBN = BN, kGemmStages = GemmCfg<BN>::kStages, kGemmBBytes = GemmCfg<BN>::kBBytes;
-  constexpr int kGemmStageBytes = GemmCfg<BN>::kStageBytes;
+  using Cfg = GemmCfg<BN, Op>;
+  constexpr bool kHiLo = Cfg::kParts == 2;
+  constexpr int kGemmBN = BN, kGemmStages = Cfg::kStages, kGemmBBytes = Cfg::kBBytes;
+  constexpr int kGemmStageBytes = Cfg::kStageBytes;
+  // stage layout: A_hi, [A_lo], B_hi, [B_lo]
+  constexpr int kBOff = Cfg::kParts * kGemmABytes;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t bars = base + kGemmStages * kGemmStageBytes;
@@ -85,7 +96,7 @@ gemm_tc_splitk_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_co
     mbar_init(bar_acc, 1);
     fence_barrier_init();
     tma_prefetch_desc(&map_a);
-    if constexpr (CONV) tma_prefetch_desc(&map_a_lo);
+    if constexpr (CONV && kHiLo) tma_prefetch_desc(&map_a_lo);
     tma_prefetch_desc(&map_b);
   }
   if (warp == 2) tmem_alloc<BN>(tmem_slot);
@@ -118,23 +129,26 @@ gemm_tc_splitk_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_co
           const int y0 = ppf >= kGemmBM ? (tile % (ppf / kGemmBM)) * g.by : 0;
           const int cx = tap % g.S - pad, cy = y0 + tap / g.S - pad;
           tma_load_4d(sa, &map_a, bar_full + 8 * st, cb * kGemmBK, cx, cy, f0);                  // A_hi
-          tma_load_4d(sa + kGemmABytes, &map_a_lo, bar_full + 8 * st, cb * kGemmBK, cx, cy, f0); // A_lo
+          if constexpr (kHiLo)
+            tma_load_4d(sa + kGemmABytes, &map_a_lo, bar_full + 8 * st, cb * kGemmBK, cx, cy, f0); // A_lo
         } else {
           tma_load_2d(sa, &map_a, bar_full + 8 * st, kc, m0);                                     // A_hi
-          tma_load_2d(sa + kGemmABytes, &map_a, bar_full + 8 * st, g.Kpad + kc, m0);              // A_lo
+          if constexpr (kHiLo)
+            tma_load_2d(sa + kGemmABytes, &map_a, bar_full + 8 * st, g.Kpad + kc, m0);            // A_lo
         }
-        tma_load_2d(sa + 2 * kGemmABytes, &map_b, bar_full + 8 * st, kc, n0);                   // B_hi
-        tma_load_2d(sa + 2 * kGemmABytes + kGemmBBytes, &map_b, bar_full + 8 * st, g.Kpad + kc, n0);   // B_lo
+        tma_load_2d(sa + kBOff, &map_b, bar_full + 8 * st, kc, n0);                              // B_hi
+        if constexpr (kHiLo)
+          tma_load_2d(sa + kBOff + kGemmBBytes, &map_b, bar_full + 8 * st, g.Kpad + kc, n0);     // B_lo
         if (++st == kGemmStages) { st = 0; ph ^= 1; }
       }
     }
   } else if (warp == 1) {
     const bool leader = elect_one();
-    constexpr uint32_t idesc = make_idesc(1, kGemmBM, kGemmBN);
+    constexpr uint32_t idesc = make_idesc(Op::kIdescFmt, kGemmBM, kGemmBN);
     const uint64_t a_hi = make_smem_desc_sw128(base);
     const uint64_t a_lo = make_smem_desc_sw128(base + kGemmABytes);
-    const uint64_t b_hi = make_smem_desc_sw128(base + 2 * kGemmABytes);
-    const uint64_t b_lo = make_smem_desc_sw128(base + 2 * kGemmABytes + kGemmBBytes);
+    const uint64_t b_hi = make_smem_desc_sw128(base + kBOff);
+    const uint64_t b_lo = make_smem_desc_sw128(base + kBOff + kGemmBBytes);
     uint32_t st = 0, ph = 0;
     for (int kb = 0; kb < nkb; ++kb) {
       mbar_wait_warp(bar_full + 8 * st, ph);
@@ -145,8 +159,10 @@ gemm_tc_splitk_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_co
         // advance 16 K-elements = 32 bytes inside the 128-byte swizzle row
         if (leader) {
           mma_bf16_ss(tmem_base, a_hi + so + ks * 2, b_hi + so + ks * 2, idesc, (kb | ks) != 0);
-          mma_bf16_ss(tmem_base, a_lo + so + ks * 2, b_hi + so + ks * 2, idesc, 1);
-          mma_bf16_ss(tmem_base, a_hi + so + ks * 2, b_lo + so + ks * 2, idesc, 1);
+          if constexpr (kHiLo) {
+            mma_bf16_ss(tmem_base, a_lo + so + ks * 2, b_hi + so + ks * 2, idesc, 1);
+            mma_bf16_ss(tmem_base, a_hi + so + ks * 2, b_lo + so + ks * 2, idesc, 1);
+          }
         }
       }
       if (leader) tc_commit(bar_empty + 8 * st);
@@ -195,11 +211,13 @@ gemm_tc_splitk_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_co
   }
 }
 
-// fc_1 weights [K][F] fp32 -> bf16 [F][hi(0..K) | pad | lo(0..K) | pad] (K-major B operand, row pitch
-// 2*Kpad); 32x32 tiles through shared memory.  The reference's K index (pin*k + c, tf.reshape of NHWC) is
-// permuted to channel-major (c*HW + pin), the order in which the H2 epilogue emits the A operand.
+// fc_1 weights [K][F] fp32 -> bf16 [F][hi(0..K) | pad | lo(0..K) | pad] (K-major B operand, row pitch 2*Kpad;
+// OpBf16x3) or fp16 [F][0..K | pad] (row pitch Kpad; OpFp16); 32x32 tiles through shared memory.  The reference's K
+// index (pin*k + c, tf.reshape of NHWC) is permuted to channel-major (c*HW + pin), the order in which the H2 epilogue
+// emits the A operand (kch = 1: no permutation).
+template <class Op = OpBf16x3>
 __global__ void __launch_bounds__(256)
-transpose_to_bf16_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ wt, int K, int F, int Kpad,
+transpose_operand_kernel(const float* __restrict__ w, typename Op::T* __restrict__ wt, int K, int F, int Kpad,
                          int kch) {
   __shared__ float tile[32][33];
   const int k0 = blockIdx.x * 32, f0 = blockIdx.y * 32;
@@ -215,10 +233,14 @@ transpose_to_bf16_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict_
       const float v = tile[tx][r];
       const int pin_ = kk / kch, c_ = kk - pin_ * kch;
       const int kd = c_ * (K / kch) + pin_;
-      const __nv_bfloat16 hi = __float2bfloat16(v);
-      __nv_bfloat16* row = wt + static_cast<size_t>(f) * (2 * static_cast<size_t>(Kpad));
-      row[kd] = hi;
-      row[Kpad + kd] = __float2bfloat16(v - __bfloat162float(hi));
+      if constexpr (Op::kParts == 2) {
+        const __nv_bfloat16 hi = __float2bfloat16(v);
+        __nv_bfloat16* row = wt + static_cast<size_t>(f) * (2 * static_cast<size_t>(Kpad));
+        row[kd] = hi;
+        row[Kpad + kd] = __float2bfloat16(v - __bfloat162float(hi));
+      } else {
+        wt[static_cast<size_t>(f) * Kpad + kd] = Op::cvt(v);
+      }
     }
   }
 }

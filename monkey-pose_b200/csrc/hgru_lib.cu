@@ -1012,7 +1012,7 @@ int pose_set_params(pose_plan_t p, const pose_params_t* q, float eps, void* stre
   const size_t K = static_cast<size_t>(p->HW) * p->HW * C;
   if (p->fc1_tc) {
     dim3 tg(static_cast<unsigned>((K + 31) / 32), (F + 31) / 32);
-    hgru::transpose_to_bf16_kernel<<<tg, 256, 0, st>>>(q->fc_1_weights, p->fc1_wt.as<__nv_bfloat16>(),
+    hgru::transpose_operand_kernel<<<tg, 256, 0, st>>>(q->fc_1_weights, p->fc1_wt.as<__nv_bfloat16>(),
                                                      static_cast<int>(K), F, p->fc_kpad, C);
   } else {
     CUDA_TRY(cudaMemcpyAsync(p->fc1_w.p, q->fc_1_weights, sizeof(float) * K * F, cudaMemcpyDeviceToDevice, st));
@@ -1416,14 +1416,20 @@ int layer_batch_norm_forward(const float* x, size_t rows, int C, const float* ga
 
 // ---- attention (centre-of-mass) CNN ----------------------------------------------------------------
 int attn_plan_create(int N, int H, int W, const int* widths, int fc_hidden, int O, attn_plan_t* out) {
+  return attn_plan_create_mode(N, H, W, widths, fc_hidden, O, HGRU_MODE_BF16X3, out);
+}
+
+int attn_plan_create_mode(int N, int H, int W, const int* widths, int fc_hidden, int O, int mode, attn_plan_t* out) {
   if (!out || !widths) return fail(HGRU_E_INVALID, "attn_plan_create: null pointer");
   *out = nullptr;
   if (N < 1 || H < 1 || W < 1 || fc_hidden < 1 || O < 1)
     return fail(HGRU_E_INVALID, "attn_plan_create: non-positive shape");
   for (int i = 0; i < 5; ++i)
     if (widths[i] < 8 || widths[i] % 8) return fail(HGRU_E_UNSUPPORTED, "attn_plan_create: widths must be multiples of 8");
+  if (mode != HGRU_MODE_BF16X3 && mode != HGRU_MODE_FP16)
+    return fail(HGRU_E_UNSUPPORTED, "attn_plan_create_mode: mode must be HGRU_MODE_BF16X3 or HGRU_MODE_FP16");
   attn_plan_s* p = new attn_plan_s();
-  p->N = N; p->n = N; p->H = H; p->W = W; p->F = fc_hidden; p->O = O;
+  p->N = N; p->n = N; p->H = H; p->W = W; p->F = fc_hidden; p->O = O; p->mode = mode;
   for (int i = 0; i < 5; ++i) p->w[i] = widths[i];
   const int rc = attn_plan_build(p);
   if (rc) {

@@ -21,9 +21,10 @@ from .tf_monkeydetector import prepare_data_test, preprocess_real_depth
 
 class FramesToJoints(object):
     """attn: `attn_model_struct` (or None: centres of mass estimated from the frames by the detector, refined on the
-    first crop when `docom`), pose: `model` (parameters loaded), md: `tfMonkeyDetector`, config: an object with
-    `image_orig_size`, `image_target_size`, `image_max_depth` (the reference's `monkeyConfig`), cube_z: seqconfig
-    ['cube'][2] (mm).  `chunks`: pieces the upload is cut into (the attention CNN starts on piece c while piece c+1 is
+    first crop when `docom`); its `compute_mode` ('bf16x3' or 'fp16') sets the attention CNN's arithmetic.
+    pose: `model` (parameters loaded), md: `tfMonkeyDetector`, config: an object with `image_orig_size`,
+    `image_target_size`, `image_max_depth` (the reference's `monkeyConfig`), cube_z: seqconfig ['cube'][2]
+    (mm).  `chunks`: pieces the upload is cut into (the attention CNN starts on piece c while piece c+1 is
     on the bus); 1 = plain stream order."""
 
     def __init__(self, attn, pose, md, config, cube_z=1200.0, num_joints=23, chunks=4, near=1000, far=3000,
